@@ -2,7 +2,7 @@
 """Benchmark of the BEV-projection hot path (BASELINE.json metric: BEV pool fwd+bwd frames/s
 and fraction of HBM peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One *step* = one pass of the camera pooling path over one batch of synthetic frames on each
@@ -12,6 +12,10 @@ the depth and context gradients.  The workload is BASELINE.json configs[1] (CFG-
 every rank processes its own frames, there is no collective on the data path ("weak" scaling).
 
 Prints ONE JSON line on rank 0.  See DESIGN.md section "Measurement" for the byte accounting.
+
+``--dump-outputs DIR``: after the timed steps, rank 0 writes what its last step returned -- the pooled BEV features
+(B, C, Y, X), the depth gradient and the context gradient -- as ``DIR/<name>.npy`` (float32).  The inputs are seeded,
+so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -152,6 +156,27 @@ def time_cuda(fn, iters, warmup):
         b.synchronize()
         ts.append(a.elapsed_time(b))
     return statistics.median(ts), min(ts)
+
+
+DUMP_MAX_ELEMENTS = 1 << 22          # per array: the three float32 outputs of a step stay under 64 MB
+
+
+def dump_outputs(out_dir: str, arrays: dict, seed: int = 0) -> None:
+    """Writes every array as ``out_dir/<name>.npy`` in float32.  An array of more than DUMP_MAX_ELEMENTS elements is
+    written as a 1-D sample of its flattened (row-major) elements: one position from each of DUMP_MAX_ELEMENTS equal
+    slices, drawn with a fixed seed, hence the same positions in every run with the same shapes."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        n, k = t.numel(), DUMP_MAX_ELEMENTS
+        if n > k:
+            gen = torch.Generator().manual_seed(seed)
+            lo = torch.arange(k, dtype=torch.int64) * n // k
+            width = torch.arange(1, k + 1, dtype=torch.int64) * n // k - lo
+            idx = lo + (torch.rand(k, generator=gen, dtype=torch.float64) * width).long()
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------
@@ -462,7 +487,16 @@ def main():
     ap.add_argument('--no-extras', action='store_true', help='skip e2e / cpu / reference-CUDA side measurements')
     ap.add_argument('--sweep', default='mini', choices=['mini', 'full'],
                     help="'full': BASELINE.json configs[4] batch 1..64 x {128,256,512}^2 with both reference arms per point")
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step to DIR/<name>.npy (float32; a fixed seeded sample of '
+                         f'arrays above {DUMP_MAX_ELEMENTS} elements).  Only the native camera pooling step '
+                         '(--impl native with --workload cfg2 or aim) dumps: it is the path two builds of the kernels '
+                         'are compared on; the CPU port and the training harness are refused')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'native' or args.workload == 'train'):
+        ap.error('--dump-outputs covers the native camera pooling step only (--impl native, --workload cfg2 or aim)')
     args.batch_given = any(a == '--batch' or a.startswith('--batch=') for a in sys.argv[1:])
     cfg = CFG_AIM if args.workload == 'aim' else CFG_2
     if args.workload == 'aim' and not args.batch_given:
@@ -482,17 +516,9 @@ def main():
         if rank != 0:
             return
         frames = 2
-        t0 = time.perf_counter()
-        vals = []
-        res = None
-        for _ in range(max(1, min(args.steps, 5))):
-            res = run_cpu_baseline(cfg, frames, 1)
-            vals.append(res['value'])
-            if time.perf_counter() - t0 > 120:
-                break
-        v = statistics.median(vals)
-        res['value'] = v
-        line = {'metric': METRIC, 'value': v, 'unit': UNIT, 'n_gpus': args.gpus, 'steps': len(vals),
+        res = run_cpu_baseline(cfg, frames, args.steps)
+        v = res['value']
+        line = {'metric': METRIC, 'value': v, 'unit': UNIT, 'n_gpus': args.gpus, 'steps': args.steps,
                 'warmup': 1, 'ms_per_step': frames / v * 1e3, 'higher_is_better': True, 'scaling': 'weak',
                 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic', 'impl': 'reference',
                 'config': dict(workload, frames_per_gpu_per_step=frames, device='cpu'),
@@ -605,12 +631,18 @@ def main():
         dist.barrier()
     torch.cuda.synchronize()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    last = None
     with ClockSampler(local_rank) as clocks:
         ev0.record()
         for _ in range(args.steps):
-            run()
+            last = run()
         ev1.record()
         torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        _, out_last, gd_last, gc_last = keep if graph is not None else last   # a replay refills the captured outputs
+        dump_outputs(args.dump_outputs, {'bev_features': out_last.permute(0, 3, 1, 2), 'grad_depth': gd_last,
+                                         'grad_context': gc_last})
+        del out_last, gd_last, gc_last
     if world > 1:
         dist.barrier()
     from mm_training_b200.sharding import aggregate_throughput

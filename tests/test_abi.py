@@ -63,14 +63,36 @@ def test_python_ops_refuse_cpu_tensors():
         voxel_pooling(torch.zeros(1, 4, 3, dtype=torch.int32), torch.zeros(1, 4, 8), [2, 2, 1])
 
 
-def test_bench_byte_model_matches_the_survey():
-    """bench.py's roofline numerator is SURVEY.md section 8(d), row (B): 32.5 MB per CFG-2 frame."""
+def _bench_module():
     import importlib.util
     spec = importlib.util.spec_from_file_location('bench_mod', os.path.join(ROOT, 'bench.py'))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_byte_model_matches_the_survey():
+    """bench.py's roofline numerator is SURVEY.md section 8(d), row (B): 32.5 MB per CFG-2 frame."""
+    bench = _bench_module()
     from mm_training_b200.configs import CFG_2, CFG_AIM
     b = bench.algorithmic_bytes(CFG_2, 150442)
     assert abs(b['step'] - 32.5e6) < 0.1e6
     assert b['fused_forward'] + b['fused_backward'] < b['step'] * 1.05
     assert abs(bench.algorithmic_bytes(CFG_AIM, 738884)['step'] - 108e6) < 1.5e6
+
+
+def test_bench_dump_outputs_is_a_fixed_bounded_sample(tmp_path):
+    """bench.py --dump-outputs: float32 .npy files; small arrays whole, large ones as the same seeded sample every run."""
+    import numpy as np
+    import torch
+    bench = _bench_module()
+    n = bench.DUMP_MAX_ELEMENTS
+    big = torch.arange(n + 1000, dtype=torch.float64)          # element value == flat position
+    small = torch.rand(2, 3, 4)
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), {'big': big, 'small': small})
+    a, b = np.load(tmp_path / 'a' / 'big.npy'), np.load(tmp_path / 'b' / 'big.npy')
+    assert a.dtype == np.float32 and np.array_equal(a, b)
+    assert a.size == n and bool((np.diff(a) > 0).all())       # distinct positions, in order
+    s = np.load(tmp_path / 'a' / 'small.npy')
+    assert s.dtype == np.float32 and np.array_equal(s, small.numpy())

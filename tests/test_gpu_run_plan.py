@@ -208,3 +208,36 @@ def test_cold_forward_with_overlapped_fill_equals_plain_forward_and_is_capturabl
     d, c = depth.clone().requires_grad_(True), ctx.clone().requires_grad_(True)
     o = voxel_pooling_fused(geom, d, c, vn)
     assert torch.equal(o.permute(0, 2, 3, 1), ref)
+
+
+def test_bench_dump_outputs_are_the_timed_step_outputs(tmp_path):
+    """bench.py --dump-outputs writes what the timed step returned: the captured outputs refilled by the last graph
+    replay (or the last eager step), the forward permuted to (B, C, Y, X), on the seeded inputs of rank 0."""
+    import importlib.util
+    import json
+    import os
+    import subprocess
+    import sys
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    for mode in ('graph', 'eager'):
+        cmd = [sys.executable, os.path.join(root, 'bench.py'), '--gpus', '1', '--batch', '2', '--steps', '3', '--warmup', '1',
+               '--no-extras', '--dump-outputs', str(tmp_path / mode)] + (['--no-graph'] if mode == 'eager' else [])
+        res = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-2000:]
+        line = json.loads(res.stdout.strip().splitlines()[-1])
+        assert line['steps'] == 3 and line['config']['launch'] == ('cuda_graph_replay' if mode == 'graph' else 'eager')
+    spec = importlib.util.spec_from_file_location('bench_mod', os.path.join(root, 'bench.py'))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    geom, vn = synthetic.camera_rig(CFG_2, 2, device=DEV, yaw_jitter_deg=5.0, seed=1)
+    depth, ctx, go = synthetic.camera_features(CFG_2, 2, device=DEV, seed=1)
+    d, c = depth.requires_grad_(True), ctx.requires_grad_(True)
+    out = voxel_pooling_fused(geom, d, c, vn.tolist())                         # (B, C, Y, X)
+    out.backward(go)
+    bench.dump_outputs(str(tmp_path / 'expect'), {'bev_features': out, 'grad_depth': d.grad, 'grad_context': c.grad})
+    for name, tol in (('bev_features', 1e-6), ('grad_depth', 1e-5), ('grad_context', 1e-5)):
+        want = np.load(tmp_path / 'expect' / f'{name}.npy')
+        graph, eager = (np.load(tmp_path / m / f'{name}.npy') for m in ('graph', 'eager'))
+        assert graph.shape == want.shape and np.array_equal(graph, eager)
+        assert np.allclose(graph, want, rtol=1e-5, atol=tol), name

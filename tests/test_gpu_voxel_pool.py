@@ -84,7 +84,7 @@ def test_reference_unit_test_recipe(kernel_path):
 
 def test_against_reference_cuda_kernel():
     if not ref_cuda_op.available():
-        pytest.skip('oracle/_ref not built')
+        pytest.skip('oracle/_ref not built: needs a checkout of the reference (make -C oracle ref REF=<checkout>)')
     geom_xyz, features = vp.reference_test_inputs()
     g, f = geom_xyz.cuda().int(), features.cuda()
     ref_out, ref_pos = ref_cuda_op.ref_forward_with_pos_memo(g, f, [128, 128, 1])
