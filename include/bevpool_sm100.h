@@ -234,6 +234,28 @@ int bevpool_grad_rows(const void *plan, const void *grad_out_nchw, void *rows_nh
 int bevpool_transpose(const void *in, void *out, int dtype, int batch, int64_t rows,
                       int64_t cols, void *stream);
 
+/* ---- BEV augmentation warp: kornia warp_affine(src, M, dsize, 'bilinear', 'zeros', align_corners=True) -------------
+ * What models/bev_depth.py's bev_augment_image applies to the pooled camera BEV with the BDA matrix.  fp32 rows of
+ * `channels` floats (channels % 4 == 0), channels-last: source cell (b, y, x) at src_rows + ((b*src_h + y)*src_w + x)
+ * * src_row_stride floats, destination pixels likewise with out_row_stride (strides >= channels, multiples of 4; the
+ * rows may sit inside a wider buffer such as the concatenated BEV features).  All sizes >= 2.
+ *   theta   device float32 (batch, 2, 3): kornia's normalised destination -> normalised source matrix, i.e.
+ *           inverse(N(dst) @ [M; 0 0 1] @ inverse(N(src)))[:, :2] with N(h, w) = [[2/(w-1), 0, -1], [0, 2/(h-1), -1],
+ *           [0, 0, 1]] (computed from M in torch: mm_training_b200/ops/bev_augment.py)
+ *   cell_start  optional (NULL or a pooling plan's CSR, batch*src_h*src_w + 1 entries): source cells with
+ *           cell_start[c + 1] == cell_start[c] are zero rows.  Forward: never read (same result, bit for bit, as a row
+ *           of zeros).  Backward: gradient rows are written for occupied cells only; the others are left untouched.
+ * forward  every destination element is written once (zeros included).  Taps are summed in the order nw, ne, sw, se.
+ * backward grad_src = adjoint of the forward, gathered per source cell in ascending destination order: no atomics,
+ *          bit-stable.  Its cost per cell grows with 4 / |det A| (A: the destination -> source pixel map), i.e. with
+ *          the magnification of the warp.  A non-finite theta gives zero rows in both directions.                     */
+int bevpool_warp_affine_forward(const float *theta, const void *src_rows, int64_t src_row_stride, void *out_rows,
+                                int64_t out_row_stride, const int32_t *cell_start, int batch, int channels, int src_h,
+                                int src_w, int dst_h, int dst_w, void *stream);
+int bevpool_warp_affine_backward(const float *theta, const void *grad_out_rows, int64_t grad_out_row_stride,
+                                 void *grad_src_rows, int64_t grad_src_row_stride, const int32_t *cell_start, int batch,
+                                 int channels, int src_h, int src_w, int dst_h, int dst_w, void *stream);
+
 /* ==== LiDAR / radar branch ==========================================================
  * Replaces what the reference reaches through models/bev_depth.py:181-183:
  *   mmcv `hard_voxelize_forward` (via mmdet3d `MVXTwoStageDetector.voxelize`), mmdet3d

@@ -55,6 +55,8 @@ _SIGNATURES = {
     'bevpool_rig_geom': [_vp, _vp, _vp, _vp, _fp, _fp, _i, _i, _i, _i, _i, _i, _vp, _vp],
     'bevpool_grad_rows': [_vp, _vp, _vp, _i, _i, _i64, _i, _i, _i, _vp],
     'bevpool_transpose': [_vp, _vp, _i, _i, _i64, _i64, _vp],
+    'bevpool_warp_affine_forward': [_vp, _vp, _i64, _vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp],
+    'bevpool_warp_affine_backward': [_vp, _vp, _i64, _vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp],
     'bevvox_temp_bytes': [_i, _i64, _ip, _i, _i, _szp],
     'bevvox_hard_voxelize_scatter': [_vp, _vp, _vp, _i, _i64, _i64, _i, _fp, _fp, _ip, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp],
     'bevvox_hard_voxelize': [_vp, _vp, _i, _i64, _i64, _i, _fp, _fp, _ip, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp],

@@ -13,7 +13,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB_PATH = os.path.join(HERE, 'libbevpool_sm100.so')
-SOURCES = ['plan.cu', 'pool.cu', 'pool_runs.cu', 'pool_bwd.cu', 'pool_bwd2.cu', 'voxelize.cu', 'depth_labels.cu', 'depth_softmax.cu']
+SOURCES = ['plan.cu', 'pool.cu', 'pool_runs.cu', 'pool_bwd.cu', 'pool_bwd2.cu', 'voxelize.cu', 'depth_labels.cu', 'depth_softmax.cu',
+           'bev_warp.cu']
 NVCC_FLAGS = ['-O3', '-std=c++17', '-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo',
               '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr']
 # never --use_fast_math: index arithmetic (voxelizer floor/div) must stay IEEE

@@ -526,11 +526,18 @@ def voxel_pooling_fused(geom_xyz: Optional[torch.Tensor], depth: torch.Tensor, c
     return VoxelPoolingFused.apply(geom_xyz, depth, context, voxel_num, plan, None, None)
 
 
+def _warp_scratch(B: int, Y: int, X: int, C: int, device) -> torch.Tensor:
+    """Uninitialised (B, Y, X, C) float32 rows between the pooling and the BDA warp.  Only the rows of occupied cells
+    are ever written or read (tests substitute a NaN-filled buffer to prove it)."""
+    return torch.empty(B, Y, X, C, dtype=torch.float32, device=device)
+
+
 class VoxelPoolingFusedConcat(Function):
-    """``torch.cat([voxel_pooling_fused(...), other_bev], dim=1)`` without the copies of the camera half."""
+    """``torch.cat([voxel_pooling_fused(...), other_bev], dim=1)`` without the copies of the camera half; with ``theta``
+    the camera half is ``warp_affine(voxel_pooling_fused(...), M, (Y, X))`` (``theta`` = ``bev_augment.warp_theta(M)``)."""
 
     @staticmethod
-    def forward(ctx, depth, context, other_bev, voxel_num, plan):
+    def forward(ctx, depth, context, other_bev, voxel_num, plan, theta=None):
         _lib.require_cuda(depth, context, other_bev)
         X, Y, _ = _voxel_num_ints(voxel_num)
         BN, D, H, W = depth.shape
@@ -547,12 +554,19 @@ class VoxelPoolingFusedConcat(Function):
             cap = max(1, plan.num_sorted)
             run_rows = torch.empty(cap, C, dtype=torch.float32, device=depth.device)
             ws = _forward_workspace(C, depth.device)
+            # with the warp, the pooled rows go to a scratch first -- occupied cells only (no zero fill): the warp skips
+            # the taps of empty cells through the plan's cell_start
+            pooled, stride = (buf, Ct) if theta is None else (_warp_scratch(B, Y, X, C, depth.device), C)
             _lib.check(_lib.lib().bevpool_fused_forward_runs_into(
-                plan.ptr, depth.data_ptr(), (context if nchw else rows).data_ptr(), 1 if nchw else 0, buf.data_ptr(), Ct,
+                plan.ptr, depth.data_ptr(), (context if nchw else rows).data_ptr(),
+                (1 if nchw else 0) | (0 if theta is None else 2), pooled.data_ptr(), stride,
                 _lib.dtype_code(depth), B, N, D, H, W, C, X, Y, run_rows.data_ptr(), cap, ws.data_ptr(),
                 _lib.stream_ptr(depth.device)), 'bevpool_fused_forward_runs_into')
+            if theta is not None:
+                from ..bev_augment import warp_forward_rows
+                warp_forward_rows(theta, pooled, C, buf, Ct, plan.cell_start, B, C, (Y, X), (Y, X))
             buf[..., C:].copy_(other_bev.permute(0, 2, 3, 1))          # the other half: the one copy a cat cannot avoid
-        ctx.plan, ctx.nchw, ctx.C, ctx.other_dtype = plan, nchw, C, other_bev.dtype
+        ctx.plan, ctx.nchw, ctx.C, ctx.other_dtype, ctx.theta = plan, nchw, C, other_bev.dtype, theta
         if nchw:
             ctx.save_for_backward(depth, context)
         else:
@@ -575,6 +589,13 @@ class VoxelPoolingFusedConcat(Function):
             g = g.float().contiguous()
         Ct = g.shape[-1]
         with torch.cuda.device(depth.device):
+            grad_rows, stride = g, Ct
+            if ctx.theta is not None:
+                # gradient of the pooled rows = warp backward of the camera half of grad_cat, occupied cells only (the
+                # pooling backward reads no other row)
+                from ..bev_augment import warp_backward_rows
+                grad_rows, stride = _warp_scratch(B, Y, X, C, depth.device), C
+                warp_backward_rows(ctx.theta, g, Ct, grad_rows, C, plan.cell_start, B, C, (Y, X), (Y, X))
             grad_depth = torch.empty_like(depth)
             if ctx.nchw:
                 grad_context = torch.empty_like(context)
@@ -582,7 +603,7 @@ class VoxelPoolingFusedConcat(Function):
             else:
                 gc_arg = torch.empty(BN, H, W, C, dtype=context.dtype, device=context.device)
             _lib.check(_lib.lib().bevpool_fused_backward_runs_from(
-                plan.ptr, g.data_ptr(), Ct, depth.data_ptr(), (context if ctx.nchw else rows).data_ptr(),
+                plan.ptr, grad_rows.data_ptr(), stride, depth.data_ptr(), (context if ctx.nchw else rows).data_ptr(),
                 grad_depth.data_ptr(), gc_arg.data_ptr(), 1 if ctx.nchw else 0, _lib.dtype_code(depth), B, N, D, H, W, C, X, Y,
                 _lib.stream_ptr(depth.device)), 'bevpool_fused_backward_runs_from')
             if not ctx.nchw:
@@ -591,21 +612,37 @@ class VoxelPoolingFusedConcat(Function):
                 else:
                     grad_context = _transpose(gc_arg, BN, H * W, C).view(BN, C, H, W)
         grad_other = g[..., C:].permute(0, 3, 1, 2).to(ctx.other_dtype)
-        return grad_depth, grad_context, grad_other, None, None
+        return grad_depth, grad_context, grad_other, None, None, None
 
 
 def voxel_pooling_fused_concat(depth: torch.Tensor, context: torch.Tensor, other_bev: torch.Tensor, voxel_num: VoxelNum,
-                               plan: PoolingPlan) -> torch.Tensor:
+                               plan: PoolingPlan, *, bda_affine: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Concat epilogue of the camera branch (``models/bev_depth.py:187-189``): returns
     ``torch.cat([voxel_pooling_fused(None, depth, context, voxel_num, plan), other_bev], dim=1)`` as a float32
     channels-last tensor.  On a run plan (fp32, W % 4 == 0) the pooled rows are written straight into the concatenated
     buffer and the backward reads its gradient rows straight out of the concatenated gradient -- neither
-    ``lss_fpn.py:466``'s ``.contiguous()`` nor the cat copies the camera half; other cases compose the two stock ops."""
+    ``lss_fpn.py:466``'s ``.contiguous()`` nor the cat copies the camera half; other cases compose the two stock ops.
+
+    ``bda_affine``: the BDA matrix as ``bev_augment_image`` passes it to kornia, (B, 2, 3), no gradient.  The camera
+    half is then ``warp_affine(voxel_pooling_fused(...), bda_affine, (Y, X))`` (``ops/bev_augment.py``).  On a run plan
+    the pooled map is never zero-filled: the warp skips the empty cells the plan knows of, and its backward produces
+    gradient rows for occupied cells only."""
     C = context.shape[1]
-    if (plan.mode == 'runs' and runs_supported(C, depth.dtype) and depth.shape[3] % 4 == 0 and other_bev.shape[1] % 4 == 0
-            and depth.is_contiguous()):
-        return VoxelPoolingFusedConcat.apply(depth, context, other_bev, voxel_num, plan)
-    return torch.cat([voxel_pooling_fused(None, depth, context, voxel_num, plan), other_bev.to(depth.dtype)], dim=1)
+    fast = (plan.mode == 'runs' and runs_supported(C, depth.dtype) and depth.shape[3] % 4 == 0
+            and other_bev.shape[1] % 4 == 0 and depth.is_contiguous())
+    if bda_affine is None:
+        if fast:
+            return VoxelPoolingFusedConcat.apply(depth, context, other_bev, voxel_num, plan, None)
+        return torch.cat([voxel_pooling_fused(None, depth, context, voxel_num, plan), other_bev.to(depth.dtype)], dim=1)
+    from ..bev_augment import warp_affine, warp_theta
+    X, Y, _ = plan.voxel_num
+    if bda_affine.shape[0] != plan.batch:
+        raise ValueError(f'bda_affine has {bda_affine.shape[0]} matrices for a batch of {plan.batch}')
+    if fast:
+        theta = warp_theta(bda_affine, (Y, X), (Y, X)).to(depth.device)
+        return VoxelPoolingFusedConcat.apply(depth, context, other_bev, voxel_num, plan, theta)
+    pooled = voxel_pooling_fused(None, depth, context, voxel_num, plan)
+    return torch.cat([warp_affine(pooled, bda_affine, (Y, X)), other_bev.to(pooled.dtype)], dim=1)
 
 
 class VoxelPoolingFusedLogits(Function):
