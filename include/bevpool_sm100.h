@@ -256,6 +256,31 @@ int bevpool_warp_affine_backward(const float *theta, const void *grad_out_rows, 
                                  void *grad_src_rows, int64_t grad_src_row_stride, const int32_t *cell_start, int batch,
                                  int channels, int src_h, int src_w, int dst_h, int dst_w, void *stream);
 
+/* ---- nearest resampling of the LiDAR BEV into the concatenated rows: F.interpolate(src, size=(dst_h, dst_w),
+ * mode='nearest') + torch.cat([camera_half, .], 1) ---------------------------------------------------------------------
+ * What models/bev_depth.py does to the LiDAR BEV before the concat with the camera BEV, any pair of sizes (up or down).
+ * Per axis src(d) = min(floor(float(d) * (float(in) / float(out))), in - 1), torch's float32 rule (ATen/native/
+ * UpSample.h); the y and x maps are separable.
+ *   src / grad_src  (batch, channels, src_h, src_w) of element type `dtype` (BEVPOOL_F32 / F16 / BF16): NCHW-contiguous
+ *           when src_is_nchw != 0, else channels_last (pixel rows of `channels` elements, 16-byte aligned for fp32,
+ *           8-byte for 16-bit types)
+ *   out_rows / grad_rows  fp32 rows of the concatenated buffer: destination cell (b, y, x) at + ((b*dst_h + y)*dst_w + x)
+ *           * row_stride floats (row_stride >= channels, multiple of 4; 16-byte aligned), i.e. the address of the first
+ *           LiDAR channel of cell 0.  Other channels of a row are not touched.
+ *   channels % 4 == 0; all sizes >= 1.
+ * forward  every destination element is an exact fp32 copy of one source element (bit-equal to the stock ops).
+ * backward grad_src = adjoint of the forward's own index maps: per source cell the sum over its preimage (ascending y,
+ *          then ascending x: torch's CUDA upsample_nearest2d_backward order), fp32 from +0, rounded once to `dtype`.
+ *          A gather (no atomics, bit-stable); every element written once, zeros for empty preimages (down-sampling).
+ * bevpool_resize_nearest_index (host only, no device work): the maps the kernels use -- src_of_dst_host[d] for d <
+ * out_size and first_dst_host[s] for s <= in_size (preimage of s = [first_dst[s], first_dst[s + 1])); either may be NULL. */
+int bevpool_resize_nearest_into(const void *src, int dtype, int src_is_nchw, int batch, int channels, int src_h,
+                                int src_w, int dst_h, int dst_w, float *out_rows, int64_t out_row_stride, void *stream);
+int bevpool_resize_nearest_backward_from(const float *grad_rows, int64_t grad_row_stride, void *grad_src, int dtype,
+                                         int src_is_nchw, int batch, int channels, int src_h, int src_w, int dst_h,
+                                         int dst_w, void *stream);
+int bevpool_resize_nearest_index(int in_size, int out_size, int32_t *src_of_dst_host, int32_t *first_dst_host);
+
 /* ==== LiDAR / radar branch ==========================================================
  * Replaces what the reference reaches through models/bev_depth.py:181-183:
  *   mmcv `hard_voxelize_forward` (via mmdet3d `MVXTwoStageDetector.voxelize`), mmdet3d

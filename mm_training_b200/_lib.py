@@ -57,7 +57,10 @@ _SIGNATURES = {
     'bevpool_transpose': [_vp, _vp, _i, _i, _i64, _i64, _vp],
     'bevpool_warp_affine_forward': [_vp, _vp, _i64, _vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp],
     'bevpool_warp_affine_backward': [_vp, _vp, _i64, _vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp],
-    'bevvox_temp_bytes': [_i, _i64, _ip, _i, _i, _szp],
+    'bevpool_resize_nearest_into': [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp],
+    'bevpool_resize_nearest_backward_from': [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
+    'bevpool_resize_nearest_index': [_i, _i, _vp, _vp],
+    'bevvox_temp_bytes':[_i, _i64, _ip, _i, _i, _szp],
     'bevvox_hard_voxelize_scatter': [_vp, _vp, _vp, _i, _i64, _i64, _i, _fp, _fp, _ip, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp],
     'bevvox_hard_voxelize': [_vp, _vp, _i, _i64, _i64, _i, _fp, _fp, _ip, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp],
     'bevvox_dynamic_voxelize': [_vp, _i64, _i, _fp, _fp, _ip, _vp, _vp],

@@ -532,20 +532,36 @@ def _warp_scratch(B: int, Y: int, X: int, C: int, device) -> torch.Tensor:
     return torch.empty(B, Y, X, C, dtype=torch.float32, device=device)
 
 
+def _other_layout(other_bev: torch.Tensor) -> Optional[int]:
+    """1 for an NCHW-contiguous ``other_bev``, 0 for channels_last, None for a layout / dtype / alignment the resampling
+    kernels do not take (csrc/bev_resample.cu: fp32 / bf16 / fp16, rows of C2 % 4 == 0 elements, vector-aligned)."""
+    if other_bev.dtype not in (torch.float32, torch.bfloat16, torch.float16) or other_bev.shape[1] % 4 != 0:
+        return None
+    if other_bev.is_contiguous():
+        return 1
+    if other_bev.permute(0, 2, 3, 1).is_contiguous() and other_bev.data_ptr() % 16 == 0:
+        return 0
+    return None
+
+
 class VoxelPoolingFusedConcat(Function):
     """``torch.cat([voxel_pooling_fused(...), other_bev], dim=1)`` without the copies of the camera half; with ``theta``
-    the camera half is ``warp_affine(voxel_pooling_fused(...), M, (Y, X))`` (``theta`` = ``bev_augment.warp_theta(M)``)."""
+    the camera half is ``warp_affine(voxel_pooling_fused(...), M, (Y, X))`` (``theta`` = ``bev_augment.warp_theta(M)``);
+    with ``resize`` the other half is ``F.interpolate(other_bev, size=(Y, X), mode='nearest')``.  The other half is
+    written by ``bevpool_resize_nearest_into`` in either case (identity maps when the sizes agree)."""
 
     @staticmethod
-    def forward(ctx, depth, context, other_bev, voxel_num, plan, theta=None):
+    def forward(ctx, depth, context, other_bev, voxel_num, plan, theta=None, resize=False):
         _lib.require_cuda(depth, context, other_bev)
         X, Y, _ = _voxel_num_ints(voxel_num)
         BN, D, H, W = depth.shape
         C = context.shape[1]
         B = plan.batch
         N = BN // B
-        assert other_bev.shape[0] == B and tuple(other_bev.shape[2:]) == (Y, X)
-        C2 = other_bev.shape[1]
+        assert other_bev.shape[0] == B and (resize or tuple(other_bev.shape[2:]) == (Y, X))
+        C2, Yl, Xl = other_bev.shape[1:]
+        other_nchw = _other_layout(other_bev)
+        assert other_nchw is not None
         Ct = C + C2
         nchw = _nchw_direct(context, depth)
         rows = None if nchw else context_rows_nhwc(context)
@@ -565,8 +581,12 @@ class VoxelPoolingFusedConcat(Function):
             if theta is not None:
                 from ..bev_augment import warp_forward_rows
                 warp_forward_rows(theta, pooled, C, buf, Ct, plan.cell_start, B, C, (Y, X), (Y, X))
-            buf[..., C:].copy_(other_bev.permute(0, 2, 3, 1))          # the other half: the one copy a cat cannot avoid
+            # the other half (resampled or not): the one copy a cat cannot avoid
+            _lib.check(_lib.lib().bevpool_resize_nearest_into(
+                other_bev.data_ptr(), _lib.dtype_code(other_bev), other_nchw, B, C2, Yl, Xl, Y, X, buf.data_ptr() + 4 * C, Ct,
+                _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_into')
         ctx.plan, ctx.nchw, ctx.C, ctx.other_dtype, ctx.theta = plan, nchw, C, other_bev.dtype, theta
+        ctx.other_shape, ctx.other_nchw, ctx.other_code = (B, C2, Yl, Xl), other_nchw, _lib.dtype_code(other_bev)
         if nchw:
             ctx.save_for_backward(depth, context)
         else:
@@ -611,12 +631,26 @@ class VoxelPoolingFusedConcat(Function):
                     grad_context = gc_arg.permute(0, 3, 1, 2)
                 else:
                     grad_context = _transpose(gc_arg, BN, H * W, C).view(BN, C, H, W)
-        grad_other = g[..., C:].permute(0, 3, 1, 2).to(ctx.other_dtype)
-        return grad_depth, grad_context, grad_other, None, None, None
+            _, C2, Yl, Xl = ctx.other_shape
+            if (Yl, Xl) == (Y, X):
+                grad_other = g[..., C:].permute(0, 3, 1, 2).to(ctx.other_dtype)      # identity maps: a view
+            elif not ctx.needs_input_grad[2]:
+                grad_other = None
+            else:
+                # adjoint gather straight out of the concatenated gradient; the layout of other_bev
+                if ctx.other_nchw:
+                    grad_other = torch.empty(B, C2, Yl, Xl, dtype=ctx.other_dtype, device=depth.device)
+                else:
+                    grad_other = torch.empty(B, Yl, Xl, C2, dtype=ctx.other_dtype, device=depth.device).permute(0, 3, 1, 2)
+                _lib.check(_lib.lib().bevpool_resize_nearest_backward_from(
+                    g.data_ptr() + 4 * C, Ct, grad_other.data_ptr(), ctx.other_code, ctx.other_nchw, B, C2,
+                    Yl, Xl, Y, X, _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_backward_from')
+        return grad_depth, grad_context, grad_other, None, None, None, None
 
 
 def voxel_pooling_fused_concat(depth: torch.Tensor, context: torch.Tensor, other_bev: torch.Tensor, voxel_num: VoxelNum,
-                               plan: PoolingPlan, *, bda_affine: Optional[torch.Tensor] = None) -> torch.Tensor:
+                               plan: PoolingPlan, *, bda_affine: Optional[torch.Tensor] = None,
+                               resize_other: Optional[str] = None) -> torch.Tensor:
     """Concat epilogue of the camera branch (``models/bev_depth.py:187-189``): returns
     ``torch.cat([voxel_pooling_fused(None, depth, context, voxel_num, plan), other_bev], dim=1)`` as a float32
     channels-last tensor.  On a run plan (fp32, W % 4 == 0) the pooled rows are written straight into the concatenated
@@ -626,23 +660,39 @@ def voxel_pooling_fused_concat(depth: torch.Tensor, context: torch.Tensor, other
     ``bda_affine``: the BDA matrix as ``bev_augment_image`` passes it to kornia, (B, 2, 3), no gradient.  The camera
     half is then ``warp_affine(voxel_pooling_fused(...), bda_affine, (Y, X))`` (``ops/bev_augment.py``).  On a run plan
     the pooled map is never zero-filled: the warp skips the empty cells the plan knows of, and its backward produces
-    gradient rows for occupied cells only."""
+    gradient rows for occupied cells only.
+
+    ``resize_other='nearest'``: ``other_bev`` (B, C2, Yl, Xl), any Yl, Xl >= 1, is resampled to the camera grid first --
+    the other half is ``F.interpolate(other_bev, size=(Y, X), mode='nearest').float()`` (``bev_depth.py:188-190``), bit
+    for bit.  On the native path (fp32 / bf16 / fp16, NCHW or channels_last, C2 % 4 == 0) the resampled rows are written
+    straight into the concatenated buffer, and the gradient of ``other_bev`` is gathered straight out of the concatenated
+    gradient: the exact adjoint of the forward's index maps, summed in fp32 in torch's order (ascending y, then x) and
+    rounded once, in the dtype and memory format of ``other_bev``; no atomics.  ``None`` (default): ``other_bev`` must
+    already be (B, C2, Y, X).  Other modes raise ``ValueError``."""
+    if resize_other not in (None, 'nearest'):
+        raise ValueError(f"resize_other must be None or 'nearest' (got {resize_other!r})")
+    if other_bev.shape[0] != plan.batch:
+        raise ValueError(f'other_bev has batch {other_bev.shape[0]}, the plan {plan.batch}')
     C = context.shape[1]
-    fast = (plan.mode == 'runs' and runs_supported(C, depth.dtype) and depth.shape[3] % 4 == 0
-            and other_bev.shape[1] % 4 == 0 and depth.is_contiguous())
-    if bda_affine is None:
-        if fast:
-            return VoxelPoolingFusedConcat.apply(depth, context, other_bev, voxel_num, plan, None)
-        return torch.cat([voxel_pooling_fused(None, depth, context, voxel_num, plan), other_bev.to(depth.dtype)], dim=1)
-    from ..bev_augment import warp_affine, warp_theta
     X, Y, _ = plan.voxel_num
-    if bda_affine.shape[0] != plan.batch:
+    fast = (plan.mode == 'runs' and runs_supported(C, depth.dtype) and depth.shape[3] % 4 == 0
+            and _other_layout(other_bev) is not None and depth.is_contiguous())
+    resize = resize_other is not None
+    if bda_affine is not None and bda_affine.shape[0] != plan.batch:
         raise ValueError(f'bda_affine has {bda_affine.shape[0]} matrices for a batch of {plan.batch}')
     if fast:
-        theta = warp_theta(bda_affine, (Y, X), (Y, X)).to(depth.device)
-        return VoxelPoolingFusedConcat.apply(depth, context, other_bev, voxel_num, plan, theta)
-    pooled = voxel_pooling_fused(None, depth, context, voxel_num, plan)
-    return torch.cat([warp_affine(pooled, bda_affine, (Y, X)), other_bev.to(pooled.dtype)], dim=1)
+        theta = None
+        if bda_affine is not None:
+            from ..bev_augment import warp_theta
+            theta = warp_theta(bda_affine, (Y, X), (Y, X)).to(depth.device)
+        return VoxelPoolingFusedConcat.apply(depth, context, other_bev, voxel_num, plan, theta, resize)
+    camera = voxel_pooling_fused(None, depth, context, voxel_num, plan)
+    if bda_affine is not None:
+        from ..bev_augment import warp_affine
+        camera = warp_affine(camera, bda_affine, (Y, X))
+    if resize:
+        other_bev = torch.nn.functional.interpolate(other_bev, size=(Y, X), mode='nearest')
+    return torch.cat([camera, other_bev.to(camera.dtype)], dim=1)
 
 
 class VoxelPoolingFusedLogits(Function):
