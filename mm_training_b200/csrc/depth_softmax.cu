@@ -36,7 +36,7 @@ depth_softmax_kernel(const T *__restrict__ logits, int64_t logits_img_stride, co
       s = s * expf(m - l);
       m = l;
     }
-    s += expf(l - m);
+    s += (l == -INFINITY) ? 0.f : expf(l - m);             // a leading -inf (m still -inf) would add expf(NaN)
   }
   bool fg = false;
   const float *op = nullptr;

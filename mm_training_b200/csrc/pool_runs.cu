@@ -407,7 +407,7 @@ depth_stats_kernel(const float *__restrict__ logits, int64_t img_stride, int D, 
       s = s * expf(m - l);
       m = l;
     }
-    s += expf(l - m);
+    s += (l == -INFINITY) ? 0.f : expf(l - m);             // a leading -inf (m still -inf) would add expf(NaN)
   }
   stats[(int64_t)blockIdx.y * HW + pix] = make_float2(m, 1.0f / s);
 }

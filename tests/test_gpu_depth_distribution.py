@@ -1,11 +1,14 @@
 """GPU parity tests of the one-pass depth distribution (csrc/depth_softmax.cu, ops/depth_distribution.py) against
-the reference's torch ops restated verbatim (layers/backbones/lss_fpn.py:423,427-434).  Floating point: rtol 1e-5
-(+ atol 1e-7: a softmax output near 1e-10 carries no more than float32 ulps of its normaliser) in fp32, 1e-2 for
-fp16 / bf16 logits; the overwritten pixels must equal the oracle bit for bit."""
+the reference's torch ops restated verbatim (layers/backbones/lss_fpn.py:423,427-434): rtol 1e-5 (+ atol 1e-7) in
+fp32, 1e-2 for fp16 / bf16 logits; the overwritten pixels must equal the oracle bit for bit.  The half-precision test
+also holds the probabilities to the fp64 bound of oracle/depth_softmax_ref.py and the fp16 / bf16 gradients to the
+rounding bracket of the fp64 backward; tests/test_gpu_depth_softmax_edges.py does so at every shape, dtype and edge
+value (masked bins, underflow, non-finite rows)."""
 import pytest
 import torch
 
 from mm_training_b200.ops.depth_distribution import depth_distribution
+from oracle import depth_softmax_ref as ds
 
 pytestmark = pytest.mark.gpu
 DEV = 'cuda'
@@ -66,11 +69,17 @@ def test_forward_and_backward_match_the_reference_ops(shape, oracle):
 def test_half_precision_logits(dtype):
     feat, orc = _case(4, 112, 80, 16, 44, seed=3, dtype=dtype)
     a = feat.to(DEV).requires_grad_(True)
-    depth, used = depth_distribution(a, 112, orc.to(DEV))
-    rdepth, rused = _reference(feat.to(DEV).float(), 112, orc.to(DEV))
+    o = orc.to(DEV)
+    depth, used = depth_distribution(a, 112, o)
+    rdepth, rused = _reference(feat.to(DEV).float(), 112, o)
     assert torch.allclose(depth, rdepth, rtol=1e-2, atol=1e-6) and torch.allclose(used, rused, rtol=1e-2, atol=1e-6)
+    ref = ds.softmax_ref(a.detach(), 112)
+    assert bool(((depth.double() - ref).abs() <= ds.forward_rel_bound(a.detach(), 112) * ref + ds.FLT_MIN).all())
     used.sum().backward()
     assert a.grad.dtype == dtype and bool(torch.isfinite(a.grad).all())
+    gref, mag = ds.softmax_backward_ref(depth.detach(), None, torch.ones_like(used), o)
+    lo, hi = ds.round_bracket(gref, ds.sum_bound(112 + 3, mag), dtype)
+    assert bool(ds.in_bracket(a.grad[:, :112], lo, hi).all())
 
 
 def test_feeds_the_fused_pooling_without_a_copy():
