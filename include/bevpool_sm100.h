@@ -381,6 +381,29 @@ int bevdepth_softmax_backward(const float *prob, const float *grad_prob, const f
                               const float *oracle, int num_images, int depth_bins, int feat_h, int feat_w,
                               void *grad_logits, int dtype, void *stream);
 
+/* ---- depth loss: binary cross-entropy of the depth distribution against the LiDAR depth labels --------------------
+ * Replaces exps/mm_training_aim.py:163-176 (get_depth_loss): permute + contiguous copy of the predictions, max over D
+ * of the labels, two boolean-mask gathers, F.binary_cross_entropy, sum / max(1.0, fg.sum()) -- with no host sync.
+ *   prob     float32 (num_images, depth_bins, H, W) contiguous (what bevdepth_softmax_forward writes)
+ *   labels   float32 (num_images * H * W, depth_bins) rows, pixel r = (image * H + y) * W + x; OR
+ *   bins     int32 (num_images * H * W): bin b in [0, depth_bins) is the one-hot row of b, anything else a zero row
+ *            (bevlabel_depth_labels' `bins`).  Exactly one of labels / bins is non-NULL.  One-hot labels give the same
+ *            bits in both forms.
+ *   A pixel is foreground when the max of its label row is > 0 (a row holding a NaN is background, as in torch.max).
+ *   Per element, fp32 (torch's CUDA kernel): e = (t - 1) * max(log1p(-p), -100) - t * max(log(p), -100); per pixel the
+ *   fp32 sum in ascending bin order; over the foreground pixels an fp64 sum in a fixed order, rounded once to S.
+ * forward  loss[0] = fl(3 * fl(S / fl(max(cnt, 1)))), fg_count[0] = cnt (device scalars).  workspace:
+ *          bevdepth_loss_workspace_bytes() bytes, contents don't-care.  Bit-stable: no floating-point atomics.
+ * backward g' = fl(fl(grad_loss[0] * 3) / fl(max(fg_count[0], 1))) read on the device; grad_prob (same shape as prob)
+ *          = +0 + g' * (p - t) / max((1 - p) * p, 1e-12) on foreground pixels, +0 elsewhere; every element written.
+ * depth_bins <= 1536 (else BEVPOOL_E_CHANNELS); pointers 4-byte aligned, the workspace 8-byte (else BEVPOOL_E_ALIGN). */
+int bevdepth_loss_workspace_bytes(int num_images, int depth_bins, int feat_h, int feat_w, size_t *bytes);
+int bevdepth_loss_forward(const float *prob, const float *labels, const int32_t *bins, int num_images, int depth_bins,
+                          int feat_h, int feat_w, void *workspace, float *loss, int32_t *fg_count, void *stream);
+int bevdepth_loss_backward(const float *prob, const float *labels, const int32_t *bins, const float *grad_loss,
+                           const int32_t *fg_count, int num_images, int depth_bins, int feat_h, int feat_w,
+                           float *grad_prob, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -68,6 +68,9 @@ _SIGNATURES = {
     'pillar_scatter_backward': [_vp, _vp, _i64, _i, _i, _i, _i, _i, _i, _vp, _vp],
     'bevdepth_softmax_forward': [_vp, _i, _i64, _vp, _i, _i, _i, _i, _vp, _vp, _vp],
     'bevdepth_softmax_backward': [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _i, _vp],
+    'bevdepth_loss_workspace_bytes': [_i, _i, _i, _i, _szp],
+    'bevdepth_loss_forward': [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
+    'bevdepth_loss_backward': [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp],
     'bevlabel_scratch_bytes': [_i, _i, _i, _szp],
     'bevlabel_depth_labels': [_vp, _vp, _i, _i, _i, _i64, _vp, _vp, _vp, _i, _i, _i, ctypes.c_float, ctypes.c_float, _i,
                               _vp, _vp, _vp, _i, _vp],
