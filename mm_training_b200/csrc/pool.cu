@@ -626,9 +626,12 @@ static int fused_backward_t(const void *plan, const void *grad, const void *dept
   const int64_t cells = (int64_t)X * Y;
   if constexpr (std::is_same<T, float>::value) {
     if (g8_supported(C) && g8_enabled()) {
-      // run plans (pair records): column kernel (pool_bwd2.cu; needs W % 4 == 0); else tile kernel (pool_bwd.cu; C <= 96)
+      // run plans (pair records): column kernel (pool_bwd2.cu; needs W % 4 == 0); else tile kernel (pool_bwd.cu; C <= 96).
+      // BEVPOOL_BW_KERNEL=1 picks the tile kernel where it can run: NCHW context and strided gradient rows exist only on
+      // the column kernel
       static const int which = env_int("BEVPOOL_BW_KERNEL", 2);
-      if (runs && which == 2 && fused_backward_col_supported(C, W, dp, gd, pv.cell_of_point))
+      const bool col_only = nchw || (g_stride != 0 && g_stride != C);
+      if (runs && (which == 2 || col_only) && fused_backward_col_supported(C, W, dp, gd, pv.cell_of_point))
         return launch_fused_backward_col(pv.cell_of_point, pv.pair_rec, g, dp, cx, gd, gc, nchw, B, N, D, H, W, C, cells, s, g_stride);
       if (g_stride != 0 && g_stride != C) return BEVPOOL_E_ALIGN;     // strided gradient rows exist only on the column kernel
       if (!nchw && fused_backward_tile_supported(C))
