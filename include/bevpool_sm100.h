@@ -168,8 +168,9 @@ int bevpool_fused_forward_runs_nchw(const void *plan, const void *depth, const v
  * channels-last buffer (B, Y, X, C_total).  out_rows = address of the first camera channel of cell 0; consecutive
  * cells are out_row_stride floats apart (>= channels, multiple of 4); the other channels of a row are not touched.  */
 #define BEVPOOL_FWD_NCHW_CONTEXT   1   /* context is (B*N, C, H, W); else pixel rows (B*N, H, W, C)                    */
-#define BEVPOOL_FWD_OUT_PREZEROED  2   /* the caller zero-filled the output rows (e.g. on a side stream while the plan  */
-                                       /* was being built): the kernels write occupied cells only                     */
+#define BEVPOOL_FWD_OUT_PREZEROED  2   /* the kernels write the rows of occupied cells only and leave the others as    */
+                                       /* they are: for output rows the caller zero-filled (e.g. on a side stream      */
+                                       /* while the plan was being built) or whose empty cells are never read          */
 int bevpool_fused_forward_runs_into(const void *plan, const void *depth, const void *context, int flags,
                                     void *out_rows, int64_t out_row_stride, int dtype, int batch, int num_cams,
                                     int depth_bins, int feat_h, int feat_w, int channels, int num_voxel_x,

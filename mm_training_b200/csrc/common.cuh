@@ -4,6 +4,7 @@
 #include <cuda_fp16.h>
 #include <cuda_bf16.h>
 #include <stdint.h>
+#include <cstdlib>
 
 #include "../../include/bevpool_sm100.h"
 
@@ -225,6 +226,26 @@ inline int check_plan_dims(int batch, int64_t num_points, int X, int Y) {
   if ((int64_t)batch * num_points >= (int64_t)INT32_MAX) return BEVPOOL_E_RANGE;
   if ((int64_t)batch * X * Y >= (int64_t)INT32_MAX) return BEVPOOL_E_RANGE;
   return BEVPOOL_OK;
+}
+// the fused entry points: the frustum (num_cams, D, H, W) of every sample, and the plan it implies
+inline int check_frustum_dims(int batch, int num_cams, int D, int H, int W, int X, int Y) {
+  if (num_cams <= 0 || D <= 0 || H <= 0 || W <= 0) return BEVPOOL_E_ARG;
+  return check_plan_dims(batch, (int64_t)num_cams * D * H * W, X, Y);
+}
+
+// tuning knobs for experiments; each caller keeps the value in a static, so a knob is read once per process
+inline int env_int(const char *name, int dflt) {
+  const char *e = std::getenv(name);
+  return e && e[0] ? std::atoi(e) : dflt;
+}
+
+inline int sm_count() {                     // per device (a process may drive several GPUs)
+  int dev = 0, n = 0;
+  static int cached[64] = {0};
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return kSMs;
+  if (cached[dev] == 0)
+    cached[dev] = (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) ? n : kSMs;
+  return cached[dev];
 }
 
 }  // namespace bevpool

@@ -21,11 +21,6 @@
 
 namespace bevpool {
 
-static int env_int(const char *name, int dflt) {   // tuning knobs for experiments
-  const char *e = std::getenv(name);
-  return e && e[0] ? std::atoi(e) : dflt;
-}
-
 // BEVPOOL_DISABLE_G8=1 forces the generic float4-per-lane kernels (used by the tests to cover both paths)
 static bool g8_enabled() {
   const char *e = std::getenv("BEVPOOL_DISABLE_G8");
@@ -513,14 +508,6 @@ transpose_kernel(const T *__restrict__ in, T *__restrict__ out, int64_t R, int64
 }
 
 // ---- launchers ----------------------------------------------------------------------------
-static int sm_count() {                     // per device (a process may drive several GPUs)
-  int dev = 0, n = 0;
-  static int cached[64] = {0};
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return kSMs;
-  if (cached[dev] == 0)
-    cached[dev] = (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) ? n : kSMs;
-  return cached[dev];
-}
 static size_t forward_workspace_bytes(int C) {
   // head + tail partial rows of every slice of the largest grid the forward may launch
   return (size_t)2 * 4 * kFwWarpsPerCta * kFwMaxCtasPerSm * sm_count() * (size_t)C * sizeof(float);
@@ -612,33 +599,21 @@ static int fused_forward_t(const void *plan, const void *depth, const void *ctx,
   return launch_forward<T, true>(pv, static_cast<const T *>(ctx), static_cast<const T *>(depth),
                                  static_cast<T *>(out), ws, (int64_t)B * X * Y, C, D * H * W, H * W, s);
 }
+// pixel-row context on any plan: tile kernel (pool_bwd.cu; fp32, C <= 96), else the generic kernel
 template <typename T>
 static int fused_backward_t(const void *plan, const void *grad, const void *depth, const void *ctx,
                             void *gdepth, void *gctx, int B, int N, int D, int H, int W, int C, int X,
-                            int Y, cudaStream_t s, bool nchw = false, bool runs = false, int64_t g_stride = 0) {
+                            int Y, cudaStream_t s) {
   const int64_t Np = (int64_t)N * D * H * W;
   const PlanView pv = plan_view(plan, B, Np, X, Y);
   const int C4 = C >> 2;
-  (void)nchw;
-  (void)runs;
   const T *g = static_cast<const T *>(grad), *dp = static_cast<const T *>(depth), *cx = static_cast<const T *>(ctx);
   T *gd = static_cast<T *>(gdepth), *gc = static_cast<T *>(gctx);
   const int64_t cells = (int64_t)X * Y;
   if constexpr (std::is_same<T, float>::value) {
-    if (g8_supported(C) && g8_enabled()) {
-      // run plans (pair records): column kernel (pool_bwd2.cu; needs W % 4 == 0); else tile kernel (pool_bwd.cu; C <= 96).
-      // BEVPOOL_BW_KERNEL=1 picks the tile kernel where it can run: NCHW context and strided gradient rows exist only on
-      // the column kernel
-      static const int which = env_int("BEVPOOL_BW_KERNEL", 2);
-      const bool col_only = nchw || (g_stride != 0 && g_stride != C);
-      if (runs && (which == 2 || col_only) && fused_backward_col_supported(C, W, dp, gd, pv.cell_of_point))
-        return launch_fused_backward_col(pv.cell_of_point, pv.pair_rec, g, dp, cx, gd, gc, nchw, B, N, D, H, W, C, cells, s, g_stride);
-      if (g_stride != 0 && g_stride != C) return BEVPOOL_E_ALIGN;     // strided gradient rows exist only on the column kernel
-      if (!nchw && fused_backward_tile_supported(C))
-        return launch_fused_backward_tile(pv.cell_of_point, g, dp, cx, gd, gc, B, N, D, H, W, C, cells, s);
-    }
+    if (g8_supported(C) && g8_enabled() && fused_backward_tile_supported(C))
+      return launch_fused_backward_tile(pv.cell_of_point, g, dp, cx, gd, gc, B, N, D, H, W, C, cells, s);
   }
-  if (nchw) return BEVPOOL_E_CHANNELS;      // the NCHW layout exists only on the column kernel
   if (C4 <= 32) return launch_fused_backward_cpl<T, 1>(pv, g, dp, cx, gd, gc, B, N, D, H, W, C, cells, s);
   if (C4 <= 64) return launch_fused_backward_cpl<T, 2>(pv, g, dp, cx, gd, gc, B, N, D, H, W, C, cells, s);
   return launch_fused_backward_cpl<T, 4>(pv, g, dp, cx, gd, gc, B, N, D, H, W, C, cells, s);
@@ -690,9 +665,7 @@ extern "C" int bevpool_fused_forward(const void *plan, const void *depth, const 
                                      void *out_nhwc, int dtype, int batch, int num_cams, int depth_bins,
                                      int feat_h, int feat_w, int channels, int X, int Y, void *workspace,
                                      void *stream) {
-  if (num_cams <= 0 || depth_bins <= 0 || feat_h <= 0 || feat_w <= 0) return BEVPOOL_E_ARG;
-  const int64_t np = (int64_t)num_cams * depth_bins * feat_h * feat_w;
-  int rc = check_plan_dims(batch, np, X, Y);
+  int rc = check_frustum_dims(batch, num_cams, depth_bins, feat_h, feat_w, X, Y);
   if (rc) return rc;
   if ((rc = check_channels(channels))) return rc;
   if (!plan || !depth || !context_nhwc || !out_nhwc) return BEVPOOL_E_ARG;
@@ -705,9 +678,7 @@ extern "C" int bevpool_fused_backward(const void *plan, const void *grad_out_nhw
                                       const void *context_nhwc, void *grad_depth, void *grad_context_nhwc,
                                       int dtype, int batch, int num_cams, int depth_bins, int feat_h,
                                       int feat_w, int channels, int X, int Y, void *stream) {
-  if (num_cams <= 0 || depth_bins <= 0 || feat_h <= 0 || feat_w <= 0) return BEVPOOL_E_ARG;
-  const int64_t np = (int64_t)num_cams * depth_bins * feat_h * feat_w;
-  int rc = check_plan_dims(batch, np, X, Y);
+  int rc = check_frustum_dims(batch, num_cams, depth_bins, feat_h, feat_w, X, Y);
   if (rc) return rc;
   if ((rc = check_channels(channels))) return rc;
   if (!plan || !grad_out_nhwc || !depth || !context_nhwc || !grad_depth || !grad_context_nhwc) return BEVPOOL_E_ARG;
@@ -716,44 +687,58 @@ extern "C" int bevpool_fused_backward(const void *plan, const void *grad_out_nhw
   BEVPOOL_DISPATCH_DTYPE(dtype, (fused_backward_t<T>(plan, grad_out_nhwc, depth, context_nhwc, grad_depth, grad_context_nhwc, batch, num_cams, depth_bins, feat_h, feat_w, channels, X, Y, s)));
 }
 
-extern "C" int bevpool_fused_backward_runs(const void *plan, const void *grad_out_nhwc, const void *depth,
-                                           const void *context, void *grad_depth, void *grad_context,
-                                           int context_is_nchw, int dtype, int batch, int num_cams, int depth_bins,
-                                           int feat_h, int feat_w, int channels, int X, int Y, void *stream) {
-  if (num_cams <= 0 || depth_bins <= 0 || feat_h <= 0 || feat_w <= 0) return BEVPOOL_E_ARG;
-  const int64_t np = (int64_t)num_cams * depth_bins * feat_h * feat_w;
-  int rc = check_plan_dims(batch, np, X, Y);
-  if (rc) return rc;
-  if (dtype != BEVPOOL_F32) return BEVPOOL_E_DTYPE;
-  if (!g8_supported(channels)) return BEVPOOL_E_CHANNELS;
-  if (!plan || !grad_out_nhwc || !depth || !context || !grad_depth || !grad_context) return BEVPOOL_E_ARG;
-  if (!aligned16(grad_out_nhwc) || !aligned16(context) || !aligned16(grad_context)) return BEVPOOL_E_ALIGN;
-  if (context_is_nchw && ((feat_w % 4) != 0 || !aligned16(depth) || !aligned16(grad_depth))) return BEVPOOL_E_ALIGN;
-  return fused_backward_t<float>(plan, grad_out_nhwc, depth, context, grad_depth, grad_context, batch, num_cams,
-                                 depth_bins, feat_h, feat_w, channels, X, Y, static_cast<cudaStream_t>(stream),
-                                 context_is_nchw != 0, true);
-}
-
-// gradient rows inside a wider channels-last buffer (the gradient of a concatenated BEV feature map): row of cell c
-// starts at grad_rows + c * grad_row_stride floats
-extern "C" int bevpool_fused_backward_runs_from(const void *plan, const void *grad_rows, int64_t grad_row_stride,
-                                                const void *depth, const void *context, void *grad_depth,
-                                                void *grad_context, int context_is_nchw, int dtype, int batch,
-                                                int num_cams, int depth_bins, int feat_h, int feat_w, int channels,
-                                                int X, int Y, void *stream) {
-  if (num_cams <= 0 || depth_bins <= 0 || feat_h <= 0 || feat_w <= 0) return BEVPOOL_E_ARG;
-  const int64_t np = (int64_t)num_cams * depth_bins * feat_h * feat_w;
-  int rc = check_plan_dims(batch, np, X, Y);
+// The run-plan backward behind both entry points below: the gradient row of cell c starts at grad_rows + c * grad_row_stride
+// floats.  col_args: the entry point takes only what the column kernel reads (W % 4 == 0, 16-byte aligned depth and
+// grad_depth) whatever the layout.  Column kernel (pool_bwd2.cu; pair records); BEVPOOL_BW_KERNEL=1 picks the pixel-row
+// kernels where they can run: NCHW context and strided gradient rows exist only on the column kernel.
+static int fused_backward_runs(const void *plan, const void *grad_rows, int64_t grad_row_stride, const void *depth,
+                               const void *context, void *grad_depth, void *grad_context, bool nchw, bool col_args,
+                               int dtype, int batch, int num_cams, int depth_bins, int feat_h, int feat_w, int channels,
+                               int X, int Y, void *stream) {
+  int rc = check_frustum_dims(batch, num_cams, depth_bins, feat_h, feat_w, X, Y);
   if (rc) return rc;
   if (dtype != BEVPOOL_F32) return BEVPOOL_E_DTYPE;
   if (!g8_supported(channels)) return BEVPOOL_E_CHANNELS;
   if (!plan || !grad_rows || !depth || !context || !grad_depth || !grad_context) return BEVPOOL_E_ARG;
   if (grad_row_stride < channels || (grad_row_stride % 4) != 0) return BEVPOOL_E_ARG;
   if (!aligned16(grad_rows) || !aligned16(context) || !aligned16(grad_context)) return BEVPOOL_E_ALIGN;
-  if ((feat_w % 4) != 0 || !aligned16(depth) || !aligned16(grad_depth)) return BEVPOOL_E_ALIGN;
-  return fused_backward_t<float>(plan, grad_rows, depth, context, grad_depth, grad_context, batch, num_cams,
-                                 depth_bins, feat_h, feat_w, channels, X, Y, static_cast<cudaStream_t>(stream),
-                                 context_is_nchw != 0, true, grad_row_stride);
+  if ((nchw || col_args) && ((feat_w % 4) != 0 || !aligned16(depth) || !aligned16(grad_depth))) return BEVPOOL_E_ALIGN;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const PlanView pv = plan_view(plan, batch, (int64_t)num_cams * depth_bins * feat_h * feat_w, X, Y);
+  const float *dp = static_cast<const float *>(depth);
+  float *gd = static_cast<float *>(grad_depth);
+  const bool strided = grad_row_stride != channels;
+  if (g8_enabled()) {
+    static const int which = env_int("BEVPOOL_BW_KERNEL", 2);
+    if ((which == 2 || nchw || strided) && fused_backward_col_supported(channels, feat_w, dp, gd, pv.cell_of_point))
+      return launch_fused_backward_col(pv.cell_of_point, pv.pair_rec, static_cast<const float *>(grad_rows), dp,
+                                       static_cast<const float *>(context), gd, static_cast<float *>(grad_context), nchw,
+                                       batch, num_cams, depth_bins, feat_h, feat_w, channels, (int64_t)X * Y, s,
+                                       grad_row_stride);
+    if (strided) return BEVPOOL_E_ALIGN;
+  }
+  if (nchw) return BEVPOOL_E_CHANNELS;
+  return fused_backward_t<float>(plan, grad_rows, depth, context, grad_depth, grad_context, batch, num_cams, depth_bins,
+                                 feat_h, feat_w, channels, X, Y, s);
+}
+
+extern "C" int bevpool_fused_backward_runs(const void *plan, const void *grad_out_nhwc, const void *depth,
+                                           const void *context, void *grad_depth, void *grad_context,
+                                           int context_is_nchw, int dtype, int batch, int num_cams, int depth_bins,
+                                           int feat_h, int feat_w, int channels, int X, int Y, void *stream) {
+  return fused_backward_runs(plan, grad_out_nhwc, channels, depth, context, grad_depth, grad_context, context_is_nchw != 0,
+                             false, dtype, batch, num_cams, depth_bins, feat_h, feat_w, channels, X, Y, stream);
+}
+
+// gradient rows inside a wider channels-last buffer (the gradient of a concatenated BEV feature map)
+extern "C" int bevpool_fused_backward_runs_from(const void *plan, const void *grad_rows, int64_t grad_row_stride,
+                                                const void *depth, const void *context, void *grad_depth,
+                                                void *grad_context, int context_is_nchw, int dtype, int batch,
+                                                int num_cams, int depth_bins, int feat_h, int feat_w, int channels,
+                                                int X, int Y, void *stream) {
+  return fused_backward_runs(plan, grad_rows, grad_row_stride, depth, context, grad_depth, grad_context,
+                             context_is_nchw != 0, true, dtype, batch, num_cams, depth_bins, feat_h, feat_w, channels, X,
+                             Y, stream);
 }
 
 extern "C" int bevpool_grad_rows(const void *plan, const void *grad_out_nchw, void *rows_nhwc, int dtype,

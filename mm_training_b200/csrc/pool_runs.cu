@@ -25,14 +25,7 @@
 #include "pool_g8.cuh"
 #include "tma.cuh"
 
-#include <cstdlib>
-
 namespace bevpool {
-
-static int env_int_runs(const char *name, int dflt) {
-  const char *e = std::getenv(name);
-  return e && e[0] ? std::atoi(e) : dflt;
-}
 
 constexpr int kRaTW = 4;                     // image columns per CTA = warps per CTA = one 16-byte depth segment
 constexpr int kRaDC = 16;                    // depth bins per staged chunk: 4 groups x 4 bins per warp
@@ -439,15 +432,6 @@ static int launch_stage_a(const CUtensorMap &ctx_map, const PlanView &pv, const 
   return BEVPOOL_OK;
 }
 
-static int sm_count_runs() {
-  int dev = 0, n = 0;
-  static int cached[64] = {0};
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return kSMs;
-  if (cached[dev] == 0)
-    cached[dev] = (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) ? n : kSMs;
-  return cached[dev];
-}
-
 // tuning knobs, read once per process (defaults = the measured best; scripts/README.md)
 struct RunKnobs {
   int chunk, fill, hints, cps_b, d_split;
@@ -455,12 +439,12 @@ struct RunKnobs {
 static const RunKnobs &run_knobs() {
   static const RunKnobs k = [] {
     RunKnobs r;
-    r.chunk = env_int_runs("BEVPOOL_RUN_CHUNK", 0);            // frames per (stage A, stage B) pair; 0 = all
-    r.fill = env_int_runs("BEVPOOL_RUN_FILL", 1) != 0;         // 0: stage B fills the empty cells itself
-    r.hints = env_int_runs("BEVPOOL_RUN_HINTS", 1) != 0;       // L2 eviction-priority hints on the fill / run-row stores
-    r.cps_b = env_int_runs("BEVPOOL_RUN_CPSB", 5);             // stage B CTAs per SM (4 warps each)
+    r.chunk = env_int("BEVPOOL_RUN_CHUNK", 0);            // frames per (stage A, stage B) pair; 0 = all
+    r.fill = env_int("BEVPOOL_RUN_FILL", 1) != 0;         // 0: stage B fills the empty cells itself
+    r.hints = env_int("BEVPOOL_RUN_HINTS", 1) != 0;       // L2 eviction-priority hints on the fill / run-row stores
+    r.cps_b = env_int("BEVPOOL_RUN_CPSB", 5);             // stage B CTAs per SM (4 warps each)
     r.cps_b = r.cps_b < 1 ? 1 : (r.cps_b > kFwMaxCtasPerSm - 1 ? kFwMaxCtasPerSm - 1 : r.cps_b);
-    r.d_split = env_int_runs("BEVPOOL_RUN_DSPLIT", 0);
+    r.d_split = env_int("BEVPOOL_RUN_DSPLIT", 0);
     return r;
   }();
   return k;
@@ -476,10 +460,9 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
   if (stats && !nchw) return BEVPOOL_E_ARG;                   // the logits entry point exists for the NCHW layout only
   if (dep_img_stride != 0 && ((dep_img_stride % 4) != 0 || dep_img_stride < (int64_t)depth_bins * feat_h * feat_w)) return BEVPOOL_E_ARG;
   if (out_stride < channels || (out_stride % 4) != 0) return BEVPOOL_E_ARG;
-  if (num_cams <= 0 || depth_bins <= 0 || feat_h <= 0 || feat_w <= 0) return BEVPOOL_E_ARG;
-  const int64_t np = (int64_t)num_cams * depth_bins * feat_h * feat_w;
-  int rc = check_plan_dims(batch, np, X, Y);
+  int rc = check_frustum_dims(batch, num_cams, depth_bins, feat_h, feat_w, X, Y);
   if (rc) return rc;
+  const int64_t np = (int64_t)num_cams * depth_bins * feat_h * feat_w;
   if (dtype != BEVPOOL_F32) return BEVPOOL_E_DTYPE;
   if (!g8_supported(channels)) return BEVPOOL_E_CHANNELS;
   if (!plan || !depth || !context || !out_nhwc || !run_rows || !workspace || run_rows_capacity <= 0) return BEVPOOL_E_ARG;
@@ -512,7 +495,7 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
     const int64_t tiles = (int64_t)nb * num_cams * ceil_div64(feat_w, kRaTW) * ceil_div64(feat_h, kRunHB);
     int d_split = kn.d_split;
     if (d_split <= 0) {
-      d_split = (int)ceil_div64((int64_t)16 * sm_count_runs(), tiles);
+      d_split = (int)ceil_div64((int64_t)16 * sm_count(), tiles);
       const int max_split = (int)ceil_div64(depth_bins, kRaDC);
       d_split = d_split < 1 ? 1 : (d_split > max_split ? max_split : d_split);
     }
@@ -530,7 +513,7 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
     if (rc) return rc;
     // stage B: even-share segmented sum of the run rows (identity ids), fill CTAs only if stage A did not fill
     const int period_b = (fill || prezeroed) ? 0 : cps_b + 1;
-    const unsigned ctas_b = (unsigned)(sm_count_runs() * (period_b ? period_b : cps_b));
+    const unsigned ctas_b = (unsigned)(sm_count() * (period_b ? period_b : cps_b));
     const int slices = (int)(period_b ? ctas_b - ctas_b / period_b : ctas_b) * kFwWarpsPerCta * 4;
     float *ws_head = static_cast<float *>(workspace);
     float *ws_tail = ws_head + (size_t)slices * channels;

@@ -18,7 +18,7 @@ import torch
 from torch.autograd import Function
 
 from .. import _lib
-from .voxel_pooling.voxel_pooling import _transpose
+from .voxel_pooling.voxel_pooling import _strided_rows, _transpose
 
 
 def _normal_transform_pixel(h: int, w: int, like: torch.Tensor) -> torch.Tensor:
@@ -51,24 +51,12 @@ def warp_theta(M: torch.Tensor, src_hw: Sequence[int], dsize: Sequence[int]) -> 
     return theta.float().contiguous()
 
 
-def _strided_rows(x: torch.Tensor):
-    """(B, C, H, W) view of channels-last rows -> (base tensor, row stride in floats), or None.  Zero-copy for the
-    output of the pooling ops and for a channel slice of a concatenated channels-last buffer."""
-    B, C, H, W = x.shape
-    s = x.stride()
-    S = s[3]
-    if (s[1] == 1 and S >= C and S % 4 == 0 and s[2] == W * S and (B == 1 or s[0] == H * W * S)
-            and x.data_ptr() % 16 == 0):
-        return x, S
-    return None
-
-
 def _rows(x: torch.Tensor):
     """(B, C, H, W) float32 -> (tensor whose data_ptr is the first row, row stride): zero-copy when ``x`` already is
     channels-last rows, else one tiled transpose of an NCHW copy."""
-    r = _strided_rows(x)
-    if r is not None:
-        return r
+    S = _strided_rows(x)
+    if S is not None:
+        return x, S
     B, C, H, W = x.shape
     return _transpose(x.contiguous(), B, C, H * W), C
 

@@ -235,6 +235,18 @@ def _transpose(x: torch.Tensor, batch: int, rows: int, cols: int) -> torch.Tenso
     return out
 
 
+def _strided_rows(x: torch.Tensor) -> Optional[int]:
+    """(B, C, H, W) view of channels-last rows -> the row stride in elements, or None.  Zero-copy for the output of the
+    pooling ops and for a channel slice of a concatenated channels-last buffer."""
+    B, C, H, W = x.shape
+    s = x.stride()
+    S = s[3]
+    if (s[1] == 1 and S >= C and S % 4 == 0 and s[2] == W * S and (B == 1 or s[0] == H * W * S)
+            and x.data_ptr() % 16 == 0):
+        return S
+    return None
+
+
 def _grad_rows_nhwc(grad_out: torch.Tensor, plan: PoolingPlan) -> torch.Tensor:
     """grad_out arrives as (B, C, Y, X) with arbitrary strides; the kernels want (B, Y, X, C) rows.
     Zero-copy when it already is a permuted NHWC buffer (what autograd hands back for the
@@ -261,6 +273,14 @@ def _forward_workspace(channels: int, device) -> torch.Tensor:
     _lib.check(_lib.lib().bevpool_forward_workspace_bytes(channels, ctypes.byref(nbytes)),
                'bevpool_forward_workspace_bytes')
     return torch.empty(nbytes.value, dtype=torch.uint8, device=device)
+
+
+def _run_scratch(plan: PoolingPlan, channels: int, device):
+    """Scratch of a run-plan forward: ``(run_rows, capacity, workspace)`` -- one float32 row per run (sized by the plan's
+    run count or its ``max_runs`` hint) and the workspace of stage B."""
+    cap = max(1, plan.num_sorted)
+    run_rows = torch.empty(cap, channels, dtype=torch.float32, device=device)
+    return run_rows, cap, _forward_workspace(channels, device)
 
 
 def pool_forward(plan: PoolingPlan, input_features: torch.Tensor) -> torch.Tensor:
@@ -300,20 +320,33 @@ def context_rows_nhwc(context: torch.Tensor) -> torch.Tensor:
     return rows
 
 
-def _nchw_direct(context: torch.Tensor, depth: torch.Tensor) -> bool:
+def _nchw_direct(context: torch.Tensor, depth: torch.Tensor, channels: Optional[int] = None) -> bool:
     """NCHW-contiguous fp32 context whose rows are multiples of 16 bytes: the kernels read it through a TMA
-    tensor map, no layout pass."""
+    tensor map, no layout pass.  ``channels``: C, when ``context`` holds more channels (DepthNet's output)."""
+    C = context.shape[1] if channels is None else channels
     return (context.is_contiguous() and context.dtype == torch.float32 and context.shape[3] % 4 == 0
-            and context.shape[1] in RUN_CHANNELS and context.data_ptr() % 16 == 0 and depth.data_ptr() % 16 == 0
-            and os.environ.get('BEVPOOL_DISABLE_G8', '0') != '1' and os.environ.get('BEVPOOL_NCHW_DIRECT', '1') != '0')
+            and runs_supported(C, context.dtype) and context.data_ptr() % 16 == 0 and depth.data_ptr() % 16 == 0
+            and os.environ.get('BEVPOOL_NCHW_DIRECT', '1') != '0')
+
+
+def _route(plan_mode: str, context: torch.Tensor, depth: torch.Tensor, context_rows: Optional[torch.Tensor] = None,
+           channels: Optional[int] = None) -> str:
+    """The kernels that pool ``context`` on a plan of ``plan_mode``: 'nchw' (run plan, ``_nchw_direct``), 'rows' (run
+    plan; pixel rows, ``context_rows`` or ``context_rows_nhwc(context)``) or 'points' (point plan, or no run kernel for
+    the dtype / channel count)."""
+    if plan_mode != 'runs' or not runs_supported(context.shape[1] if channels is None else channels, depth.dtype):
+        return 'points'
+    return 'nchw' if context_rows is None and _nchw_direct(context, depth, channels) else 'rows'
 
 
 def fused_forward(plan: PoolingPlan, depth: torch.Tensor, context: torch.Tensor,
                   context_rows: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None,
                   prezeroed: bool = False) -> torch.Tensor:
     """depth (B*N, D, H, W), context (B*N, C, H, W) NCHW or channels_last -> (B, Y, X, C).  ``out``: a caller-provided
-    (B, Y, X, C) buffer; ``prezeroed``: it already holds zeros (run plans only: the kernels then write occupied cells
-    only -- see ``fused_forward_cold``)."""
+    (B, Y, X, C) buffer; on a run plan also rows at a uniform cell stride, such as ``buf[..., :C]`` of a wider
+    channels-last ``buf``.  ``prezeroed`` (run plans): the kernels write the rows of occupied cells only and leave the
+    others as they are -- for an ``out`` that already holds zeros (``fused_forward_cold``) or whose empty cells are never
+    read (the BDA warp's scratch).  A point plan writes every cell either way."""
     BN, D, H, W = depth.shape
     C = context.shape[1]
     X, Y, _ = plan.voxel_num
@@ -321,31 +354,33 @@ def fused_forward(plan: PoolingPlan, depth: torch.Tensor, context: torch.Tensor,
     N = BN // B
     assert context.shape == (BN, C, H, W) and depth.dtype == context.dtype
     assert B * N == BN and plan.num_points == N * D * H * W
+    route = _route(plan.mode, context, depth, context_rows)
     with torch.cuda.device(depth.device):
         if out is None:
-            out = torch.empty(B, Y, X, C, dtype=depth.dtype, device=depth.device)
-            prezeroed = False
-        assert out.shape == (B, Y, X, C) and out.is_contiguous() and out.dtype == depth.dtype
-        if plan.mode == 'runs':
-            if not runs_supported(C, depth.dtype):
+            out, prezeroed = torch.empty(B, Y, X, C, dtype=depth.dtype, device=depth.device), False
+        assert out.shape == (B, Y, X, C) and out.dtype == depth.dtype
+        stride = C if out.is_contiguous() else _strided_rows(out.permute(0, 3, 1, 2))
+        assert stride is not None, 'out must be (B, Y, X, C) rows at a uniform cell stride'
+        if route == 'points':
+            if plan.mode == 'runs':
                 raise ValueError(f'run plans need float32 and C in {RUN_CHANNELS}; build a point plan for C={C}, {depth.dtype}')
-            assert plan.frustum == (N, D, H, W)
-            cap = max(1, plan.num_sorted)
-            run_rows = torch.empty(cap, C, dtype=torch.float32, device=depth.device)
+            if stride != C:
+                raise ValueError('a point plan writes packed (B, Y, X, C) rows: out must be contiguous')
+            ctx_nhwc = context_rows_nhwc(context) if context_rows is None else context_rows
             ws = _forward_workspace(C, out.device)
-            nchw = context_rows is None and _nchw_direct(context, depth)
-            ctx_arg = context if nchw else (context_rows_nhwc(context) if context_rows is None else context_rows)
-            _lib.check(_lib.lib().bevpool_fused_forward_runs_into(
-                plan.ptr, depth.data_ptr(), ctx_arg.data_ptr(), (1 if nchw else 0) | (2 if prezeroed else 0), out.data_ptr(), C,
-                _lib.dtype_code(depth), B, N, D, H, W, C, X, Y, run_rows.data_ptr(), cap, ws.data_ptr(),
-                _lib.stream_ptr(depth.device)), 'bevpool_fused_forward_runs_into')
+            _lib.check(_lib.lib().bevpool_fused_forward(plan.ptr, depth.data_ptr(), ctx_nhwc.data_ptr(),
+                                                        out.data_ptr(), _lib.dtype_code(depth), B, N, D, H, W,
+                                                        C, X, Y, ws.data_ptr(), _lib.stream_ptr(depth.device)),
+                       'bevpool_fused_forward')
             return out
-        ctx_nhwc = context_rows_nhwc(context) if context_rows is None else context_rows
-        ws = _forward_workspace(C, out.device)
-        _lib.check(_lib.lib().bevpool_fused_forward(plan.ptr, depth.data_ptr(), ctx_nhwc.data_ptr(),
-                                                    out.data_ptr(), _lib.dtype_code(depth), B, N, D, H, W,
-                                                    C, X, Y, ws.data_ptr(), _lib.stream_ptr(depth.device)),
-                   'bevpool_fused_forward')
+        assert plan.frustum == (N, D, H, W)
+        run_rows, cap, ws = _run_scratch(plan, C, depth.device)
+        nchw = route == 'nchw'
+        ctx_arg = context if nchw else (context_rows_nhwc(context) if context_rows is None else context_rows)
+        _lib.check(_lib.lib().bevpool_fused_forward_runs_into(
+            plan.ptr, depth.data_ptr(), ctx_arg.data_ptr(), (1 if nchw else 0) | (2 if prezeroed else 0), out.data_ptr(),
+            stride, _lib.dtype_code(depth), B, N, D, H, W, C, X, Y, run_rows.data_ptr(), cap, ws.data_ptr(),
+            _lib.stream_ptr(depth.device)), 'bevpool_fused_forward_runs_into')
     return out
 
 
@@ -381,50 +416,54 @@ def fused_forward_cold(make_plan, batch: int, voxel_num: VoxelNum, depth: torch.
             out.zero_()
         plan = make_plan()
         cur.wait_stream(side)          # (every later use of `out`, its free included, is ordered behind this join)
-        if plan.mode != 'runs':
-            return plan, fused_forward(plan, depth, context, out=out)
         return plan, fused_forward(plan, depth, context, out=out, prezeroed=True)
 
 
-def fused_backward(plan: PoolingPlan, grad_output: torch.Tensor, depth: torch.Tensor,
-                   context: torch.Tensor, context_rows: Optional[torch.Tensor] = None):
-    """grad_output (B, C, Y, X), any strides -> (grad_depth, grad_context).  grad_context has the
-    memory format of ``context``: channels_last in -> channels_last out (zero-copy), NCHW in ->
-    NCHW out (written NCHW by the kernel through a TMA tensor map; one tiled transpose on the generic path)."""
+def _fused_backward_rows(plan: PoolingPlan, route: str, grad_rows: torch.Tensor, row_stride: Optional[int],
+                         depth: torch.Tensor, context: torch.Tensor, context_rows: Optional[torch.Tensor]):
+    """Fused backward on ``route`` (``_route``) -> (grad_depth, grad_context).  ``row_stride`` None: ``grad_rows`` are
+    packed (B, Y, X, C) rows (``_grad_rows_nhwc``); else the row of cell c starts ``c * row_stride`` floats after the
+    first (run plans with W % 4 == 0 only).  grad_context has the memory format of ``context``: channels_last in ->
+    channels_last out (zero-copy), NCHW in -> NCHW out (written NCHW on the 'nchw' route, else one tiled transpose)."""
     BN, D, H, W = depth.shape
     C = context.shape[1]
     X, Y, _ = plan.voxel_num
     B = plan.batch
     N = BN // B
+    nchw = route == 'nchw'
+    assert row_stride is None or route != 'points'
+    grad_depth = torch.empty_like(depth)
+    if nchw:
+        ctx_arg, grad_ctx_arg = context, torch.empty_like(context)
+    else:
+        ctx_arg = context_rows_nhwc(context) if context_rows is None else context_rows
+        grad_ctx_arg = torch.empty(BN, H, W, C, dtype=context.dtype, device=context.device)
+    args = (depth.data_ptr(), ctx_arg.data_ptr(), grad_depth.data_ptr(), grad_ctx_arg.data_ptr())
+    dims = (_lib.dtype_code(depth), B, N, D, H, W, C, X, Y, _lib.stream_ptr(depth.device))
+    L = _lib.lib()
+    if route == 'points':
+        _lib.check(L.bevpool_fused_backward(plan.ptr, grad_rows.data_ptr(), *args, *dims), 'bevpool_fused_backward')
+    elif row_stride is None:
+        _lib.check(L.bevpool_fused_backward_runs(plan.ptr, grad_rows.data_ptr(), *args, int(nchw), *dims),
+                   'bevpool_fused_backward_runs')
+    else:
+        _lib.check(L.bevpool_fused_backward_runs_from(plan.ptr, grad_rows.data_ptr(), row_stride, *args, int(nchw), *dims),
+                   'bevpool_fused_backward_runs_from')
+    if nchw:
+        return grad_depth, grad_ctx_arg
+    if context.permute(0, 2, 3, 1).is_contiguous():
+        return grad_depth, grad_ctx_arg.permute(0, 3, 1, 2)
+    return grad_depth, _transpose(grad_ctx_arg, BN, H * W, C).view(BN, C, H, W)
+
+
+def fused_backward(plan: PoolingPlan, grad_output: torch.Tensor, depth: torch.Tensor,
+                   context: torch.Tensor, context_rows: Optional[torch.Tensor] = None):
+    """grad_output (B, C, Y, X), any strides -> (grad_depth, grad_context) in the memory format of ``context``
+    (``_fused_backward_rows``)."""
     with torch.cuda.device(depth.device):
         rows = _grad_rows_nhwc(grad_output, plan)
-        grad_depth = torch.empty_like(depth)
-        runs = plan.mode == 'runs' and runs_supported(C, depth.dtype)
-        if runs and context_rows is None and _nchw_direct(context, depth):
-            grad_context = torch.empty_like(context)
-            _lib.check(_lib.lib().bevpool_fused_backward_runs(
-                plan.ptr, rows.data_ptr(), depth.data_ptr(), context.data_ptr(), grad_depth.data_ptr(),
-                grad_context.data_ptr(), 1, _lib.dtype_code(depth), B, N, D, H, W, C, X, Y,
-                _lib.stream_ptr(depth.device)), 'bevpool_fused_backward_runs')
-            return grad_depth, grad_context
-        channels_last = context.permute(0, 2, 3, 1).is_contiguous()
-        ctx_nhwc = context_rows_nhwc(context) if context_rows is None else context_rows
-        grad_ctx_nhwc = torch.empty(BN, H, W, C, dtype=context.dtype, device=context.device)
-        if runs:
-            _lib.check(_lib.lib().bevpool_fused_backward_runs(
-                plan.ptr, rows.data_ptr(), depth.data_ptr(), ctx_nhwc.data_ptr(), grad_depth.data_ptr(),
-                grad_ctx_nhwc.data_ptr(), 0, _lib.dtype_code(depth), B, N, D, H, W, C, X, Y,
-                _lib.stream_ptr(depth.device)), 'bevpool_fused_backward_runs')
-        else:
-            _lib.check(_lib.lib().bevpool_fused_backward(
-                plan.ptr, rows.data_ptr(), depth.data_ptr(), ctx_nhwc.data_ptr(), grad_depth.data_ptr(),
-                grad_ctx_nhwc.data_ptr(), _lib.dtype_code(depth), B, N, D, H, W, C, X, Y,
-                _lib.stream_ptr(depth.device)), 'bevpool_fused_backward')
-        if channels_last:
-            grad_context = grad_ctx_nhwc.permute(0, 3, 1, 2)
-        else:
-            grad_context = _transpose(grad_ctx_nhwc, BN, H * W, C).view(BN, C, H, W)
-    return grad_depth, grad_context
+        return _fused_backward_rows(plan, _route(plan.mode, context, depth, context_rows), rows, None, depth, context,
+                                    context_rows)
 
 
 class VoxelPooling(Function):
@@ -468,51 +507,36 @@ class VoxelPoolingFused(Function):
         assert depth.is_contiguous()
         X, Y, Z = _voxel_num_ints(voxel_num)
         with torch.cuda.device(depth.device):
-            if plan is None and make_plan is not None:
-                # cold call with a caller-supplied plan builder (e.g. from the camera rig): fill overlapped with the build
-                if _nchw_direct(context, depth):
+            out = None
+            if plan is None:
+                runs = True                   # a caller-supplied builder (the camera rig) makes run plans
+                if make_plan is None:
+                    assert geom_xyz.is_contiguous()
+                    # (a run plan reads its run count back once to size the scratch rows: not while capturing)
+                    runs = (geom_xyz.dim() == 6 and runs_supported(context.shape[1], depth.dtype)
+                            and not torch.cuda.is_current_stream_capturing())
+                    frustum = tuple(geom_xyz.shape[1:5]) if runs else None      # (N, D, H, W): sort runs, not points
+                    make_plan, batch = (lambda: PoolingPlan(geom_xyz, (X, Y, Z), frustum)), geom_xyz.shape[0]
+                if runs and _route('runs', context, depth) == 'nchw':
+                    # cold call: the zero fill of the output may overlap the plan build
                     plan, out = fused_forward_cold(make_plan, int(batch), (X, Y, Z), depth, context)
-                    if plan.mode == 'runs':
-                        ctx.plan, ctx.direct = plan, True
-                        ctx.save_for_backward(depth, context)
-                        return out.permute(0, 3, 1, 2)
                 else:
                     plan = make_plan()
-            if plan is None:
-                assert geom_xyz.is_contiguous()
-                frustum = None
-                # (a run plan reads its run count back once to size the scratch rows: not while capturing)
-                if (geom_xyz.dim() == 6 and runs_supported(context.shape[1], depth.dtype)
-                        and not torch.cuda.is_current_stream_capturing()):
-                    frustum = tuple(geom_xyz.shape[1:5])      # (N, D, H, W): sort runs, not points
-                if frustum is not None and _nchw_direct(context, depth):
-                    # cold call: zero fill of the output overlapped with the plan build
-                    plan, out = fused_forward_cold(lambda: PoolingPlan(geom_xyz, (X, Y, Z), frustum), int(geom_xyz.shape[0]),
-                                                   (X, Y, Z), depth, context)
-                    ctx.plan, ctx.direct = plan, True
-                    ctx.save_for_backward(depth, context)
-                    return out.permute(0, 3, 1, 2)
-                plan = PoolingPlan(geom_xyz, (X, Y, Z), frustum)
             assert plan.voxel_num == (X, Y, Z)
-            direct = plan.mode == 'runs' and _nchw_direct(context, depth)
-            context_rows = None if direct else context_rows_nhwc(context)
-            out = fused_forward(plan, depth, context, context_rows)
-        ctx.plan = plan
-        ctx.direct = direct
-        if direct:
-            ctx.save_for_backward(depth, context)
-        else:
-            ctx.save_for_backward(depth, context, context_rows)   # the rows are reused by backward
+            route = _route(plan.mode, context, depth)
+            context_rows = None if route == 'nchw' else context_rows_nhwc(context)     # reused by backward
+            if out is None:
+                out = fused_forward(plan, depth, context, context_rows)
+        ctx.plan, ctx.route = plan, route
+        ctx.save_for_backward(depth, context, context_rows)
         return out.permute(0, 3, 1, 2)
 
     @staticmethod
     def backward(ctx, grad_out):
-        if ctx.direct:
-            (depth, context), context_rows = ctx.saved_tensors, None
-        else:
-            depth, context, context_rows = ctx.saved_tensors
+        depth, context, context_rows = ctx.saved_tensors
         with torch.cuda.device(grad_out.device):
-            grad_depth, grad_context = fused_backward(ctx.plan, grad_out, depth, context, context_rows)
+            rows = _grad_rows_nhwc(grad_out, ctx.plan)
+            grad_depth, grad_context = _fused_backward_rows(ctx.plan, ctx.route, rows, None, depth, context, context_rows)
         return None, grad_depth, grad_context, None, None, None, None
 
 
@@ -554,83 +578,54 @@ class VoxelPoolingFusedConcat(Function):
     def forward(ctx, depth, context, other_bev, voxel_num, plan, theta=None, resize=False):
         _lib.require_cuda(depth, context, other_bev)
         X, Y, _ = _voxel_num_ints(voxel_num)
-        BN, D, H, W = depth.shape
         C = context.shape[1]
         B = plan.batch
-        N = BN // B
         assert other_bev.shape[0] == B and (resize or tuple(other_bev.shape[2:]) == (Y, X))
         C2, Yl, Xl = other_bev.shape[1:]
         other_nchw = _other_layout(other_bev)
         assert other_nchw is not None
         Ct = C + C2
-        nchw = _nchw_direct(context, depth)
-        rows = None if nchw else context_rows_nhwc(context)
+        route = _route(plan.mode, context, depth)
         with torch.cuda.device(depth.device):
+            rows = None if route == 'nchw' else context_rows_nhwc(context)
             buf = torch.empty(B, Y, X, Ct, dtype=torch.float32, device=depth.device)
-            cap = max(1, plan.num_sorted)
-            run_rows = torch.empty(cap, C, dtype=torch.float32, device=depth.device)
-            ws = _forward_workspace(C, depth.device)
-            # with the warp, the pooled rows go to a scratch first -- occupied cells only (no zero fill): the warp skips
-            # the taps of empty cells through the plan's cell_start
-            pooled, stride = (buf, Ct) if theta is None else (_warp_scratch(B, Y, X, C, depth.device), C)
-            _lib.check(_lib.lib().bevpool_fused_forward_runs_into(
-                plan.ptr, depth.data_ptr(), (context if nchw else rows).data_ptr(),
-                (1 if nchw else 0) | (0 if theta is None else 2), pooled.data_ptr(), stride,
-                _lib.dtype_code(depth), B, N, D, H, W, C, X, Y, run_rows.data_ptr(), cap, ws.data_ptr(),
-                _lib.stream_ptr(depth.device)), 'bevpool_fused_forward_runs_into')
-            if theta is not None:
+            if theta is None:
+                fused_forward(plan, depth, context, rows, out=buf[..., :C])
+            else:
+                # the pooled rows go to a scratch first, occupied cells only (no zero fill): the warp skips the taps of
+                # empty cells through the plan's cell_start
                 from ..bev_augment import warp_forward_rows
+                pooled = fused_forward(plan, depth, context, rows, out=_warp_scratch(B, Y, X, C, depth.device),
+                                       prezeroed=True)
                 warp_forward_rows(theta, pooled, C, buf, Ct, plan.cell_start, B, C, (Y, X), (Y, X))
             # the other half (resampled or not): the one copy a cat cannot avoid
             _lib.check(_lib.lib().bevpool_resize_nearest_into(
-                other_bev.data_ptr(), _lib.dtype_code(other_bev), other_nchw, B, C2, Yl, Xl, Y, X, buf.data_ptr() + 4 * C, Ct,
-                _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_into')
-        ctx.plan, ctx.nchw, ctx.C, ctx.other_dtype, ctx.theta = plan, nchw, C, other_bev.dtype, theta
+                other_bev.data_ptr(), _lib.dtype_code(other_bev), other_nchw, B, C2, Yl, Xl, Y, X, buf[..., C:].data_ptr(),
+                Ct, _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_into')
+        ctx.plan, ctx.route, ctx.C, ctx.other_dtype, ctx.theta = plan, route, C, other_bev.dtype, theta
         ctx.other_shape, ctx.other_nchw, ctx.other_code = (B, C2, Yl, Xl), other_nchw, _lib.dtype_code(other_bev)
-        if nchw:
-            ctx.save_for_backward(depth, context)
-        else:
-            ctx.save_for_backward(depth, context, rows)
+        ctx.save_for_backward(depth, context, rows)
         return buf.permute(0, 3, 1, 2)
 
     @staticmethod
     def backward(ctx, grad_cat):
         plan, C = ctx.plan, ctx.C
-        if ctx.nchw:
-            (depth, context), rows = ctx.saved_tensors, None
-        else:
-            depth, context, rows = ctx.saved_tensors
-        BN, D, H, W = depth.shape
+        depth, context, rows = ctx.saved_tensors
         B = plan.batch
-        N = BN // B
         X, Y, _ = plan.voxel_num
         g = grad_cat.permute(0, 2, 3, 1)
         if not g.is_contiguous() or g.dtype != torch.float32:           # channels_last gradients (the usual case) pass as they are
             g = g.float().contiguous()
         Ct = g.shape[-1]
         with torch.cuda.device(depth.device):
-            grad_rows, stride = g, Ct
+            grad_rows, stride = g[..., :C], Ct
             if ctx.theta is not None:
                 # gradient of the pooled rows = warp backward of the camera half of grad_cat, occupied cells only (the
                 # pooling backward reads no other row)
                 from ..bev_augment import warp_backward_rows
                 grad_rows, stride = _warp_scratch(B, Y, X, C, depth.device), C
                 warp_backward_rows(ctx.theta, g, Ct, grad_rows, C, plan.cell_start, B, C, (Y, X), (Y, X))
-            grad_depth = torch.empty_like(depth)
-            if ctx.nchw:
-                grad_context = torch.empty_like(context)
-                gc_arg = grad_context
-            else:
-                gc_arg = torch.empty(BN, H, W, C, dtype=context.dtype, device=context.device)
-            _lib.check(_lib.lib().bevpool_fused_backward_runs_from(
-                plan.ptr, grad_rows.data_ptr(), stride, depth.data_ptr(), (context if ctx.nchw else rows).data_ptr(),
-                grad_depth.data_ptr(), gc_arg.data_ptr(), 1 if ctx.nchw else 0, _lib.dtype_code(depth), B, N, D, H, W, C, X, Y,
-                _lib.stream_ptr(depth.device)), 'bevpool_fused_backward_runs_from')
-            if not ctx.nchw:
-                if context.permute(0, 2, 3, 1).is_contiguous():
-                    grad_context = gc_arg.permute(0, 3, 1, 2)
-                else:
-                    grad_context = _transpose(gc_arg, BN, H * W, C).view(BN, C, H, W)
+            grad_depth, grad_context = _fused_backward_rows(plan, ctx.route, grad_rows, stride, depth, context, rows)
             _, C2, Yl, Xl = ctx.other_shape
             if (Yl, Xl) == (Y, X):
                 grad_other = g[..., C:].permute(0, 3, 1, 2).to(ctx.other_dtype)      # identity maps: a view
@@ -643,7 +638,7 @@ class VoxelPoolingFusedConcat(Function):
                 else:
                     grad_other = torch.empty(B, Yl, Xl, C2, dtype=ctx.other_dtype, device=depth.device).permute(0, 3, 1, 2)
                 _lib.check(_lib.lib().bevpool_resize_nearest_backward_from(
-                    g.data_ptr() + 4 * C, Ct, grad_other.data_ptr(), ctx.other_code, ctx.other_nchw, B, C2,
+                    g[..., C:].data_ptr(), Ct, grad_other.data_ptr(), ctx.other_code, ctx.other_nchw, B, C2,
                     Yl, Xl, Y, X, _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_backward_from')
         return grad_depth, grad_context, grad_other, None, None, None, None
 
@@ -673,9 +668,8 @@ def voxel_pooling_fused_concat(depth: torch.Tensor, context: torch.Tensor, other
         raise ValueError(f"resize_other must be None or 'nearest' (got {resize_other!r})")
     if other_bev.shape[0] != plan.batch:
         raise ValueError(f'other_bev has batch {other_bev.shape[0]}, the plan {plan.batch}')
-    C = context.shape[1]
     X, Y, _ = plan.voxel_num
-    fast = (plan.mode == 'runs' and runs_supported(C, depth.dtype) and depth.shape[3] % 4 == 0
+    fast = (_route(plan.mode, context, depth) != 'points' and depth.shape[3] % 4 == 0
             and _other_layout(other_bev) is not None and depth.is_contiguous())
     resize = resize_other is not None
     if bda_affine is not None and bda_affine.shape[0] != plan.batch:
@@ -712,9 +706,7 @@ class VoxelPoolingFusedLogits(Function):
         with torch.cuda.device(dev):
             out = torch.empty(B, Y, X, C, dtype=torch.float32, device=dev)
             stats = torch.empty(BN, H, W, 2, dtype=torch.float32, device=dev)
-            cap = max(1, plan.num_sorted)
-            run_rows = torch.empty(cap, C, dtype=torch.float32, device=dev)
-            ws = _forward_workspace(C, dev)
+            run_rows, cap, ws = _run_scratch(plan, C, dev)
             _lib.check(_lib.lib().bevpool_fused_forward_runs_logits(
                 plan.ptr, depth_feature.data_ptr(), Ct, D, stats.data_ptr(), out.data_ptr(), 0, _lib.dtype_code(depth_feature),
                 B, N, D, H, W, C, X, Y, run_rows.data_ptr(), cap, ws.data_ptr(), _lib.stream_ptr(dev)),
@@ -731,7 +723,9 @@ class VoxelPoolingFusedLogits(Function):
         with torch.cuda.device(grad_out.device):
             prob, _, _ = softmax_forward(depth_feature[:, :D], None)          # recomputed: the forward never stored it
             context = depth_feature[:, D:D + C].contiguous()
-            grad_depth, grad_context = fused_backward(ctx.plan, grad_out, prob, context)
+            rows = _grad_rows_nhwc(grad_out, ctx.plan)
+            # the route the gate admitted: prob and the context copy are fresh NCHW tensors of the same width
+            grad_depth, grad_context = _fused_backward_rows(ctx.plan, 'nchw', rows, None, prob, context, None)
             grad_logits = softmax_backward(prob, None, grad_depth, None, depth_feature.dtype)
             grad_feature = torch.zeros_like(depth_feature) if depth_feature.shape[1] > D + C else torch.empty_like(depth_feature)
             grad_feature[:, :D] = grad_logits
@@ -747,9 +741,7 @@ def voxel_pooling_fused_logits(depth_feature: torch.Tensor, depth_channels: int,
     W % 4 == 0, C in RUN_CHANNELS; other cases compose the stock ops).  For training runs that also need the
     probabilities (depth loss) use ``depth_distribution`` + ``voxel_pooling_fused``."""
     D, C = int(depth_channels), int(channels)
-    if (plan.mode == 'runs' and runs_supported(C, depth_feature.dtype) and depth_feature.shape[3] % 4 == 0
-            and depth_feature.is_contiguous() and depth_feature.data_ptr() % 16 == 0
-            and os.environ.get('BEVPOOL_NCHW_DIRECT', '1') != '0'):
+    if _route(plan.mode, depth_feature, depth_feature, channels=C) == 'nchw':
         return VoxelPoolingFusedLogits.apply(depth_feature, D, C, voxel_num, plan)
     return voxel_pooling_fused(None, depth_feature[:, :D].softmax(1).contiguous(), depth_feature[:, D:D + C].contiguous(),
                                voxel_num, plan)

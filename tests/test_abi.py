@@ -56,6 +56,60 @@ def test_argument_errors_are_codes_not_crashes(L):
     assert L.bevpool_transpose(None, None, 0, 1, 4, 4, None) == -1
 
 
+# The eight fused entry points: parameter names in ABI order.  Every case below breaks one argument of an otherwise
+# valid call and must come back with its code before the library touches the device (the pointers are fake).
+_FUSED_PARAMS = {
+    'bevpool_fused_forward': 'plan depth ctx out dtype B N D H W C X Y ws stream',
+    'bevpool_fused_backward': 'plan grad depth ctx gdepth gctx dtype B N D H W C X Y stream',
+    'bevpool_fused_forward_runs': 'plan depth ctx out dtype B N D H W C X Y rows cap ws stream',
+    'bevpool_fused_forward_runs_nchw': 'plan depth ctx out dtype B N D H W C X Y rows cap ws stream',
+    'bevpool_fused_forward_runs_into': 'plan depth ctx flags out stride dtype B N D H W C X Y rows cap ws stream',
+    'bevpool_fused_forward_runs_logits': 'plan feat Cf offset stats out stride dtype B N D H W C X Y rows cap ws stream',
+    'bevpool_fused_backward_runs': 'plan grad depth ctx gdepth gctx nchw dtype B N D H W C X Y stream',
+    'bevpool_fused_backward_runs_from': 'plan grad stride depth ctx gdepth gctx nchw dtype B N D H W C X Y stream',
+}
+_P, _MISALIGNED = 0x10000, 0x10004
+_VALID = dict(plan=_P, depth=_P, ctx=_P, out=_P, grad=_P, gdepth=_P, gctx=_P, ws=_P, rows=_P, feat=_P, stats=_P,
+              stream=None, dtype=0, B=2, N=2, D=8, H=4, W=8, C=80, X=16, Y=16, cap=64, flags=0, stride=128, nchw=0,
+              Cf=96, offset=8)
+E_ARG, E_RANGE, E_CHANNELS, E_ALIGN, E_DTYPE = -1, -2, -3, -4, -5
+_COMMON = [(dict(plan=None), E_ARG), (dict(N=0), E_ARG), (dict(W=0), E_ARG), (dict(B=1, X=65536, Y=65536), E_RANGE)]
+_RUNS = _COMMON + [(dict(C=84), E_CHANNELS), (dict(C=48), E_CHANNELS), (dict(dtype=1), E_DTYPE), (dict(dtype=2), E_DTYPE),
+                   (dict(ctx=_MISALIGNED), E_ALIGN)]
+_FUSED_ERRORS = {
+    'bevpool_fused_forward': _COMMON + [(dict(C=81), E_CHANNELS), (dict(C=516), E_CHANNELS), (dict(dtype=7), E_DTYPE),
+                                        (dict(ctx=_MISALIGNED), E_ALIGN), (dict(out=_MISALIGNED), E_ALIGN)],
+    'bevpool_fused_backward': _COMMON + [(dict(C=81), E_CHANNELS), (dict(C=0), E_CHANNELS), (dict(dtype=7), E_DTYPE),
+                                         (dict(gdepth=None), E_ARG), (dict(grad=_MISALIGNED), E_ALIGN),
+                                         (dict(gctx=_MISALIGNED), E_ALIGN)],
+    'bevpool_fused_forward_runs': _RUNS + [(dict(rows=None), E_ARG), (dict(cap=0), E_ARG), (dict(ws=None), E_ARG),
+                                           (dict(rows=_MISALIGNED), E_ALIGN)],
+    'bevpool_fused_forward_runs_nchw': _RUNS + [(dict(W=5), E_ALIGN), (dict(cap=0), E_ARG)],
+    'bevpool_fused_forward_runs_into': _RUNS + [(dict(stride=0), E_ARG), (dict(stride=-4), E_ARG), (dict(stride=76), E_ARG),
+                                                (dict(stride=82), E_ARG), (dict(flags=1, W=5), E_ALIGN),
+                                                (dict(flags=3, W=6), E_ALIGN), (dict(out=_MISALIGNED), E_ALIGN)],
+    'bevpool_fused_forward_runs_logits': [(dict(feat=None), E_ARG), (dict(stats=None), E_ARG), (dict(N=0), E_ARG),
+                                          (dict(offset=-1), E_ARG), (dict(offset=17), E_ARG), (dict(Cf=87, offset=8), E_ARG),
+                                          (dict(D=97, offset=0, C=16), E_ARG), (dict(dtype=1), E_DTYPE),
+                                          (dict(feat=_MISALIGNED), E_ALIGN), (dict(W=6), E_ALIGN)],
+    'bevpool_fused_backward_runs': _RUNS + [(dict(gctx=None), E_ARG), (dict(grad=_MISALIGNED), E_ALIGN),
+                                            (dict(nchw=1, W=5), E_ALIGN), (dict(nchw=1, depth=_MISALIGNED), E_ALIGN),
+                                            (dict(nchw=1, gdepth=_MISALIGNED), E_ALIGN)],
+    'bevpool_fused_backward_runs_from': _RUNS + [(dict(stride=0), E_ARG), (dict(stride=-80), E_ARG), (dict(stride=76), E_ARG),
+                                                 (dict(stride=82), E_ARG), (dict(W=5), E_ALIGN), (dict(nchw=1, W=5), E_ALIGN),
+                                                 (dict(depth=_MISALIGNED), E_ALIGN), (dict(gdepth=_MISALIGNED), E_ALIGN),
+                                                 (dict(grad=_MISALIGNED), E_ALIGN)],
+}
+
+
+@pytest.mark.parametrize('name', sorted(_FUSED_PARAMS))
+def test_fused_entry_point_argument_errors(L, name):
+    params = _FUSED_PARAMS[name].split()
+    for change, code in _FUSED_ERRORS[name]:
+        args = dict(_VALID, **change)
+        assert getattr(L, name)(*[args[p] for p in params]) == code, (name, change)
+
+
 def test_python_ops_refuse_cpu_tensors():
     import torch
     from mm_training_b200.ops.voxel_pooling import voxel_pooling

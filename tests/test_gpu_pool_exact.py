@@ -24,7 +24,7 @@ from mm_training_b200.configs import CFG_2, CFG_AIM
 from mm_training_b200.ops.voxel_pooling import (LiftSplatGeometry, build_plan, rig_variant, voxel_pooling,
                                                 voxel_pooling_fused, voxel_pooling_fused_concat,
                                                 voxel_pooling_fused_logits, voxel_pooling_rig)
-from mm_training_b200.ops.voxel_pooling.voxel_pooling import RUN_CHANNELS
+from mm_training_b200.ops.voxel_pooling.voxel_pooling import RUN_CHANNELS, VoxelPoolingFused
 from oracle import pool_exact_ref as px
 from oracle.depth_softmax_ref import sum_bound
 
@@ -366,6 +366,22 @@ def test_core_cold_forward_prezeroed(monkeypatch):
     got, ks = _fused(geom, depth, ctx, go, vn)
     _equal(got, want, 'cold')
     _fw_runs(ks, True, B, N, D, H, W)
+
+
+def test_plan_builder_forward_runs_once():
+    """A plan builder handed to the op (the camera rig's route) that returns a point plan: the pooling forward runs once,
+    with the kernels and grids of the call that is given that plan."""
+    B, N, D, H, W, C, vn, coherent = RUN_CASES[0]                 # fp32 NCHW context, C = 80, W % 4 == 0
+    geom = px.frustum_geom(27, B, N, D, H, W, vn, coherent).to(DEV)
+    (depth, ctx, _), want = _exact(geom, vn, N, C, 27)
+    forward = re.compile(r'\b(pool_forward_\w+|frustum_reduce_kernel)\b')
+    runs = []
+    for plan, make_plan in ((None, lambda: build_plan(geom, vn)), (build_plan(geom, vn), None)):
+        out, ks = _trace(lambda: VoxelPoolingFused.apply(None, depth, ctx, vn, plan, make_plan, B))
+        _equal((out.permute(0, 2, 3, 1),), want[:1], ('plan builder', plan is None))
+        runs.append([k for k in ks if forward.search(k[0])])
+    assert len(_launches(runs[0], 'pool_forward_share_kernel')) == 1, runs[0]
+    assert runs[0] == runs[1]
 
 
 @pytest.mark.parametrize('extra', [0, 3])
