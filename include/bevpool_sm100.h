@@ -200,6 +200,28 @@ int bevpool_fused_backward_runs_from(const void *plan, const void *grad_rows, in
                                      int feat_h, int feat_w, int channels, int num_voxel_x, int num_voxel_y,
                                      void *stream);
 
+/* ---- mixed precision (autocast): fp32 depth, fp16 / bf16 context ------------------------------------
+ * Under autocast DepthNet's output is bf16 / fp16, the depth softmax runs in fp32 and the context slice keeps the
+ * 16-bit type.  These two entry points take that pair as it is: context_dtype (BEVPOOL_F32 / F16 / BF16, else
+ * BEVPOOL_E_DTYPE) is the element type of context and grad_context; depth, output, gradient rows and grad_depth are
+ * fp32.  The kernels widen the context to fp32 where they load it (exact) and keep the fp32 sums and their order, so
+ * the output and grad_depth equal those of the fp32 entry points on the widened context bit for bit, and grad_context
+ * is the fp32 gradient rounded once to nearest even (fp16: +-inf beyond 65504).  BEVPOOL_F32 runs the fp32 code.
+ * A 16-bit NCHW context needs feat_w % 8 == 0 (tensor-map rows of 16 bytes; else BEVPOOL_E_ALIGN: pass pixel rows).
+ * forward: flags and out_rows / out_row_stride (> 0) as in ..._runs_into.
+ * backward: grad_row_stride as in ..._runs_from, 0 = packed (B, Y, X, C) rows; a 16-bit context needs
+ * feat_w % 4 == 0 and 16-byte aligned depth and grad_depth (the column kernel) on either layout.                    */
+int bevpool_fused_forward_runs_mixed(const void *plan, const void *depth, const void *context, int context_dtype,
+                                     int flags, void *out_rows, int64_t out_row_stride, int batch, int num_cams,
+                                     int depth_bins, int feat_h, int feat_w, int channels, int num_voxel_x,
+                                     int num_voxel_y, void *run_rows, int64_t run_rows_capacity, void *workspace,
+                                     void *stream);
+int bevpool_fused_backward_runs_mixed(const void *plan, const void *grad_rows, int64_t grad_row_stride,
+                                      const void *depth, const void *context, void *grad_depth, void *grad_context,
+                                      int context_is_nchw, int context_dtype, int batch, int num_cams, int depth_bins,
+                                      int feat_h, int feat_w, int channels, int num_voxel_x, int num_voxel_y,
+                                      void *stream);
+
 /* ---- run plan straight from the camera rig: no geom_xyz tensor -------------------------------------
  * Replaces layers/backbones/lss_fpn.py:328-361 (get_geometry) + :461-462 (index quantisation) as the
  * producer of the cell indices.  Inputs (all device pointers unless *_host):

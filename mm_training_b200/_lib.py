@@ -49,6 +49,8 @@ _SIGNATURES = {
     'bevpool_fused_forward_runs_logits': [_vp, _vp, _i, _i, _vp, _vp, _i64, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp, _vp],
     'bevpool_fused_backward_runs': [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     'bevpool_fused_backward_runs_from': [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
+    'bevpool_fused_forward_runs_mixed': [_vp, _vp, _vp, _i, _i, _vp, _i64, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp, _vp],
+    'bevpool_fused_backward_runs_mixed': [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     'bevpool_plan_status': [_vp, _ip, _vp],
     'bevpool_runplan_rig_sizes': [_i, _i, _i, _i, _i, _i, _i, _szp, _szp],
     'bevpool_runplan_build_rig': [_vp, _vp, _vp, _vp, _fp, _fp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp],

@@ -207,11 +207,13 @@ inline PlanView plan_view(const void *plan, int batch, int64_t num_points, int X
 }
 
 // pool_bwd2.cu: column kernel of the fused backward (fp32, g8 channel counts, W % 4 == 0); reads context and writes
-// the context gradient either as pixel rows (B*N, H, W, C) or, through TMA tensor maps, as NCHW (B*N, C, H, W)
+// the context gradient either as pixel rows (B*N, H, W, C) or, through TMA tensor maps, as NCHW (B*N, C, H, W).
+// ctx_dtype: element type of context and grad_context (BEVPOOL_F32 / F16 / BF16; 16-bit NCHW needs W % 8 == 0).
 int launch_fused_backward_col(const int32_t *cell_of_point, const int4 *pair_rec, const float *grad_rows, const float *depth,
-                              const float *ctx, float *grad_depth, float *grad_ctx, bool nchw, int batch, int num_cams,
+                              const void *ctx, float *grad_depth, void *grad_ctx, bool nchw, int batch, int num_cams,
                               int D, int H, int W, int C, int64_t cells_per_sample, cudaStream_t s,
-                              int64_t grad_row_stride = 0);     // floats between consecutive cells' gradient rows (0: C)
+                              int64_t grad_row_stride = 0,      // floats between consecutive cells' gradient rows (0: C)
+                              int ctx_dtype = BEVPOOL_F32);
 bool fused_backward_col_supported(int C, int W, const void *depth, const void *grad_depth, const void *cell_of_point);
 
 // pool_bwd.cu: tile kernel of the fused backward (fp32, g8 channel counts; any W)

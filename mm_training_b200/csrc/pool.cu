@@ -694,10 +694,11 @@ extern "C" int bevpool_fused_backward(const void *plan, const void *grad_out_nhw
 static int fused_backward_runs(const void *plan, const void *grad_rows, int64_t grad_row_stride, const void *depth,
                                const void *context, void *grad_depth, void *grad_context, bool nchw, bool col_args,
                                int dtype, int batch, int num_cams, int depth_bins, int feat_h, int feat_w, int channels,
-                               int X, int Y, void *stream) {
+                               int X, int Y, void *stream, int ctx_dtype = BEVPOOL_F32) {
   int rc = check_frustum_dims(batch, num_cams, depth_bins, feat_h, feat_w, X, Y);
   if (rc) return rc;
   if (dtype != BEVPOOL_F32) return BEVPOOL_E_DTYPE;
+  if (ctx_dtype != BEVPOOL_F32 && ctx_dtype != BEVPOOL_F16 && ctx_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
   if (!g8_supported(channels)) return BEVPOOL_E_CHANNELS;
   if (!plan || !grad_rows || !depth || !context || !grad_depth || !grad_context) return BEVPOOL_E_ARG;
   if (grad_row_stride < channels || (grad_row_stride % 4) != 0) return BEVPOOL_E_ARG;
@@ -707,6 +708,14 @@ static int fused_backward_runs(const void *plan, const void *grad_rows, int64_t 
   const PlanView pv = plan_view(plan, batch, (int64_t)num_cams * depth_bins * feat_h * feat_w, X, Y);
   const float *dp = static_cast<const float *>(depth);
   float *gd = static_cast<float *>(grad_depth);
+  if (ctx_dtype != BEVPOOL_F32) {
+    // a 16-bit context exists on the column kernel only (the tuning knobs that pick other kernels do not apply)
+    if (nchw && (feat_w % 8) != 0) return BEVPOOL_E_ALIGN;     // the tensor-map rows must be multiples of 16 bytes
+    if (!fused_backward_col_supported(channels, feat_w, dp, gd, pv.cell_of_point)) return BEVPOOL_E_ALIGN;
+    return launch_fused_backward_col(pv.cell_of_point, pv.pair_rec, static_cast<const float *>(grad_rows), dp, context, gd,
+                                     grad_context, nchw, batch, num_cams, depth_bins, feat_h, feat_w, channels, (int64_t)X * Y,
+                                     s, grad_row_stride, ctx_dtype);
+  }
   const bool strided = grad_row_stride != channels;
   if (g8_enabled()) {
     static const int which = env_int("BEVPOOL_BW_KERNEL", 2);
@@ -739,6 +748,21 @@ extern "C" int bevpool_fused_backward_runs_from(const void *plan, const void *gr
   return fused_backward_runs(plan, grad_rows, grad_row_stride, depth, context, grad_depth, grad_context,
                              context_is_nchw != 0, true, dtype, batch, num_cams, depth_bins, feat_h, feat_w, channels, X,
                              Y, stream);
+}
+
+// Autocast: fp32 depth and gradient rows with an fp16 / bf16 context; grad_context in the context's element type, the
+// fp32 sums of ..._runs_from rounded once.  grad_row_stride 0: packed rows (as ..._runs); an fp32 context runs exactly
+// what ..._runs (stride 0) or ..._runs_from does.
+extern "C" int bevpool_fused_backward_runs_mixed(const void *plan, const void *grad_rows, int64_t grad_row_stride,
+                                                 const void *depth, const void *context, void *grad_depth,
+                                                 void *grad_context, int context_is_nchw, int context_dtype, int batch,
+                                                 int num_cams, int depth_bins, int feat_h, int feat_w, int channels, int X,
+                                                 int Y, void *stream) {
+  if (grad_row_stride < 0) return BEVPOOL_E_ARG;
+  const bool packed = grad_row_stride == 0;
+  return fused_backward_runs(plan, grad_rows, packed ? channels : grad_row_stride, depth, context, grad_depth, grad_context,
+                             context_is_nchw != 0, !packed || context_dtype != BEVPOOL_F32, BEVPOOL_F32, batch, num_cams,
+                             depth_bins, feat_h, feat_w, channels, X, Y, stream, context_dtype);
 }
 
 extern "C" int bevpool_grad_rows(const void *plan, const void *grad_out_nchw, void *rows_nhwc, int dtype,

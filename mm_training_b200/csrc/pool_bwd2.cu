@@ -81,13 +81,43 @@ __device__ __forceinline__ void sts_f4(uint32_t addr, float4 v) {
   asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
 
-template <int NV2, bool kNchw, bool kStaticBins>
+// one pixel row of a 16-bit context in the g8 layout (channels of g8_channel), widened to fp32 / rounded from fp32
+template <int NV2, typename TC>
+__device__ __forceinline__ void g8_load_row_half(const TC *row, int l8, float (&v)[2 * NV2]) {
+  constexpr int NF4 = NV2 / 2, NF2 = NV2 & 1;
+#pragma unroll
+  for (int k = 0; k < NF4; ++k) {
+    const uint2 u = __ldg(reinterpret_cast<const uint2 *>(row + 32 * k + 4 * l8));
+    const float2 a = CtxType<TC>::to_float2(u.x), b = CtxType<TC>::to_float2(u.y);
+    v[4 * k + 0] = a.x; v[4 * k + 1] = a.y; v[4 * k + 2] = b.x; v[4 * k + 3] = b.y;
+  }
+  if (NF2) {
+    const float2 a = CtxType<TC>::to_float2(__ldg(reinterpret_cast<const unsigned *>(row + 32 * NF4 + 2 * l8)));
+    v[4 * NF4 + 0] = a.x; v[4 * NF4 + 1] = a.y;
+  }
+}
+template <int NV2, typename TC>
+__device__ __forceinline__ void g8_store_row_half(TC *row, int l8, const float (&v)[2 * NV2]) {
+  constexpr int NF4 = NV2 / 2, NF2 = NV2 & 1;
+#pragma unroll
+  for (int k = 0; k < NF4; ++k)
+    *reinterpret_cast<uint2 *>(row + 32 * k + 4 * l8) =
+        make_uint2(CtxType<TC>::from_float2(v[4 * k], v[4 * k + 1]), CtxType<TC>::from_float2(v[4 * k + 2], v[4 * k + 3]));
+  if (NF2) *reinterpret_cast<uint32_t *>(row + 32 * NF4 + 2 * l8) = CtxType<TC>::from_float2(v[4 * NF4], v[4 * NF4 + 1]);
+}
+
+// TC: element type of context and grad_context (fp32, or fp16 / bf16 under autocast).  A 16-bit context is widened to
+// fp32 where it is loaded and the fp32 context gradient is rounded once where it is stored, so grad_depth and
+// grad_context equal the fp32 kernel's on context.float(), the latter rounded to TC.  The NCHW box of a 16-bit context
+// is 8 columns wide (a tensor-map box row is at least 16 bytes), of which the CTA uses its 4; its gradient leaves in
+// 8-byte stores (4 columns of one channel row), which no 4-column tensor-map box could write.
+template <int NV2, bool kNchw, bool kStaticBins, typename TC = float>
 __global__ void __launch_bounds__(kBcThreads, (NV2 <= 5 ? 3 : 2))
 fused_backward_col_kernel(const __grid_constant__ CUtensorMap ctx_map, const __grid_constant__ CUtensorMap gctx_map,
                           const int32_t *__restrict__ cell_of_point, const int4 *__restrict__ pair_rec,
                           const float *__restrict__ grad_rows, const float *__restrict__ depth,
-                          const float *__restrict__ ctx_nhwc, float *__restrict__ grad_depth,
-                          float *__restrict__ grad_ctx_nhwc, int num_cams, int D, int H, int W,
+                          const TC *__restrict__ ctx_nhwc, float *__restrict__ grad_depth,
+                          TC *__restrict__ grad_ctx_nhwc, int num_cams, int D, int H, int W,
                           int64_t cells_per_sample, int tiles_h, int tiles_w, int64_t g_stride) {
   pdl_wait();
   pdl_trigger();
@@ -105,6 +135,7 @@ fused_backward_col_kernel(const __grid_constant__ CUtensorMap ctx_map, const __g
   uint32_t *s_mask = reinterpret_cast<uint32_t *>(s_raw + S::off_mask);
   uint64_t *s_bar = reinterpret_cast<uint64_t *>(s_raw + S::off_bar);
 
+  constexpr int kBoxW = 16 / (int)sizeof(TC);                       // columns of the NCHW context box
   const int tid = threadIdx.x, lane = tid & 31, wl = tid >> 5;      // warp = image column of the tile
   const int l8 = lane & 7, rg = lane >> 3;                          // lane = (rows 4*rg .. 4*rg+3, channel eighth)
   int bid = blockIdx.x;
@@ -128,8 +159,8 @@ fused_backward_col_kernel(const __grid_constant__ CUtensorMap ctx_map, const __g
     }
     __syncthreads();
     if (tid == 0) {
-      mbar_expect_tx(s_bar, (uint32_t)(kBcTW * kBcTH * C * 4));
-      tma_load_4d(s_g, &ctx_map, w0, h0, 0, bn, s_bar);
+      mbar_expect_tx(s_bar, (uint32_t)(kBcTH * C * 16));                   // box rows are 16 bytes
+      tma_load_4d(s_g, &ctx_map, sizeof(TC) == 4 ? w0 : (w0 & ~(kBoxW - 1)), h0, 0, bn, s_bar);
     }
   }
 
@@ -213,16 +244,22 @@ fused_backward_col_kernel(const __grid_constant__ CUtensorMap ctx_map, const __g
     for (int r = 0; r < NREG; ++r) cx[j][r] = gacc[j][r] = 0.f;
   if (kNchw) {
     mbar_wait(s_bar, 0);
+    const TC *box = reinterpret_cast<const TC *>(s_g);
+    const int col = (sizeof(TC) == 4 ? 0 : (w0 & (kBoxW - 1))) + wl;
 #pragma unroll
     for (int j = 0; j < 4; ++j)
 #pragma unroll
-      for (int r = 0; r < NREG; ++r) cx[j][r] = s_g[(g8_channel<NV2>(r, l8) * kBcTH + 4 * rg + j) * kBcTW + wl];
+      for (int r = 0; r < NREG; ++r) cx[j][r] = CtxType<TC>::to_float(box[(g8_channel<NV2>(r, l8) * kBcTH + 4 * rg + j) * kBoxW + col]);
   } else {
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int h = h0 + 4 * rg + j;
-      if (h < H && w0 + wl < W)
-        g8_load_row<NV2, true>(reinterpret_cast<const char *>(ctx_nhwc + ((int64_t)bn * HW + h * W + w0 + wl) * C), l8, cx[j]);
+      if (h < H && w0 + wl < W) {
+        if constexpr (sizeof(TC) == 4)
+          g8_load_row<NV2, true>(reinterpret_cast<const char *>(ctx_nhwc + ((int64_t)bn * HW + h * W + w0 + wl) * C), l8, cx[j]);
+        else
+          g8_load_row_half<NV2, TC>(ctx_nhwc + ((int64_t)bn * HW + h * W + w0 + wl) * C, l8, cx[j]);
+      }
     }
   }
   for (int i = tid; i < kBcDC * kBcDepStride; i += kBcThreads) s_res[i] = 0.f;
@@ -412,7 +449,21 @@ fused_backward_col_kernel(const __grid_constant__ CUtensorMap ctx_map, const __g
   cp_async_wait_all();
 
   // ---- context gradient
-  if (kNchw) {
+  if constexpr (kNchw && sizeof(TC) == 2) {
+    __syncthreads();                         // every copy into the row stages has landed and been consumed
+    TC *s_gc = reinterpret_cast<TC *>(s_g);  // [channel][row][4 columns], rounded once
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+#pragma unroll
+      for (int r = 0; r < NREG; ++r) s_gc[(g8_channel<NV2>(r, l8) * kBcTH + 4 * rg + j) * kBcTW + wl] = CtxType<TC>::from_float(gacc[j][r]);
+    __syncthreads();
+    for (int i = tid; i < C * kBcTH; i += kBcThreads) {                // (channel, row) = (i / 16, i % 16)
+      const int h = h0 + (i & (kBcTH - 1));
+      if (h < H)
+        *reinterpret_cast<uint2 *>(grad_ctx_nhwc + (((int64_t)bn * C + i / kBcTH) * H + h) * W + w0) =
+            *reinterpret_cast<const uint2 *>(s_gc + i * kBcTW);
+    }
+  } else if (kNchw) {
     __syncthreads();                         // every copy into the row stages has landed and been consumed
 #pragma unroll
     for (int j = 0; j < 4; ++j)
@@ -429,21 +480,27 @@ fused_backward_col_kernel(const __grid_constant__ CUtensorMap ctx_map, const __g
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int h = h0 + 4 * rg + j;
-      if (h < H && w0 + wl < W)
-        g8_store_row<NV2>(reinterpret_cast<char *>(grad_ctx_nhwc + ((int64_t)bn * HW + h * W + w0 + wl) * C), l8, gacc[j]);
+      if (h < H && w0 + wl < W) {
+        if constexpr (sizeof(TC) == 4)
+          g8_store_row<NV2>(reinterpret_cast<char *>(grad_ctx_nhwc + ((int64_t)bn * HW + h * W + w0 + wl) * C), l8, gacc[j]);
+        else
+          g8_store_row_half<NV2, TC>(grad_ctx_nhwc + ((int64_t)bn * HW + h * W + w0 + wl) * C, l8, gacc[j]);
+      }
     }
   }
 }
 
-template <int NV2, bool kNchw, bool kStaticBins>
+template <int NV2, bool kNchw, bool kStaticBins, typename TC = float>
 static int launch_bc(const CUtensorMap &ctx_map, const CUtensorMap &gctx_map, const int32_t *cell_of_point,
-                     const int4 *pair_rec, const float *grad_rows, const float *depth, const float *ctx_nhwc, float *grad_depth,
-                     float *grad_ctx_nhwc, int num_cams, int D, int H, int W, int64_t cells_per_sample, int64_t ctas,
+                     const int4 *pair_rec, const float *grad_rows, const float *depth, const void *ctx, float *grad_depth,
+                     void *grad_ctx, int num_cams, int D, int H, int W, int64_t cells_per_sample, int64_t ctas,
                      int tiles_h, int tiles_w, int64_t g_stride, cudaStream_t s) {
   constexpr size_t smem = BcSmem<NV2>::bytes;
-  BEVPOOL_RETURN_IF_CUDA(cudaFuncSetAttribute(fused_backward_col_kernel<NV2, kNchw, kStaticBins>,
+  const TC *ctx_nhwc = static_cast<const TC *>(ctx);
+  TC *grad_ctx_nhwc = static_cast<TC *>(grad_ctx);
+  BEVPOOL_RETURN_IF_CUDA(cudaFuncSetAttribute(fused_backward_col_kernel<NV2, kNchw, kStaticBins, TC>,
                                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  BEVPOOL_RETURN_IF_CUDA(launch_pdl(fused_backward_col_kernel<NV2, kNchw, kStaticBins>, dim3((unsigned)ctas), dim3(kBcThreads), smem, s,
+  BEVPOOL_RETURN_IF_CUDA(launch_pdl(fused_backward_col_kernel<NV2, kNchw, kStaticBins, TC>, dim3((unsigned)ctas), dim3(kBcThreads), smem, s,
                                     ctx_map, gctx_map, cell_of_point, pair_rec, grad_rows, depth, ctx_nhwc, grad_depth, grad_ctx_nhwc,
                                     num_cams, D, H, W, cells_per_sample, tiles_h, tiles_w, g_stride));
   BEVPOOL_LAUNCH_CHECK();
@@ -454,15 +511,36 @@ bool fused_backward_col_supported(int C, int W, const void *depth, const void *g
   return g8_supported(C) && (W % 4 == 0) && aligned16(depth) && aligned16(grad_depth) && aligned16(cell_of_point);
 }
 
-// context / grad_context: NCHW (B*N, C, H, W) when `nchw`, else pixel rows (B*N, H, W, C)
+// context / grad_context: NCHW (B*N, C, H, W) when `nchw`, else pixel rows (B*N, H, W, C); elements of ctx_dtype.  A 16-bit
+// context always takes the static-bins loop: both loops give the same bits.
 int launch_fused_backward_col(const int32_t *cell_of_point, const int4 *pair_rec, const float *grad_rows, const float *depth,
-                              const float *ctx, float *grad_depth, float *grad_ctx, bool nchw, int batch, int num_cams,
-                              int D, int H, int W, int C, int64_t cells_per_sample, cudaStream_t s, int64_t grad_row_stride) {
+                              const void *ctx, float *grad_depth, void *grad_ctx, bool nchw, int batch, int num_cams,
+                              int D, int H, int W, int C, int64_t cells_per_sample, cudaStream_t s, int64_t grad_row_stride,
+                              int ctx_dtype) {
   if (grad_row_stride <= 0) grad_row_stride = C;
   const int64_t tiles_h = ceil_div64(H, kBcTH), tiles_w = ceil_div64(W, kBcTW);
   const int64_t ctas = (int64_t)batch * num_cams * tiles_h * tiles_w;
   if (ctas >= (int64_t)INT32_MAX) return BEVPOOL_E_RANGE;
   CUtensorMap ctx_map{}, gctx_map{};
+  if (ctx_dtype != BEVPOOL_F32) {
+    const bool f16 = ctx_dtype == BEVPOOL_F16;
+    if (nchw) {
+      const uint64_t dims[4] = {(uint64_t)W, (uint64_t)H, (uint64_t)C, (uint64_t)batch * num_cams};
+      const uint64_t strides[3] = {(uint64_t)W * 2, (uint64_t)H * W * 2, (uint64_t)C * H * W * 2};
+      const uint32_t box[4] = {8, kBcTH, (uint32_t)C, 1};
+      const int rc = make_tensor_map(&ctx_map, f16 ? CtxType<__half>::kMap : CtxType<__nv_bfloat16>::kMap, ctx, 4, dims, strides, box);
+      if (rc) return rc;
+    }
+    int rc = BEVPOOL_OK;
+#define BEVPOOL_BC_ARGS ctx_map, gctx_map, cell_of_point, pair_rec, grad_rows, depth, ctx, grad_depth, grad_ctx, num_cams, D, H, W, \
+                        cells_per_sample, ctas, (int)tiles_h, (int)tiles_w, grad_row_stride, s
+    if (f16 && nchw) { BEVPOOL_G8_DISPATCH(C, (rc = launch_bc<NV2, true, true, __half>(BEVPOOL_BC_ARGS))); }
+    else if (f16) { BEVPOOL_G8_DISPATCH(C, (rc = launch_bc<NV2, false, true, __half>(BEVPOOL_BC_ARGS))); }
+    else if (nchw) { BEVPOOL_G8_DISPATCH(C, (rc = launch_bc<NV2, true, true, __nv_bfloat16>(BEVPOOL_BC_ARGS))); }
+    else { BEVPOOL_G8_DISPATCH(C, (rc = launch_bc<NV2, false, true, __nv_bfloat16>(BEVPOOL_BC_ARGS))); }
+#undef BEVPOOL_BC_ARGS
+    return rc;
+  }
   if (nchw) {
     const uint64_t dims[4] = {(uint64_t)W, (uint64_t)H, (uint64_t)C, (uint64_t)batch * num_cams};
     const uint64_t strides[3] = {(uint64_t)W * 4, (uint64_t)H * W * 4, (uint64_t)C * H * W * 4};

@@ -47,20 +47,25 @@ struct RaSmem {
   static constexpr size_t bytes = off_bar + 16;
 };
 
-// In-place layout change of a TMA box of the NCHW context tensor, [channel][16 rows][4 columns], into pixel
-// rows [row][column][channel], through registers (all threads read, barrier, all threads write).  Element e of
+// In-place layout change of a TMA box of the NCHW context tensor, [channel][16 rows][16 bytes of columns], into fp32
+// pixel rows [row][column][channel], through registers (all threads read, barrier, all threads write).  Element e of
 // the thread walks the channels fastest with the row rotated by the channel, so the transposed writes are
-// conflict-free and the reads 4-way conflicted at worst (once per CTA: ~1 % of its lifetime).
-template <int C>
-__device__ __forceinline__ void nchw_box_to_rows(float *s_ctx, int tid) {
+// conflict-free and the fp32 reads 4-way conflicted at worst (once per CTA: ~1 % of its lifetime).  A box row is
+// 16 bytes (the tensor-map minimum): the CTA's 4 columns for fp32; for fp16 / bf16 the 8 columns from w0 & ~7, of
+// which the CTA's 4 are converted.
+template <int C, typename TC>
+__device__ __forceinline__ void nchw_box_to_rows(float *s_ctx, int tid, int w0) {
   constexpr int kElems = kRunHB * kRaTW * C, kPer = (kElems + kRaThreads - 1) / kRaThreads;
+  constexpr int kBoxW = 16 / (int)sizeof(TC);
+  const int col0 = sizeof(TC) == 4 ? 0 : (w0 & (kBoxW - 1));
+  const TC *box = reinterpret_cast<const TC *>(s_ctx);
   float v[kPer];
 #pragma unroll
   for (int k = 0; k < kPer; ++k) {
     const int e = k * kRaThreads + tid;
     if (e < kElems) {
       const int c = e % C, rest = e / C, w = rest & (kRaTW - 1), h = ((rest >> 2) + c) & (kRunHB - 1);
-      v[k] = s_ctx[(c * kRunHB + h) * kRaTW + w];
+      v[k] = CtxType<TC>::to_float(box[(c * kRunHB + h) * kBoxW + col0 + w]);
     }
   }
   __syncthreads();
@@ -72,6 +77,22 @@ __device__ __forceinline__ void nchw_box_to_rows(float *s_ctx, int tid) {
       s_ctx[(h * kRaTW + w) * C + c] = v[k];
     }
   }
+  __syncthreads();
+}
+
+// fp16 / bf16 pixel rows [row][column][channel], as the bulk copies left them at the start of the tile buffer, widened
+// in place to the fp32 rows the reduction reads (same index, twice the bytes); a thread moves element pairs.
+template <int C, typename TC>
+__device__ __forceinline__ void half_rows_to_f32(float *s_ctx, int tid) {
+  constexpr int kPairs = kRunHB * kRaTW * C / 2, kPer = kPairs / kRaThreads;
+  static_assert(kPairs % kRaThreads == 0, "whole pairs per thread");
+  const uint32_t *src = reinterpret_cast<const uint32_t *>(s_ctx);
+  float2 v[kPer];
+#pragma unroll
+  for (int k = 0; k < kPer; ++k) v[k] = CtxType<TC>::to_float2(src[k * kRaThreads + tid]);
+  __syncthreads();
+#pragma unroll
+  for (int k = 0; k < kPer; ++k) reinterpret_cast<float2 *>(s_ctx)[k * kRaThreads + tid] = v[k];
   __syncthreads();
 }
 
@@ -87,11 +108,14 @@ __device__ __forceinline__ void nchw_box_to_rows(float *s_ctx, int tid) {
 // kLogits: `depth` holds the DepthNet LOGITS (lss_fpn.py:423 folded in): consecutive images are dep_img_stride floats
 // apart (a channel slice of depth_feature needs no copy) and `stats` holds {max, 1 / sum exp(l - max)} per pixel
 // (depth_stats_kernel below); the staging threads turn a logit into its probability while they transpose it.
-template <int NV2, bool kNchw, bool kLogits = false>
+// TC: element type of the context (fp32, or fp16 / bf16 under autocast).  A 16-bit context arrives in the first half
+// of the tile buffer and is widened to fp32 rows before the first chunk is reduced (exactly: every fp16 / bf16 value
+// is an fp32 value), so the reduction and its summation order are those of the fp32 kernel.
+template <int NV2, bool kNchw, bool kLogits = false, typename TC = float>
 __global__ void __launch_bounds__(kRaThreads, 4)
 frustum_reduce_kernel(const __grid_constant__ CUtensorMap ctx_map, const int32_t *__restrict__ run_code,
                       const int4 *__restrict__ pair_rec, const float *__restrict__ depth,
-                      const float *__restrict__ ctx_nhwc, float *__restrict__ run_rows,
+                      const TC *__restrict__ ctx_nhwc, float *__restrict__ run_rows,
                       const int32_t *__restrict__ cell_start, float *__restrict__ out, int32_t *__restrict__ status,
                       int img0, int64_t cell_base, int64_t num_cells, int D, int H, int W, int d_split, int d_per_cta,
                       int tiles_h, int tiles_w, int64_t capacity, int vec, int fill, int hints, int64_t out_stride,
@@ -137,13 +161,13 @@ frustum_reduce_kernel(const __grid_constant__ CUtensorMap ctx_map, const int32_t
   __syncthreads();
   if (tid == 0) {
     if (kNchw) {
-      mbar_expect_tx(s_bar, (uint32_t)(kRunHB * kRaTW * C * 4));
-      tma_load_4d(s_ctx, &ctx_map, w0, h0, 0, bn, s_bar);
+      mbar_expect_tx(s_bar, (uint32_t)(kRunHB * C * 16));                  // box rows are 16 bytes
+      tma_load_4d(s_ctx, &ctx_map, sizeof(TC) == 4 ? w0 : (w0 & ~(16 / (int)sizeof(TC) - 1)), h0, 0, bn, s_bar);
     } else {
-      const uint32_t row_bytes = (uint32_t)cols_here * C * 4;
+      const uint32_t row_bytes = (uint32_t)(cols_here * C * sizeof(TC));
       mbar_expect_tx(s_bar, row_bytes * rows_here);
       for (int r = 0; r < rows_here; ++r)
-        tma_load_1d(s_ctx + r * (kRaTW * C), ctx_nhwc + (((int64_t)bn * H + h0 + r) * W + w0) * C, row_bytes, s_bar);
+        tma_load_1d(reinterpret_cast<TC *>(s_ctx) + r * (kRaTW * C), ctx_nhwc + (((int64_t)bn * H + h0 + r) * W + w0) * C, row_bytes, s_bar);
     }
   }
 
@@ -299,7 +323,8 @@ frustum_reduce_kernel(const __grid_constant__ CUtensorMap ctx_map, const int32_t
     if (!ctx_ready) {                                       // first chunk: the context tile must have landed
       mbar_wait(s_bar, 0);
       ctx_ready = true;
-      if (kNchw) nchw_box_to_rows<C>(s_ctx, tid);
+      if constexpr (kNchw) nchw_box_to_rows<C, TC>(s_ctx, tid, w0);
+      else if constexpr (sizeof(TC) == 2) half_rows_to_f32<C, TC>(s_ctx, tid);
     }
     __syncthreads();                                        // transposed depths visible
 
@@ -409,8 +434,8 @@ depth_stats_kernel(const float *__restrict__ logits, int64_t img_stride, int D, 
 
 using namespace bevpool;
 
-template <int NV2, bool kNchw, bool kLogits = false>
-static int launch_stage_a(const CUtensorMap &ctx_map, const PlanView &pv, const float *dp, const float *cx, float *rr,
+template <int NV2, bool kNchw, bool kLogits = false, typename TC = float>
+static int launch_stage_a(const CUtensorMap &ctx_map, const PlanView &pv, const float *dp, const TC *cx, float *rr,
                           float *out, int32_t *status, int img0, int64_t cell_base, int64_t num_cells, int nb, int num_cams,
                           int D, int H, int W, int64_t capacity, int vec, int fill, int hints, int d_split, int64_t out_stride,
                           cudaStream_t s, int64_t dep_img_stride = 0, const float2 *stats = nullptr) {
@@ -424,8 +449,8 @@ static int launch_stage_a(const CUtensorMap &ctx_map, const PlanView &pv, const 
   (void)C;
   const size_t smem = RaSmem<NV2>::bytes;
   if (smem > 48 * 1024)
-    BEVPOOL_RETURN_IF_CUDA(cudaFuncSetAttribute(frustum_reduce_kernel<NV2, kNchw, kLogits>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  BEVPOOL_RETURN_IF_CUDA(launch_pdl_if(pdl_forward_enabled(), frustum_reduce_kernel<NV2, kNchw, kLogits>, dim3((unsigned)ctas), dim3(kRaThreads), smem, s,
+    BEVPOOL_RETURN_IF_CUDA(cudaFuncSetAttribute(frustum_reduce_kernel<NV2, kNchw, kLogits, TC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  BEVPOOL_RETURN_IF_CUDA(launch_pdl_if(pdl_forward_enabled(), frustum_reduce_kernel<NV2, kNchw, kLogits, TC>, dim3((unsigned)ctas), dim3(kRaThreads), smem, s,
       ctx_map, pv.run_code, pv.pair_rec, dp, cx, rr, pv.cell_start, out, status, img0, cell_base, num_cells, D, H, W, splits, d_per_cta, tiles_h,
       tiles_w, capacity, vec, fill, hints, out_stride, dep_img_stride, stats));
   BEVPOOL_LAUNCH_CHECK();
@@ -450,11 +475,31 @@ static const RunKnobs &run_knobs() {
   return k;
 }
 
+// stage A of every frame group for a 16-bit context (no logits variant)
+template <typename TC>
+static int launch_stage_a_half(bool nchw, const CUtensorMap &ctx_map, const PlanView &pv, const float *dp, const void *cx,
+                               float *rr, float *out, int32_t *status, int img0, int64_t cell_base, int64_t num_cells, int nb,
+                               int num_cams, int D, int H, int W, int C, int64_t capacity, int vec, int fill, int hints,
+                               int d_split, int64_t out_stride, cudaStream_t s) {
+  const TC *c = static_cast<const TC *>(cx);
+  int rc = BEVPOOL_OK;
+  if (nchw) {
+    BEVPOOL_G8_DISPATCH(C, (rc = launch_stage_a<NV2, true, false, TC>(ctx_map, pv, dp, c, rr, out, status, img0, cell_base, num_cells, nb,
+                                                                      num_cams, D, H, W, capacity, vec, fill, hints, d_split, out_stride, s)));
+  } else {
+    BEVPOOL_G8_DISPATCH(C, (rc = launch_stage_a<NV2, false, false, TC>(ctx_map, pv, dp, c, rr, out, status, img0, cell_base, num_cells, nb,
+                                                                       num_cams, D, H, W, capacity, vec, fill, hints, d_split, out_stride, s)));
+  }
+  return rc;
+}
+
+// ctx_dtype: element type of `context` (BEVPOOL_F32 / F16 / BF16); depth, run rows and output are fp32 (`dtype`)
 static int fused_forward_runs_impl(const void *plan, const void *depth, const void *context, bool nchw, void *out_nhwc,
                                    int dtype, int batch, int num_cams, int depth_bins, int feat_h, int feat_w,
                                    int channels, int X, int Y, void *run_rows, int64_t run_rows_capacity,
                                    void *workspace, void *stream, int64_t out_stride = 0, int64_t dep_img_stride = 0,
-                                   const float2 *stats = nullptr, int64_t ctx_img_stride = 0, bool prezeroed = false) {
+                                   const float2 *stats = nullptr, int64_t ctx_img_stride = 0, bool prezeroed = false,
+                                   int ctx_dtype = BEVPOOL_F32) {
   if (ctx_img_stride <= 0) ctx_img_stride = (int64_t)channels * feat_h * feat_w;
   if (out_stride == 0) out_stride = channels;
   if (stats && !nchw) return BEVPOOL_E_ARG;                   // the logits entry point exists for the NCHW layout only
@@ -464,10 +509,12 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
   if (rc) return rc;
   const int64_t np = (int64_t)num_cams * depth_bins * feat_h * feat_w;
   if (dtype != BEVPOOL_F32) return BEVPOOL_E_DTYPE;
+  if (ctx_dtype != BEVPOOL_F32 && ctx_dtype != BEVPOOL_F16 && ctx_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
   if (!g8_supported(channels)) return BEVPOOL_E_CHANNELS;
   if (!plan || !depth || !context || !out_nhwc || !run_rows || !workspace || run_rows_capacity <= 0) return BEVPOOL_E_ARG;
   if (!aligned16(context) || !aligned16(out_nhwc) || !aligned16(run_rows) || !aligned16(workspace)) return BEVPOOL_E_ALIGN;
-  if (nchw && (feat_w % 4) != 0) return BEVPOOL_E_ALIGN;      // the tensor-map rows must be multiples of 16 bytes
+  const int esz = ctx_dtype == BEVPOOL_F32 ? 4 : 2;
+  if (nchw && (feat_w * esz) % 16 != 0) return BEVPOOL_E_ALIGN;      // the tensor-map rows must be multiples of 16 bytes
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const PlanView pv = plan_view(plan, batch, np, X, Y);
   int32_t *status = plan_status(const_cast<void *>(plan));
@@ -483,9 +530,15 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
   CUtensorMap ctx_map{};
   if (nchw) {
     const uint64_t dims[4] = {(uint64_t)feat_w, (uint64_t)feat_h, (uint64_t)channels, (uint64_t)batch * num_cams};
-    const uint64_t strides[3] = {(uint64_t)feat_w * 4, (uint64_t)feat_h * feat_w * 4, (uint64_t)ctx_img_stride * 4};
-    const uint32_t box[4] = {kRaTW, kRunHB, (uint32_t)channels, 1};
-    if ((rc = make_tensor_map_f32(&ctx_map, cx, 4, dims, strides, box))) return rc;
+    const uint64_t strides[3] = {(uint64_t)feat_w * esz, (uint64_t)feat_h * feat_w * esz, (uint64_t)ctx_img_stride * esz};
+    if (ctx_dtype == BEVPOOL_F32) {
+      const uint32_t box[4] = {kRaTW, kRunHB, (uint32_t)channels, 1};
+      if ((rc = make_tensor_map_f32(&ctx_map, cx, 4, dims, strides, box))) return rc;
+    } else {                                                      // 16-byte box rows: 8 columns, the CTA uses 4 of them
+      const uint32_t box[4] = {8, kRunHB, (uint32_t)channels, 1};
+      const CUtensorMapDataType t = ctx_dtype == BEVPOOL_F16 ? CtxType<__half>::kMap : CtxType<__nv_bfloat16>::kMap;
+      if ((rc = make_tensor_map(&ctx_map, t, context, 4, dims, strides, box))) return rc;
+    }
   }
   const FastDiv one = make_fastdiv(1u);
   for (int b0 = 0; b0 < batch; b0 += fpc) {
@@ -499,7 +552,14 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
       const int max_split = (int)ceil_div64(depth_bins, kRaDC);
       d_split = d_split < 1 ? 1 : (d_split > max_split ? max_split : d_split);
     }
-    if (nchw && stats) {
+    if (ctx_dtype == BEVPOOL_F16) {
+      rc = launch_stage_a_half<__half>(nchw, ctx_map, pv, dp, context, rr, out, status, b0 * num_cams, cell_base, ncells, nb, num_cams,
+                                       depth_bins, feat_h, feat_w, channels, run_rows_capacity, vec, fill, hints, d_split, out_stride, s);
+    } else if (ctx_dtype == BEVPOOL_BF16) {
+      rc = launch_stage_a_half<__nv_bfloat16>(nchw, ctx_map, pv, dp, context, rr, out, status, b0 * num_cams, cell_base, ncells, nb,
+                                              num_cams, depth_bins, feat_h, feat_w, channels, run_rows_capacity, vec, fill, hints,
+                                              d_split, out_stride, s);
+    } else if (nchw && stats) {
       BEVPOOL_G8_DISPATCH(channels, (rc = launch_stage_a<NV2, true, true>(ctx_map, pv, dp, cx, rr, out, status, b0 * num_cams, cell_base, ncells, nb,
                                                                           num_cams, depth_bins, feat_h, feat_w, run_rows_capacity, vec, fill, hints,
                                                                           d_split, out_stride, s, dep_img_stride, stats)));
@@ -562,6 +622,18 @@ extern "C" int bevpool_fused_forward_runs_into(const void *plan, const void *dep
   return fused_forward_runs_impl(plan, depth, context, (context_is_nchw & 1) != 0, out_rows, dtype, batch, num_cams, depth_bins,
                                  feat_h, feat_w, channels, X, Y, run_rows, run_rows_capacity, workspace, stream, out_row_stride,
                                  0, nullptr, 0, (context_is_nchw & 2) != 0);
+}
+
+// Autocast: fp32 depth (the softmax runs in fp32) with the fp16 / bf16 context slice of DepthNet's output.  The context
+// is widened to fp32 where stage A loads it, so the output equals that of ..._runs_into on context.float(), bit for bit.
+extern "C" int bevpool_fused_forward_runs_mixed(const void *plan, const void *depth, const void *context, int context_dtype,
+                                                int flags, void *out_rows, int64_t out_row_stride, int batch, int num_cams,
+                                                int depth_bins, int feat_h, int feat_w, int channels, int X, int Y,
+                                                void *run_rows, int64_t run_rows_capacity, void *workspace, void *stream) {
+  if (out_row_stride <= 0) return BEVPOOL_E_ARG;
+  return fused_forward_runs_impl(plan, depth, context, (flags & 1) != 0, out_rows, BEVPOOL_F32, batch, num_cams, depth_bins,
+                                 feat_h, feat_w, channels, X, Y, run_rows, run_rows_capacity, workspace, stream, out_row_stride,
+                                 0, nullptr, 0, (flags & 2) != 0, context_dtype);
 }
 
 // lss_fpn.py:423 + :441-443 folded into the forward: the kernel reads DepthNet's output tensor itself -- depth_feature

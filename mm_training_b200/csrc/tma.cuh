@@ -37,10 +37,10 @@ inline EncodeTiledFn tensor_map_encoder() {
   return fn;
 }
 
-// fp32 tensor of `rank` dims (fastest first); strides in BYTES for dims 1..rank-1 (multiples of 16).
-// Out-of-bounds elements of a box read as zero and are not written by stores.
-inline int make_tensor_map_f32(CUtensorMap *map, const void *base, int rank, const uint64_t *dims,
-                               const uint64_t *strides_bytes, const uint32_t *box) {
+// tensor of `rank` dims (fastest first) with elements of `type`; strides in BYTES for dims 1..rank-1 (multiples of 16),
+// box[0] * element size a multiple of 16 bytes.  Out-of-bounds elements of a box read as zero and are not written by stores.
+inline int make_tensor_map(CUtensorMap *map, CUtensorMapDataType type, const void *base, int rank, const uint64_t *dims,
+                           const uint64_t *strides_bytes, const uint32_t *box) {
   EncodeTiledFn enc = tensor_map_encoder();
   if (!enc) return (int)cudaErrorNotSupported;
   // The encoder is a driver entry point and wants the primary context current on the calling thread; a thread that
@@ -54,7 +54,7 @@ inline int make_tensor_map_f32(CUtensorMap *map, const void *base, int rank, con
   cuuint32_t bx[5], es[5];
   for (int i = 0; i < rank; ++i) { gd[i] = dims[i]; bx[i] = box[i]; es[i] = 1; }
   for (int i = 0; i + 1 < rank; ++i) gs[i] = strides_bytes[i];
-  const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank, const_cast<void *>(base), gd, gs, bx, es,
+  const CUresult r = enc(map, type, (cuuint32_t)rank, const_cast<void *>(base), gd, gs, bx, es,
                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -69,6 +69,40 @@ inline int make_tensor_map_f32(CUtensorMap *map, const void *base, int rank, con
   }
   return BEVPOOL_OK;
 }
+
+inline int make_tensor_map_f32(CUtensorMap *map, const void *base, int rank, const uint64_t *dims,
+                               const uint64_t *strides_bytes, const uint32_t *box) {
+  return make_tensor_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, base, rank, dims, strides_bytes, box);
+}
+
+// element type and tensor-map type of a context tensor: fp32, or fp16 / bf16 converted to fp32 where it is loaded
+template <typename T> struct CtxType;
+template <> struct CtxType<float> {
+  static constexpr CUtensorMapDataType kMap = CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+  static __device__ __forceinline__ float to_float(float v) { return v; }
+};
+// 16-bit types: a pair of elements travels as one 32-bit word; every conversion to 16 bits rounds to nearest even
+// (fp16 beyond 65504 becomes +-inf), as torch's `.to(dtype)` does
+template <> struct CtxType<__half> {
+  static constexpr CUtensorMapDataType kMap = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+  static __device__ __forceinline__ float to_float(__half v) { return __half2float(v); }
+  static __device__ __forceinline__ float2 to_float2(uint32_t u) { return __half22float2(*reinterpret_cast<const __half2 *>(&u)); }
+  static __device__ __forceinline__ __half from_float(float v) { return __float2half_rn(v); }
+  static __device__ __forceinline__ uint32_t from_float2(float a, float b) {
+    const __half2 h = __floats2half2_rn(a, b);
+    return *reinterpret_cast<const uint32_t *>(&h);
+  }
+};
+template <> struct CtxType<__nv_bfloat16> {
+  static constexpr CUtensorMapDataType kMap = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  static __device__ __forceinline__ float to_float(__nv_bfloat16 v) { return __bfloat162float(v); }
+  static __device__ __forceinline__ float2 to_float2(uint32_t u) { return make_float2(__uint_as_float(u << 16), __uint_as_float(u & 0xffff0000u)); }
+  static __device__ __forceinline__ __nv_bfloat16 from_float(float v) { return __float2bfloat16_rn(v); }
+  static __device__ __forceinline__ uint32_t from_float2(float a, float b) {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    return *reinterpret_cast<const uint32_t *>(&h);
+  }
+};
 
 // ---- device side -------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }

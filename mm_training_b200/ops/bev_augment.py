@@ -33,7 +33,13 @@ def _normal_transform_pixel(h: int, w: int, like: torch.Tensor) -> torch.Tensor:
 def warp_theta(M: torch.Tensor, src_hw: Sequence[int], dsize: Sequence[int]) -> torch.Tensor:
     """(B, 2, 3) float32: the normalised destination -> source matrix kornia's ``warp_affine`` passes to
     ``F.affine_grid``, computed on ``M``'s device with kornia's ops (``inv_ex`` for its ``inverse``: the same LU values
-    without a host synchronisation)."""
+    without a host synchronisation).  Always in fp32 or fp64, autocast off: under bf16 autocast the products would round
+    the matrix to bf16 (moving the warp by whole cells) and ``inv_ex`` takes no 16-bit input."""
+    with torch.autocast(device_type=M.device.type, enabled=False):
+        return _warp_theta(M, src_hw, dsize)
+
+
+def _warp_theta(M: torch.Tensor, src_hw: Sequence[int], dsize: Sequence[int]) -> torch.Tensor:
     H, W = (int(v) for v in src_hw)
     Hd, Wd = (int(v) for v in dsize)
     if M.dim() != 3 or tuple(M.shape[1:]) != (2, 3):

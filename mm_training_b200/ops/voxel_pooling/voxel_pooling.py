@@ -329,13 +329,33 @@ def _nchw_direct(context: torch.Tensor, depth: torch.Tensor, channels: Optional[
             and os.environ.get('BEVPOOL_NCHW_DIRECT', '1') != '0')
 
 
+def _mixed(depth: torch.Tensor, context: torch.Tensor) -> bool:
+    """The autocast pair: fp32 depth (softmax runs in fp32) with an fp16 / bf16 context.  Pooled in fp32."""
+    return depth.dtype == torch.float32 and context.dtype in (torch.float16, torch.bfloat16)
+
+
+def _mixed_route(context: torch.Tensor, depth: torch.Tensor, context_rows: Optional[torch.Tensor]) -> str:
+    """``_route`` of a mixed call on a run plan.  The 16-bit context kernels exist for the column backward only, which
+    needs W % 4 == 0 and a 16-byte aligned contiguous depth; a tensor-map row of a 16-bit NCHW context is 16 bytes
+    only when W % 8 == 0, so W = 44 (CFG-2) takes pixel rows."""
+    W = depth.shape[3]
+    if W % 4 != 0 or not depth.is_contiguous() or depth.data_ptr() % 16 != 0 or context.data_ptr() % 16 != 0:
+        return 'points'
+    if (context_rows is None and context.is_contiguous() and W % 8 == 0
+            and os.environ.get('BEVPOOL_NCHW_DIRECT', '1') != '0'):
+        return 'nchw'
+    return 'rows'
+
+
 def _route(plan_mode: str, context: torch.Tensor, depth: torch.Tensor, context_rows: Optional[torch.Tensor] = None,
            channels: Optional[int] = None) -> str:
     """The kernels that pool ``context`` on a plan of ``plan_mode``: 'nchw' (run plan, ``_nchw_direct``), 'rows' (run
     plan; pixel rows, ``context_rows`` or ``context_rows_nhwc(context)``) or 'points' (point plan, or no run kernel for
-    the dtype / channel count)."""
+    the dtype / channel count).  A mixed call (``_mixed``) on 'points' pools ``context.float()``."""
     if plan_mode != 'runs' or not runs_supported(context.shape[1] if channels is None else channels, depth.dtype):
         return 'points'
+    if _mixed(depth, context):
+        return _mixed_route(context, depth, context_rows)
     return 'nchw' if context_rows is None and _nchw_direct(context, depth, channels) else 'rows'
 
 
@@ -346,15 +366,20 @@ def fused_forward(plan: PoolingPlan, depth: torch.Tensor, context: torch.Tensor,
     (B, Y, X, C) buffer; on a run plan also rows at a uniform cell stride, such as ``buf[..., :C]`` of a wider
     channels-last ``buf``.  ``prezeroed`` (run plans): the kernels write the rows of occupied cells only and leave the
     others as they are -- for an ``out`` that already holds zeros (``fused_forward_cold``) or whose empty cells are never
-    read (the BDA warp's scratch).  A point plan writes every cell either way."""
+    read (the BDA warp's scratch).  A point plan writes every cell either way.  fp32 ``depth`` with an fp16 / bf16
+    ``context`` (autocast) gives fp32 rows equal, bit for bit, to the call on ``context.float()``."""
     BN, D, H, W = depth.shape
     C = context.shape[1]
     X, Y, _ = plan.voxel_num
     B = plan.batch
     N = BN // B
-    assert context.shape == (BN, C, H, W) and depth.dtype == context.dtype
+    mixed = _mixed(depth, context)
+    assert context.shape == (BN, C, H, W) and (depth.dtype == context.dtype or mixed)
     assert B * N == BN and plan.num_points == N * D * H * W
     route = _route(plan.mode, context, depth, context_rows)
+    if mixed and route == 'points':             # no run kernel takes it: pool context.float(), the call it stands for
+        context, context_rows, mixed = context.float(), None, False
+        route = _route(plan.mode, context, depth)
     with torch.cuda.device(depth.device):
         if out is None:
             out, prezeroed = torch.empty(B, Y, X, C, dtype=depth.dtype, device=depth.device), False
@@ -377,8 +402,15 @@ def fused_forward(plan: PoolingPlan, depth: torch.Tensor, context: torch.Tensor,
         run_rows, cap, ws = _run_scratch(plan, C, depth.device)
         nchw = route == 'nchw'
         ctx_arg = context if nchw else (context_rows_nhwc(context) if context_rows is None else context_rows)
+        flags = (1 if nchw else 0) | (2 if prezeroed else 0)
+        if mixed:
+            _lib.check(_lib.lib().bevpool_fused_forward_runs_mixed(
+                plan.ptr, depth.data_ptr(), ctx_arg.data_ptr(), _lib.dtype_code(context), flags, out.data_ptr(), stride,
+                B, N, D, H, W, C, X, Y, run_rows.data_ptr(), cap, ws.data_ptr(), _lib.stream_ptr(depth.device)),
+                'bevpool_fused_forward_runs_mixed')
+            return out
         _lib.check(_lib.lib().bevpool_fused_forward_runs_into(
-            plan.ptr, depth.data_ptr(), ctx_arg.data_ptr(), (1 if nchw else 0) | (2 if prezeroed else 0), out.data_ptr(),
+            plan.ptr, depth.data_ptr(), ctx_arg.data_ptr(), flags, out.data_ptr(),
             stride, _lib.dtype_code(depth), B, N, D, H, W, C, X, Y, run_rows.data_ptr(), cap, ws.data_ptr(),
             _lib.stream_ptr(depth.device)), 'bevpool_fused_forward_runs_into')
     return out
@@ -424,12 +456,20 @@ def _fused_backward_rows(plan: PoolingPlan, route: str, grad_rows: torch.Tensor,
     """Fused backward on ``route`` (``_route``) -> (grad_depth, grad_context).  ``row_stride`` None: ``grad_rows`` are
     packed (B, Y, X, C) rows (``_grad_rows_nhwc``); else the row of cell c starts ``c * row_stride`` floats after the
     first (run plans with W % 4 == 0 only).  grad_context has the memory format of ``context``: channels_last in ->
-    channels_last out (zero-copy), NCHW in -> NCHW out (written NCHW on the 'nchw' route, else one tiled transpose)."""
+    channels_last out (zero-copy), NCHW in -> NCHW out (written NCHW on the 'nchw' route, else one tiled transpose).
+    A mixed call (``_mixed``) returns grad_context in the dtype of ``context``: the fp32 gradient of the call on
+    ``context.float()`` rounded once, as autograd's cast would round it."""
     BN, D, H, W = depth.shape
     C = context.shape[1]
     X, Y, _ = plan.voxel_num
     B = plan.batch
     N = BN // B
+    mixed = _mixed(depth, context)
+    if mixed and route == 'points':
+        upcast = context.float()                    # as in fused_forward
+        grad_depth, grad_context = _fused_backward_rows(plan, _route(plan.mode, upcast, depth), grad_rows, row_stride,
+                                                        depth, upcast, None)
+        return grad_depth, grad_context.to(context.dtype)
     nchw = route == 'nchw'
     assert row_stride is None or route != 'points'
     grad_depth = torch.empty_like(depth)
@@ -441,7 +481,10 @@ def _fused_backward_rows(plan: PoolingPlan, route: str, grad_rows: torch.Tensor,
     args = (depth.data_ptr(), ctx_arg.data_ptr(), grad_depth.data_ptr(), grad_ctx_arg.data_ptr())
     dims = (_lib.dtype_code(depth), B, N, D, H, W, C, X, Y, _lib.stream_ptr(depth.device))
     L = _lib.lib()
-    if route == 'points':
+    if mixed:
+        _lib.check(L.bevpool_fused_backward_runs_mixed(plan.ptr, grad_rows.data_ptr(), row_stride or 0, *args, int(nchw),
+                                                       _lib.dtype_code(context), *dims[1:]), 'bevpool_fused_backward_runs_mixed')
+    elif route == 'points':
         _lib.check(L.bevpool_fused_backward(plan.ptr, grad_rows.data_ptr(), *args, *dims), 'bevpool_fused_backward')
     elif row_stride is None:
         _lib.check(L.bevpool_fused_backward_runs(plan.ptr, grad_rows.data_ptr(), *args, int(nchw), *dims),
@@ -524,7 +567,9 @@ class VoxelPoolingFused(Function):
                     plan = make_plan()
             assert plan.voxel_num == (X, Y, Z)
             route = _route(plan.mode, context, depth)
-            context_rows = None if route == 'nchw' else context_rows_nhwc(context)     # reused by backward
+            # reused by backward; a mixed call on 'points' pools context.float() and makes its own rows
+            upcast = route == 'points' and _mixed(depth, context)
+            context_rows = None if route == 'nchw' or upcast else context_rows_nhwc(context)
             if out is None:
                 out = fused_forward(plan, depth, context, context_rows)
         ctx.plan, ctx.route = plan, route
@@ -546,7 +591,11 @@ def voxel_pooling_fused(geom_xyz: Optional[torch.Tensor], depth: torch.Tensor, c
 
     geom_xyz: int32 (B, N, D, H, W, 3) (ignored when ``plan`` is given); depth (B*N, D, H, W)
     softmax probabilities; context (B*N, C, H, W), NCHW or channels_last.  Returns (B, C, Y, X)
-    as a permuted view of a (B, Y, X, C) buffer, like the reference op."""
+    as a permuted view of a (B, Y, X, C) buffer, like the reference op.
+
+    Under autocast (fp32 ``depth``, fp16 / bf16 ``context``) the result is fp32 and equals, bit for bit, the call on
+    ``context.float()``; so do ``grad_depth`` and ``grad_context`` (in the dtype and memory format of ``context``).  On a
+    run plan the kernels read the 16-bit context themselves; other cases pool ``context.float()``."""
     return VoxelPoolingFused.apply(geom_xyz, depth, context, voxel_num, plan, None, None)
 
 
