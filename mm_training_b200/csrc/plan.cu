@@ -379,31 +379,38 @@ __device__ __forceinline__ float rig_dot4(const float (&m)[4], float px, float p
   }
 }
 
-// trunc((e - lo) / vs) with IEEE semantics.  The quotient by reciprocal is within 2 ulp of the true quotient:
-// when it is farther than that from every integer it truncates to the same value, otherwise (a fraction of a
-// percent of the points) the exact division decides.  rig_quantise3 does the three coordinates of a point with ONE
-// branch to the exact path.
+// trunc((e - lo) / vs) with IEEE semantics; a NaN, infinite or int32-overflowing quotient gives INT_MIN, which every
+// bounds test drops.  q' = (e - lo) * fl(1 / vs) differs from the correctly rounded quotient by at most 3 * 2^-24 |q|
+// (one rounding each on 1 / vs, on q' and on the quotient), i.e. by less than 7.3e-4 while |q'| < 4096: when q' is
+// farther than 1e-3 from every integer both truncate to the same value; otherwise (a fraction of a percent of the
+// points at shipped shapes, and every quotient from 4096 up) the exact division decides.  rig_quantise3 does the three
+// coordinates of a point with ONE branch to the exact path.
+__device__ __forceinline__ int rig_trunc_exact(float t, float vs) {
+  const float q = __fdiv_rn(t, vs);
+  return fabsf(q) < 2147483648.f ? __float2int_rz(q) : INT_MIN;     // NaN compares false
+}
 __device__ __forceinline__ int rig_quantise(float e, float lo, float vs, float inv_vs) {
   const float t = __fsub_rn(e, lo);
   const float qf = __fmul_rn(t, inv_vs);
   const float fr = fabsf(qf - rintf(qf));
-  if (fr > 1e-3f && fabsf(qf) < 4194304.f) return __float2int_rz(qf);
-  return __float2int_rz(__fdiv_rn(t, vs));
+  if (fr > 1e-3f && fabsf(qf) < 4096.f) return __float2int_rz(qf);   // NaN / inf q' give a NaN fr: exact path
+  return rig_trunc_exact(t, vs);
 }
 __device__ __forceinline__ void rig_quantise3(float ex, float ey, float ez, const RigParams &rp, int &ix, int &iy, int &iz) {
   const float tx = __fsub_rn(ex, rp.lo[0]), ty = __fsub_rn(ey, rp.lo[1]), tz = __fsub_rn(ez, rp.lo[2]);
   const float qx = __fmul_rn(tx, rp.inv_vs[0]), qy = __fmul_rn(ty, rp.inv_vs[1]), qz = __fmul_rn(tz, rp.inv_vs[2]);
   const float fx = fabsf(qx - rintf(qx)), fy = fabsf(qy - rintf(qy)), fz = fabsf(qz - rintf(qz));
   const float big = fmaxf(fmaxf(fabsf(qx), fabsf(qy)), fabsf(qz));
-  // (NaN compares false -> exact path)
-  if (fminf(fminf(fx, fy), fz) > 1e-3f && big < 4194304.f) {
+  // A NaN or infinite q' has a NaN fraction.  fminf / fmaxf drop a NaN operand, so each fraction is compared on its
+  // own: a NaN fails its comparison and the point takes the exact path.
+  if (fx > 1e-3f && fy > 1e-3f && fz > 1e-3f && big < 4096.f) {
     ix = __float2int_rz(qx);
     iy = __float2int_rz(qy);
     iz = __float2int_rz(qz);
   } else {
-    ix = __float2int_rz(__fdiv_rn(tx, rp.vs[0]));
-    iy = __float2int_rz(__fdiv_rn(ty, rp.vs[1]));
-    iz = __float2int_rz(__fdiv_rn(tz, rp.vs[2]));
+    ix = rig_trunc_exact(tx, rp.vs[0]);
+    iy = rig_trunc_exact(ty, rp.vs[1]);
+    iz = rig_trunc_exact(tz, rp.vs[2]);
   }
 }
 
@@ -460,7 +467,7 @@ plan_key_rig_kernel(RigParams rp, const int32_t *__restrict__ geom, int num_cams
   // cell indices agree at the first and the last row of a pair they agree on every row in between (a level camera:
   // m[.][1] == 0 for x and y), and the rows whose z index lies in [0, Z) form ONE interval, found by two binary
   // searches on z alone: ~10 coordinate evaluations per pair instead of 48, one head, no per-row voting.  Bit-identical
-  // to the per-row walk below by construction; it needs fy sorted (checked per CTA) and finite end points.  A warp
+  // to the per-row walk below by construction; it needs fy sorted (checked per CTA) and end points below 1e30.  A warp
   // takes it only when all its pairs qualify; tilted cameras and geom_xyz plans walk the rows.
   bool warp_fast = false;
   if (kVariant >= 0) {
@@ -481,7 +488,11 @@ plan_key_rig_kernel(RigParams rp, const int32_t *__restrict__ geom, int num_cams
       const float big = fmaxf(fmaxf(fmaxf(fabsf(ea0), fabsf(ea1)), fmaxf(fabsf(ea2), fabsf(eb0))), fmaxf(fabsf(eb1), fabsf(eb2)));
       rig_quantise3(ea0, ea1, ea2, rp, ix0, iy0, iz0);
       rig_quantise3(eb0, eb1, eb2, rp, ix1, iy1, iz1);
-      fast = big < 1e30f && ix0 == ix1 && iy0 == iy1;          // (NaN compares false -> per-row walk)
+      // big < 1e30f sends end points that overflowed to +-inf down the walk; fmaxf drops a NaN operand, so it does not
+      // see NaN.  A NaN end point gets INT_MIN from rig_quantise3 instead.  A NaN or inf needs a non-finite entry in
+      // its combine row, which makes that coordinate non-finite -- INT_MIN -- on every row, so the pair is dropped
+      // here exactly as the walk drops each row.
+      fast = big < 1e30f && ix0 == ix1 && iy0 == iy1;
     }
     warp_fast = __all_sync(0xffffffffu, fast);
     if (warp_fast) {

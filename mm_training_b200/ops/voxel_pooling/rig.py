@@ -91,8 +91,11 @@ class LiftSplatGeometry:
     def combine(sensor2ego_mat: torch.Tensor, intrin_mat: torch.Tensor) -> torch.Tensor:
         """``sensor2ego @ inverse(intrin)`` (B, N, 4, 4) -- ``lss_fpn.py:354``, left in torch (B*N tiny matrices); always
         float32 (autocast off).  ``inv_ex(check_errors=False)`` runs the LU kernels of ``torch.inverse`` (same values)
-        without its singularity check, which is a host synchronisation per call; a singular intrinsic matrix gives inf / nan
-        coordinates here and every point of that image is dropped (the reference raises)."""
+        without its singularity check, which is a host synchronisation per call.  A singular intrinsic matrix (or a NaN / inf
+        in ``sensor2ego_mat``) gives non-finite entries here, where the reference raises.  The plan kernels then give
+        INT_MIN for every coordinate whose ``combine`` row is not finite, so every point of that image is dropped: it
+        adds nothing to the pooled output, gets a zero depth gradient, and the other images' plan entries are those of
+        a plan without it (``tests/test_gpu_quantise.py``)."""
         with torch.autocast(device_type=sensor2ego_mat.device.type, enabled=False):
             inv = torch.linalg.inv_ex(intrin_mat.float(), check_errors=False).inverse
             return sensor2ego_mat.float().matmul(inv).contiguous()
