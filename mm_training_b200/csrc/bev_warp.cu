@@ -12,9 +12,10 @@
 // that sits on an integer could go either way).
 //
 // Optional cell_start (a pooling plan's CSR, B*H*W + 1 entries): source cells with cell_start[c + 1] == cell_start[c]
-// are known to be zero rows.  The forward skips such taps without reading the row (adding w * 0 to an accumulator
-// that starts at +0 never changes its bits, so the result is identical to reading a zero row); the backward writes
-// gradient rows for occupied cells only and leaves the others untouched.
+// are known to be zero rows.  The forward skips such taps without reading the row (adding w * 0, w >= +0, never
+// changes the accumulator's value, so the result equals reading a zero row -- by value: an accumulator at -0 from an
+// underflowed negative product stays -0 where the zero row would make it +0); the backward writes gradient rows for
+// occupied cells only and leaves the others untouched.
 #include "common.cuh"
 
 #include <math.h>
@@ -71,9 +72,10 @@ __device__ __forceinline__ void load_theta(const float *theta, int b, float (&th
 
 // Candidate window of source cell (sx, sy): destination pixels whose footprint can touch it.  A footprint touches the
 // cell iff the pixel's source coordinate lies in [sx - 1, sx + 1) x [sy - 1, sy + 1); the window is the bounding box
-// of that square's preimage under the (double precision) destination -> source pixel map, widened by one destination
-// pixel to absorb the float32 rounding of the kernel's coordinates, clipped to the grid.  Empty when theta is not
-// finite (then no destination pixel has a finite coordinate); the whole grid when the map is singular.
+// of that square's preimage under the (double precision) destination -> source pixel map, the square first widened by
+// a bound on the float32 error of the kernel's coordinates (a flat one-pixel margin dropped taps at magnifications
+// around 10^5), clipped to the grid.  Empty when theta is not finite (then no destination pixel has a finite
+// coordinate); the whole grid when the map is singular.
 __device__ __forceinline__ void warp_window(const float (&th)[6], int sx, int sy, int Ws, int Hs, int Wd, int Hd,
                                             int &x_lo, int &x_hi, int &y_lo, int &y_hi) {
   bool finite = true;
@@ -95,8 +97,13 @@ __device__ __forceinline__ void warp_window(const float (&th)[6], int sx, int sy
   const double i00 = a11 / det, i01 = -a01 / det, i10 = -a10 / det, i11 = a00 / det;
   const double u = sx - b0, v = sy - b1;
   const double cx = i00 * u + i01 * v, cy = i10 * u + i11 * v;
-  const double ex = fabs(i00) + fabs(i01), ey = fabs(i10) + fabs(i11);
-  const double xl = floor(cx - ex) - 1.0, xh = ceil(cx + ex) + 1.0, yl = floor(cy - ey) - 1.0, yh = ceil(cy + ey) + 1.0;
+  // float32 error of warp_taps' coordinates, in source pixels: |ix - exact| <= (Ws - 1) u (3 S + 1) with
+  // S = |th0| + |th1| + |th2| and u = 2^-24 (2u from linspace, one rounding per fmaf / add / multiply); taken
+  // as (Ws - 1) 2^-22 (S + 1), then mapped to destination pixels through |A^-1|
+  const double dx = (Ws - 1) * 0x1p-22 * (fabs((double)th[0]) + fabs((double)th[1]) + fabs((double)th[2]) + 1.0);
+  const double dy = (Hs - 1) * 0x1p-22 * (fabs((double)th[3]) + fabs((double)th[4]) + fabs((double)th[5]) + 1.0);
+  const double ex = fabs(i00) * (1.0 + dx) + fabs(i01) * (1.0 + dy), ey = fabs(i10) * (1.0 + dx) + fabs(i11) * (1.0 + dy);
+  const double xl = floor(cx - ex), xh = ceil(cx + ex), yl = floor(cy - ey), yh = ceil(cy + ey);
   if (!(isfinite(xl) && isfinite(xh) && isfinite(yl) && isfinite(yh))) return;
   x_lo = (int)fmin(fmax(xl, 0.0), (double)Wd);
   x_hi = (int)fmax(fmin(xh, Wd - 1.0), -1.0);
