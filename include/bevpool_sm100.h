@@ -316,21 +316,22 @@ int bevpool_resize_nearest_index(int in_size, int out_size, int32_t *src_of_dst_
  *   max_sample_points  largest per-sample point count (host value, sizes the launch)
  *   voxel_size_host[3], range_host[6] = [xmin,ymin,zmin,xmax,ymax,zmax], grid_host[3] = [gx,gy,gz]
  *   outputs are packed like mmdet3d's concatenation: rows of sample b start at voxel_base[b]
- *     voxels     (batch*max_voxels, max_points, F) float32   rows >= voxel_base[batch] untouched
+ *     voxels     (batch*max_voxels, max_points, F) float32
  *     coors      (batch*max_voxels, 4) int32 [b, z, y, x]
  *     num_points (batch*max_voxels) int32
  *     voxel_base device int32[batch + 1] (written): row offsets; [batch] = total voxel count M
  *     voxel_mean optional (batch*max_voxels, mean_features) float32 = HardSimpleVFE, or NULL
  *   temp: bevvox_temp_bytes() bytes of scratch.
  * Grids of up to 2^26 cells per batch (the aiMotive pillar grid has 2^19 per sample) use a dense first-point table
- * like mmcv's CPU kernel, larger ones a hash table; the outputs are identical.  `voxels` and `num_points` are fully
- * overwritten (rows beyond voxel_base[batch] are zero on the dense path).  mean_features <= 16.
- * bevvox_hard_voxelize_scatter (dense path only) takes the clouds either concatenated or as a DEVICE array of `batch`
- * per-sample base pointers (points == NULL; the reference passes a list of tensors: no concatenation pass) and, with
- * canvas != NULL, also writes the dense canvas (batch, mean_features, gz, gy, gx) of the fused HardSimpleVFE mean --
- * voxelize -> VFE -> scatter of models/bev_depth.py:181-183 in one call.  canvas_is_zeroed == 0: the call writes every
- * element of the canvas (with a voxel_mean output: one in-order pass over the canvas after the voxels are final, no
- * fill; without: a zero fill on a side stream + scattered stores); != 0: the caller zero-filled it already and only the
+ * like mmcv's CPU kernel, larger ones a hash table; the outputs are identical.  Every row of `voxels`, `num_points`,
+ * `coors` and `voxel_mean` is written: rows >= voxel_base[batch] are zero, on both paths.  mean_features <= 16.
+ * bevvox_hard_voxelize_scatter takes the clouds either concatenated or, on the dense path only, as a DEVICE array of
+ * `batch` per-sample base pointers (points == NULL; the reference passes a list of tensors: no concatenation pass) and,
+ * with canvas != NULL, also writes the dense canvas (batch, mean_features, gz, gy, gx) of the fused HardSimpleVFE mean
+ * -- voxelize -> VFE -> scatter of models/bev_depth.py:181-183 in one call.  Only the voxel_base[batch] live rows reach
+ * the canvas (the count is read on the device: no host synchronisation).  canvas_is_zeroed == 0: the call writes every
+ * element of the canvas (dense path with a voxel_mean output: one in-order pass over the canvas after the voxels are
+ * final, no fill; otherwise a zero fill + scattered stores); != 0: the caller zero-filled it already and only the
  * occupied cells are stored.                                                                                          */
 int bevvox_temp_bytes(int batch, int64_t total_points, const int *grid_host, int max_voxels, int max_points,
                       size_t *temp_bytes);

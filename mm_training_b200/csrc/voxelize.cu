@@ -16,8 +16,8 @@
 //      (mmcv's voxel numbering), capped at max_voxels
 //   3. per voxel, the max_points smallest point indices via a chain of atomicMin on a sorted
 //      slot list (each slot ends up holding the r-th smallest index whatever the interleaving)
-//   4. gather: every element of voxels / num_points is written exactly once, zero padding
-//      included; optional fused VFE mean (HardSimpleVFE)
+//   4. gather: every row of voxels / num_points / coors / mean is written, rows beyond the voxel
+//      count as zeros; optional fused VFE mean (HardSimpleVFE) and its canvas (live rows only)
 // mmcv's own deterministic CUDA path needs an O(N^2) predecessor scan and a single-thread
 // numbering kernel for the same result.
 #include "common.cuh"
@@ -174,18 +174,22 @@ vox_assign_kernel(const float *__restrict__ points, const int32_t *__restrict__ 
 }
 
 // ---- 4. gather ---------------------------------------------------------------------------------
-// one warp per voxel row: copies max_points x F floats (zeros for unused slots), writes num_points
-// and, optionally, the mean of the first `mean_features` columns (HardSimpleVFE).
+// one warp per row of the padded output (batch * max_voxels rows): copies max_points x F floats (zeros for unused
+// slots), writes num_points and, optionally, the mean of the first `mean_features` columns (HardSimpleVFE) and its
+// canvas cells (batch, mean_features, gz, gy, gx), zero-filled before.  Rows >= voxel_base[batch] are written as zeros
+// (voxels, num_points, coors, mean) and never reach the canvas.
 __global__ void __launch_bounds__(256)
 vox_gather_kernel(const float *__restrict__ points, int F, const int32_t *__restrict__ lists,
                   const int32_t *__restrict__ counts, const int32_t *__restrict__ voxel_base, int batch,
-                  int max_points, float *__restrict__ voxels, int32_t *__restrict__ num_points,
-                  float *__restrict__ voxel_mean, int mean_features) {
+                  int64_t total_rows, int max_points, float *__restrict__ voxels, int32_t *__restrict__ num_points,
+                  int32_t *__restrict__ coors, float *__restrict__ voxel_mean, int mean_features, VoxGeom g,
+                  float *__restrict__ canvas) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
-  if (row >= voxel_base[batch]) return;
+  if (row >= total_rows) return;
+  const bool live = row < voxel_base[batch];
   const int32_t *list = lists + (int64_t)row * max_points;
-  const int cnt = min(counts[row], max_points);
+  const int cnt = live ? min(counts[row], max_points) : 0;
   float *vout = voxels + (int64_t)row * max_points * F;
   const int total = max_points * F;
   for (int e = lane; e < total; e += 32) {
@@ -194,11 +198,22 @@ vox_gather_kernel(const float *__restrict__ points, int F, const int32_t *__rest
     if (t < cnt) v = __ldg(points + (int64_t)list[t] * F + c);
     vout[e] = v;
   }
-  if (lane == 0) num_points[row] = cnt;
-  if (voxel_mean && lane < mean_features) {
-    float s = 0.f;
-    for (int t = 0; t < cnt; ++t) s += __ldg(points + (int64_t)list[t] * F + lane);   // sequential, slot order
-    voxel_mean[(int64_t)row * mean_features + lane] = s / (float)cnt;
+  if (lane == 0) {
+    num_points[row] = cnt;
+    if (!live) reinterpret_cast<int4 *>(coors)[row] = make_int4(0, 0, 0, 0);   // (live rows: vox_assign_kernel)
+  }
+  if ((voxel_mean || canvas) && lane < mean_features) {
+    float m = 0.f;
+    if (live) {
+      float s = 0.f;
+      for (int t = 0; t < cnt; ++t) s += __ldg(points + (int64_t)list[t] * F + lane);   // sequential, slot order
+      m = s / (float)cnt;
+    }
+    if (voxel_mean) voxel_mean[(int64_t)row * mean_features + lane] = m;
+    if (canvas && live) {
+      const int4 c = reinterpret_cast<const int4 *>(coors)[row];                        // (b, z, y, x)
+      canvas[((((int64_t)c.x * mean_features + lane) * g.gz + c.y) * g.gy + c.z) * g.gx + c.w] = m;
+    }
   }
 }
 
@@ -674,7 +689,7 @@ __device__ __forceinline__ void vox_sort16_desc(int (&w)[16]) {
 // running sums for the HardSimpleVFE mean in slot order, count = number of filled slots.  The tile then leaves as ONE
 // contiguous span of 32 * max_points * F floats written with 16-byte stores -- every element of `voxels` is written
 // exactly once, coalesced (no memset of the 93 %-padding tensor, no 20-byte scattered stores).  Rows beyond the voxel
-// count are written as zeros with num_points = 0.
+// count are written as zeros (voxels, num_points, coors, mean).
 constexpr int kFinWarps = 4;
 template <int FM>                                       // FM >= F: bound of the per-point register arrays (8 or 16)
 __global__ void __launch_bounds__(kFinWarps * 32)
@@ -784,6 +799,10 @@ vox_finalize_kernel(VoxPoints pts, const int32_t *__restrict__ offsets, int F, V
           if (canvas) canvas[((((int64_t)b * mean_features + k) * g.gz + z) * g.gy + y) * g.gx + x] = m;
         }
       }
+    } else {                                               // padding row: zero coordinates and mean
+      reinterpret_cast<int4 *>(coors)[row] = make_int4(0, 0, 0, 0);
+      if (voxel_mean)
+        for (int k = 0; k < mean_features; ++k) voxel_mean[row * mean_features + k] = 0.f;
     }
     num_points[row] = cnt;
   }
@@ -872,6 +891,8 @@ vox_finalize_coop_kernel(VoxPoints pts, const int32_t *__restrict__ offsets, int
     z = (int)(cy / (uint32_t)g.gy);
     y = (int)(cy - (uint32_t)z * (uint32_t)g.gy);
     reinterpret_cast<int4 *>(coors)[row] = make_int4(b, z, y, x);
+  } else if (row < total_rows) {
+    reinterpret_cast<int4 *>(coors)[row] = make_int4(0, 0, 0, 0);        // padding row (its mean: below)
   }
   if (row < total_rows) num_points[row] = cnt;
   s_src[lane] = pts.per_sample ? pts.per_sample[b] - (int64_t)begin * F : pts.cat;
@@ -950,6 +971,8 @@ vox_finalize_coop_kernel(VoxPoints pts, const int32_t *__restrict__ offsets, int
           if (voxel_mean) voxel_mean[orow * mean_features + f] = m;
           if (canvas) canvas[rcell + (int64_t)f * canvas_plane] = m;
         }
+      } else if (voxel_mean && hrow0 + rl < total_rows) {   // padding row (live rows hold at least one point)
+        for (int f = par; f < mean_features; f += 2) voxel_mean[(hrow0 + rl) * mean_features + f] = 0.f;
       }
     }
     // the half's 16 rows are one contiguous span of the output
@@ -1288,7 +1311,9 @@ static int hard_voxelize_impl(const float *points, const float *const *sample_pt
                                max_points, max_voxels, voxels, coors, num_points, voxel_base, voxel_mean, mean_features,
                                canvas, temp, stream, !canvas_prezeroed);
   }
-  if (canvas || !points) return BEVPOOL_E_RANGE;   // the fused canvas and per-sample pointers exist on the dense-grid path only
+  if (sample_ptrs) return BEVPOOL_E_RANGE;          // per-sample pointers exist on the dense-grid path only
+  if (canvas && !canvas_prezeroed)                  // the gather kernel stores the occupied cells
+    BEVPOOL_RETURN_IF_CUDA(cudaMemsetAsync(canvas, 0, (size_t)batch * mean_features * g.gx * g.gy * g.gz * sizeof(float), stream));
   const VoxTemp L = vox_temp_layout(batch, total_points, max_voxels, max_points);
   char *tb = static_cast<char *>(temp);
   int32_t *counts = reinterpret_cast<int32_t *>(tb + L.off_counts);
@@ -1321,8 +1346,8 @@ static int hard_voxelize_impl(const float *points, const float *const *sample_pt
   }
   const int64_t rows = (int64_t)batch * max_voxels;
   vox_gather_kernel<<<(unsigned)ceil_div64(rows, 8), 256, 0, stream>>>(points, num_features, lists, counts, voxel_base,
-                                                                      batch, max_points, voxels, num_points,
-                                                                      voxel_mean, mean_features);
+                                                                      batch, rows, max_points, voxels, num_points, coors,
+                                                                      voxel_mean, mean_features, g, canvas);
   BEVPOOL_LAUNCH_CHECK();
   return BEVPOOL_OK;
 }
@@ -1339,9 +1364,9 @@ extern "C" int bevvox_hard_voxelize(const float *points, const int32_t *sample_o
 }
 
 // voxelize + HardSimpleVFE + pillar scatter in one call (models/bev_depth.py:181-183 with a dense-scatter middle
-// encoder).  The clouds are given either concatenated (`points`) or as a DEVICE array of `batch` per-sample base
-// pointers (`sample_ptrs`, points == NULL): the list of tensors the reference passes, without a torch.cat.  canvas
-// (batch, mean_features, gz, gy, gx) may be NULL (no scatter).  Dense-grid path only.
+// encoder).  The clouds are given either concatenated (`points`) or, on the dense-grid path, as a DEVICE array of
+// `batch` per-sample base pointers (`sample_ptrs`, points == NULL): the list of tensors the reference passes, without a
+// torch.cat.  canvas (batch, mean_features, gz, gy, gx) may be NULL (no scatter).
 extern "C" int bevvox_hard_voxelize_scatter(const float *points, const float *const *sample_ptrs,
                                             const int32_t *sample_offsets, int batch, int64_t total_points,
                                             int64_t max_sample_points, int num_features, const float *voxel_size_host,
@@ -1349,7 +1374,6 @@ extern "C" int bevvox_hard_voxelize_scatter(const float *points, const float *co
                                             int max_voxels, float *voxels, int32_t *coors, int32_t *num_points,
                                             int32_t *voxel_base, float *voxel_mean, int mean_features, float *canvas,
                                             int canvas_is_zeroed, void *temp, void *stream_) {
-  if (grid_host && !vox_dense_ok(batch, grid_host)) return BEVPOOL_E_RANGE;
   return hard_voxelize_impl(points, sample_ptrs, sample_offsets, batch, total_points, max_sample_points, num_features,
                             voxel_size_host, range_host, grid_host, max_points, max_voxels, voxels, coors, num_points,
                             voxel_base, voxel_mean, mean_features, canvas, temp, stream_, canvas_is_zeroed != 0);

@@ -84,9 +84,12 @@ def hard_voxelize_batch(points_list: Sequence[torch.Tensor], voxel_size, point_c
     (M, mean_features) or None)`` with the samples' voxels concatenated in order (mmdet3d's packing).  M is
     data dependent, so the exact-size result costs ONE D2H sync (mmcv pays one per sample) and ``voxel_base`` comes
     back on the CPU.  ``padded=True`` skips the sync (CUDA-graph capturable): the tensors keep their ``B *
-    max_voxels`` rows -- rows >= voxel_base[B] are zero -- and ``voxel_base`` stays on the device.
+    max_voxels`` rows -- every row >= voxel_base[B] of ``voxels``, ``num_points``, ``coors`` and ``voxel_mean`` is zero,
+    on the dense-table and the hash pipeline alike -- and ``voxel_base`` stays on the device.
     ``scatter=True`` (needs ``mean_features``) appends the dense BEV canvas ``(B, mean_features * gz, gy, gx)`` of the
-    fused HardSimpleVFE mean: voxelize -> VFE -> scatter of ``models/bev_depth.py:181-183`` in one call.
+    fused HardSimpleVFE mean: voxelize -> VFE -> scatter of ``models/bev_depth.py:181-183`` in one call.  Only the live
+    rows reach it.  The mean is mmdet3d's, summed in float32 from +0 over the voxel's points in point order and divided
+    once by the count (``oracle.voxelize_ref.vfe_mean_exact``), bit for bit on every pipeline.
     """
     assert len(points_list) > 0
     _lib.require_cuda(*points_list)
@@ -127,20 +130,13 @@ def hard_voxelize_batch(points_list: Sequence[torch.Tensor], voxel_size, point_c
                 _f32_array(voxel_size), _f32_array(point_cloud_range), grid_c, max_num_points, max_voxels,
                 voxels.data_ptr(), coors.data_ptr(), num_points.data_ptr(), voxel_base.data_ptr(),
                 mean.data_ptr() if mean is not None else None, mean_features]
-        canvas = None
-        if dense:
-            if scatter:
-                canvas = torch.empty(B, mean_features * gz, gy, gx, dtype=torch.float32, device=dev)
-            _lib.check(L.bevvox_hard_voxelize_scatter(
-                points.data_ptr() if (points is not None and total > 0) else None,
-                sample_ptrs.data_ptr() if sample_ptrs is not None else None, *tail,
-                canvas.data_ptr() if canvas is not None else None, 0, temp.data_ptr(), _lib.stream_ptr(dev)),
-                'bevvox_hard_voxelize_scatter')
-        else:
-            _lib.check(L.bevvox_hard_voxelize(points.data_ptr() if total > 0 else None, *tail, temp.data_ptr(),
-                                              _lib.stream_ptr(dev)), 'bevvox_hard_voxelize')
-            if scatter:              # hash path (huge grids): the separate scatter kernel
-                canvas = pillar_scatter(mean, coors, B, (gz, gy, gx), unique_coors=True)
+        # (the canvas takes only the voxel_base[B] live rows, counted on the device, on both paths)
+        canvas = torch.empty(B, mean_features * gz, gy, gx, dtype=torch.float32, device=dev) if scatter else None
+        _lib.check(L.bevvox_hard_voxelize_scatter(
+            points.data_ptr() if (points is not None and total > 0) else None,
+            sample_ptrs.data_ptr() if sample_ptrs is not None else None, *tail,
+            canvas.data_ptr() if canvas is not None else None, 0, temp.data_ptr(), _lib.stream_ptr(dev)),
+            'bevvox_hard_voxelize_scatter')
         if padded:
             out = (voxels, num_points, coors, voxel_base, mean)
             return out + (canvas,) if scatter else out

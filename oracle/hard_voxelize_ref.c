@@ -31,10 +31,11 @@ int hard_voxelize_ref(const float *points, int num_points, int num_features,
                       const float *voxel_size, const float *range, const int *grid,
                       int max_points, int max_voxels, float *voxels, int *coors,
                       int *num_points_per_voxel) {
+  /* cell -> voxel id + 1 (0: no voxel yet), indexed in 64 bits: grids of 2^31 cells and more are valid.  calloc'd
+   * pages are zero until written, so such a grid costs memory only where the cloud has points. */
   const long gx = grid[0], gy = grid[1], gz = grid[2];
-  int *coor_to_voxelidx = (int *)malloc(sizeof(int) * (size_t)(gx * gy * gz));
+  int *coor_to_voxelidx = (int *)calloc((size_t)gx * (size_t)gy * (size_t)gz, sizeof(int));
   if (!coor_to_voxelidx) return -1;
-  for (long i = 0; i < gx * gy * gz; ++i) coor_to_voxelidx[i] = -1;
 
   int voxel_num = 0;
   for (int i = 0; i < num_points; ++i) {
@@ -50,11 +51,11 @@ int hard_voxelize_ref(const float *points, int num_points, int num_features,
     }
     if (failed) continue;
     long cell = ((long)coor[0] * gy + coor[1]) * gx + coor[2];
-    int vid = coor_to_voxelidx[cell];
+    int vid = coor_to_voxelidx[cell] - 1;
     if (vid == -1) {
       if (max_voxels != -1 && voxel_num >= max_voxels) continue;
       vid = voxel_num++;
-      coor_to_voxelidx[cell] = vid;
+      coor_to_voxelidx[cell] = vid + 1;
       coors[vid * 3 + 0] = coor[0];
       coors[vid * 3 + 1] = coor[1];
       coors[vid * 3 + 2] = coor[2];

@@ -147,6 +147,32 @@ def hard_simple_vfe_ref(voxels, num_points, num_features=5):
     return s / num_points.astype(np.float32)[:, None]
 
 
+def vfe_mean_exact(voxels, num_points, nf):
+    """The HardSimpleVFE mean exactly as every finalize and gather kernel of ``csrc/voxelize.cu`` computes it, in numpy
+    float32: a sum that starts from +0.0f, adds the ``cnt`` filled slots one at a time in slot order (= ascending point
+    index), then ONE IEEE division by ``float(cnt)``.  Rows with ``cnt == 0`` (the padding rows) are +0.  Unlike
+    ``hard_simple_vfe_ref`` (numpy's pairwise ``sum``, the statement of mmdet3d's op) the summation order is fixed, so
+    the kernels' means can be compared bit for bit."""
+    v = np.asarray(voxels, dtype=np.float32)
+    cnt = np.asarray(num_points).astype(np.int64)
+    m = v.shape[0]
+    s = np.zeros((m, nf), np.float32)
+    out = np.zeros((m, nf), np.float32)
+    full = cnt > 0
+    with np.errstate(invalid='ignore', over='ignore'):     # (NaN / inf inputs propagate, as on the GPU)
+        for t in range(v.shape[1]):
+            live = (t < cnt)[:, None]
+            s = np.where(live, s + v[:, t, :nf], s)        # (slots >= cnt are not added: -0 + +0 would be +0)
+        out[full] = s[full] / cnt[full].astype(np.float32)[:, None]
+    return out
+
+
+def canvas_exact(voxels, num_points, coors, nf, batch_size, grid_zyx):
+    """Dense canvas (B, nf*nz, ny, nx) of ``vfe_mean_exact`` at ``coors`` [b, z, y, x]: what the fused
+    ``voxelize(..., scatter=True)`` writes."""
+    return pillar_scatter_ref(vfe_mean_exact(voxels, num_points, nf), coors, batch_size, grid_zyx)
+
+
 def pillar_scatter_ref(voxel_features, coors, batch_size, grid_zyx):
     """Scatter (M, C) voxel features to a dense zero canvas at ``coors`` [b, z, y, x]
     -> (B, C*nz, ny, nx): PointPillarsScatter for nz == 1, ``SparseConvTensor.dense()``

@@ -133,3 +133,95 @@ def test_reciprocal_cell_index_rule_equals_the_exact_division():
         ordinary = np.arange(p.size) >= near.size                    # the uniformly drawn coordinates
         ordinary &= (q > 0) & (q < 4000)
         assert fast_ok[ordinary].mean() > 0.99                       # (the exact path is the rare one on ordinary data)
+
+
+# ---- the VFE mean as the kernels compute it (oracle.voxelize_ref.vfe_mean_exact) -------------------------------------
+def _rows(rows, width=None):
+    """(M, T, 1) voxels and counts from ragged rows of a single feature column."""
+    t = width or max(len(r) for r in rows)
+    v = np.zeros((len(rows), t, 1), np.float32)
+    for i, r in enumerate(rows):
+        v[i, :len(r), 0] = r
+    return v, np.array([len(r) for r in rows], np.int32)
+
+
+def test_vfe_mean_exact_sums_in_slot_order():
+    two24 = np.float32(2 ** 24)
+    v, n = _rows([[2 ** 24, 1, 1], [1e8, 3, -1e8], [1, 1, 2 ** 24]])
+    m = vz.vfe_mean_exact(v, n, 1)[:, 0]
+    # 2^24 + 1 rounds back to 2^24 (ties to even) twice: fl(2^24 / 3), not fl((2^24 + 2) / 3)
+    assert m[0] == two24 / np.float32(3) and m[0] != np.float32(2 ** 24 + 2) / np.float32(3)
+    # 1e8 + 3 rounds to 1e8 (ulp 8), the -1e8 cancels it: +0, where the exact mean is 1
+    assert m[1] == 0.0 and not np.signbit(m[1])
+    # the other order keeps both ones: 2 + 2^24 is exact
+    assert m[2] == np.float32(2 ** 24 + 2) / np.float32(3)
+
+
+def test_vfe_mean_exact_signed_zero_and_non_finite():
+    nan, inf = np.float32(np.nan), np.float32(np.inf)
+    v, n = _rows([[-0.0], [-0.0, -0.0], [1.0, nan, 2.0], [inf, 1.0], [-inf, 5.0], [inf, -inf], [3e38, 3e38]], width=4)
+    v[:, 2:, 0] = -0.0                                     # (slots beyond the count must not be added)
+    m = vz.vfe_mean_exact(v, n, 1)[:, 0]
+    assert m[0] == 0.0 and not np.signbit(m[0])           # +0 + -0 = +0, and +0 / 1 = +0
+    assert m[1] == 0.0 and not np.signbit(m[1])
+    assert np.isnan(m[2]) and m[3] == inf and m[4] == -inf and np.isnan(m[5])
+    assert m[6] == inf                                    # the float32 sum overflows before the division
+    # a padding row (count 0) is +0, not 0 / 0
+    z = vz.vfe_mean_exact(np.zeros((2, 3, 2), np.float32), np.zeros(2, np.int32), 2)
+    assert np.array_equal(z.view(np.int32), np.zeros((2, 2), np.int32))
+
+
+@pytest.mark.parametrize('T', [1, 3, 15, 35])
+def test_vfe_mean_exact_error_bound(T):
+    # sequential float32 summation then one rounding of the division: |m - mean| <= gamma_cnt * sum|v| / cnt
+    rng = np.random.default_rng(T)
+    M, nf = 4000, 5
+    v = (rng.standard_normal((M, T, nf)) * 10.0 ** rng.integers(-3, 6, (M, T, 1))).astype(np.float32)
+    n = rng.integers(1, T + 1, M).astype(np.int32)
+    m = vz.vfe_mean_exact(v, n, nf).astype(np.float64)
+    live = (np.arange(T)[None, :] < n[:, None])[:, :, None]
+    v64 = np.where(live, v.astype(np.float64), 0.0)
+    exact = v64.sum(1) / n[:, None]
+    u = 2.0 ** -24
+    gamma = (n * u / (1 - n * u))[:, None]
+    assert np.all(np.abs(m - exact) <= gamma * np.abs(v64).sum(1) / n[:, None])
+
+
+def test_vfe_mean_exact_differs_from_numpy_pairwise_sum():
+    # numpy's float32 sum of a contiguous row runs eight partial sums: on this row it keeps the ones the serial sum loses,
+    # so a test comparing against it could not tell the kernels' summation order from another one
+    row = np.concatenate([[2 ** 24], np.ones(15)]).astype(np.float32)
+    v, n = _rows([row])
+    serial = vz.vfe_mean_exact(v, n, 1)[0, 0]
+    pairwise = np.float32(np.sum(row, dtype=np.float32)) / np.float32(16)
+    assert serial == np.float32(2 ** 24) / np.float32(16) and serial != pairwise
+
+
+def test_canvas_exact_places_the_exact_mean():
+    pts = synthetic.lidar_sweep(3000, 5, seed=6)
+    vox, num, coors = vz.voxelize_batch_ref([pts, pts[::-1].copy()], CFG_3.voxel_size, CFG_3.point_cloud_range, 15, 2000)
+    canvas = vz.canvas_exact(vox, num, coors, 4, 2, (1, 256, 2048))
+    mean = vz.vfe_mean_exact(vox, num, 4)
+    assert canvas.shape == (2, 4, 256, 2048)
+    got = canvas[coors[:, 0], :, coors[:, 2], coors[:, 3]]
+    assert np.array_equal(got.view(np.int32), mean.view(np.int32))
+    assert int((canvas != 0).any(1).sum()) <= vox.shape[0]
+
+
+def test_c_and_numpy_agree_beyond_2_to_the_31_cells():
+    # 65536 x 32769 x 1 = 2^31 + 2^16 cells: cell ids past 2^31 must not wrap in either oracle
+    vs, rg = [1.0, 1.0, 1.0], [0, 0, 0, 65536, 32769, 1]
+    assert int(np.prod(vz.grid_size_ref(vs, rg))) > 2 ** 31
+    rng = np.random.default_rng(7)
+    n = 3000
+    x = np.concatenate([rng.integers(0, 65536, n), [65535, 0, 65535, 3]])
+    y = np.concatenate([rng.choice([0, 1, 32767, 32768], n), [32768, 32768, 0, 32768]])
+    pts = np.stack([x + 0.5, y + 0.25, np.full(x.size, 0.5), np.arange(x.size)], 1).astype(np.float32)
+    pts = np.concatenate([pts, pts[:50]])                   # revisits: slots beyond the first
+    a = vz.hard_voxelize_c(pts, vs, rg, 3, 10 ** 6)
+    b = vz.hard_voxelize_numpy(pts, vs, rg, 3, 10 ** 6)
+    for p, q in zip(a, b):
+        assert np.array_equal(p, q)
+    cells = np.unique(y.astype(np.int64) * 65536 + x)
+    assert a[0].shape[0] == cells.size and cells.max() >= 2 ** 31
+    assert [0, 32768, 65535] in a[1].tolist()              # (z, y, x) of cell 2^31 + 65535
