@@ -222,6 +222,43 @@ int bevpool_fused_backward_runs_mixed(const void *plan, const void *grad_rows, i
                                       int feat_h, int feat_w, int channels, int num_voxel_x, int num_voxel_y,
                                       void *stream);
 
+/* ---- fp16 / bf16 concatenated BEV rows (the concat epilogue under autocast) ----------------------------------------
+ * Every value is computed in fp32 exactly as by the fp32 entry points; the only new rounding is one round-to-nearest-
+ * even of each output element where it is stored (fp16: +-inf beyond 65504), so the rows equal the fp32 rows
+ * `.to(dtype)` bit for bit.  Run rows, stage-B partial sums, warp taps and resampling sums stay fp32.  Row pointers and
+ * strides count elements of the 16-bit type; rows 16-byte aligned, strides multiples of 4.  A 16-bit dtype argument
+ * must be BEVPOOL_F16 or BEVPOOL_BF16 (BEVPOOL_F32 or anything else: BEVPOOL_E_DTYPE).
+ * bevpool_fused_forward_runs_into16  ..._runs_mixed (context_dtype F32 / F16 / BF16, flags as there) writing out_dtype
+ *           rows at out_row_stride elements.
+ * bevpool_warp_affine_forward16 / _backward16  the BDA warp between fp32 rows of the pooled map and 16-bit
+ *           concatenated rows: forward fp32 src -> out_dtype destination rows; backward grad_dtype gradient rows -> fp32
+ *           grad_src rows (occupied cells only when cell_start is given).  Same taps, order and skipping as the fp32 ones.
+ * bevpool_resize_nearest_into16 / _backward_from16  the LiDAR half: source / grad_src as in ..._into (`dtype`), rows of
+ *           row_dtype; backward sums in fp32 in the same order and rounds once to `dtype`.
+ * bevpool_grad_rows_widen  camera slice of a 16-bit concatenated gradient (grad_rows at grad_row_stride elements) ->
+ *           packed fp32 (batch, num_voxel_y, num_voxel_x, channels) rows, written for the cells a pooling plan's
+ *           cell_start (batch*Y*X + 1 entries) marks occupied only: the rows the pooling backward reads.              */
+int bevpool_fused_forward_runs_into16(const void *plan, const void *depth, const void *context, int context_dtype,
+                                      int flags, void *out_rows, int64_t out_row_stride, int out_dtype, int batch,
+                                      int num_cams, int depth_bins, int feat_h, int feat_w, int channels, int num_voxel_x,
+                                      int num_voxel_y, void *run_rows, int64_t run_rows_capacity, void *workspace,
+                                      void *stream);
+int bevpool_warp_affine_forward16(const float *theta, const void *src_rows, int64_t src_row_stride, void *out_rows,
+                                  int64_t out_row_stride, int out_dtype, const int32_t *cell_start, int batch,
+                                  int channels, int src_h, int src_w, int dst_h, int dst_w, void *stream);
+int bevpool_warp_affine_backward16(const float *theta, const void *grad_out_rows, int64_t grad_out_row_stride,
+                                   int grad_dtype, void *grad_src_rows, int64_t grad_src_row_stride,
+                                   const int32_t *cell_start, int batch, int channels, int src_h, int src_w, int dst_h,
+                                   int dst_w, void *stream);
+int bevpool_resize_nearest_into16(const void *src, int dtype, int src_is_nchw, int batch, int channels, int src_h,
+                                  int src_w, int dst_h, int dst_w, void *out_rows, int64_t out_row_stride, int row_dtype,
+                                  void *stream);
+int bevpool_resize_nearest_backward_from16(const void *grad_rows, int64_t grad_row_stride, int row_dtype, void *grad_src,
+                                           int dtype, int src_is_nchw, int batch, int channels, int src_h, int src_w,
+                                           int dst_h, int dst_w, void *stream);
+int bevpool_grad_rows_widen(const int32_t *cell_start, const void *grad_rows, int64_t grad_row_stride, int grad_dtype,
+                            float *rows, int batch, int channels, int num_voxel_x, int num_voxel_y, void *stream);
+
 /* ---- run plan straight from the camera rig: no geom_xyz tensor -------------------------------------
  * Replaces layers/backbones/lss_fpn.py:328-361 (get_geometry) + :461-462 (index quantisation) as the
  * producer of the cell indices.  Inputs (all device pointers unless *_host):

@@ -51,6 +51,8 @@ _SIGNATURES = {
     'bevpool_fused_backward_runs_from': [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     'bevpool_fused_forward_runs_mixed': [_vp, _vp, _vp, _i, _i, _vp, _i64, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp, _vp],
     'bevpool_fused_backward_runs_mixed': [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
+    'bevpool_fused_forward_runs_into16': [_vp, _vp, _vp, _i, _i, _vp, _i64, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp,
+                                          _vp],
     'bevpool_plan_status': [_vp, _ip, _vp],
     'bevpool_runplan_rig_sizes': [_i, _i, _i, _i, _i, _i, _i, _szp, _szp],
     'bevpool_runplan_build_rig': [_vp, _vp, _vp, _vp, _fp, _fp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp],
@@ -62,6 +64,11 @@ _SIGNATURES = {
     'bevpool_resize_nearest_into': [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _vp],
     'bevpool_resize_nearest_backward_from': [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     'bevpool_resize_nearest_index': [_i, _i, _vp, _vp],
+    'bevpool_warp_affine_forward16': [_vp, _vp, _i64, _vp, _i64, _i, _vp, _i, _i, _i, _i, _i, _i, _vp],
+    'bevpool_warp_affine_backward16': [_vp, _vp, _i64, _i, _vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp],
+    'bevpool_resize_nearest_into16': [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i64, _i, _vp],
+    'bevpool_resize_nearest_backward_from16': [_vp, _i64, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
+    'bevpool_grad_rows_widen': [_vp, _vp, _i64, _i, _vp, _i, _i, _i, _i, _vp],
     'bevvox_temp_bytes':[_i, _i64, _ip, _i, _i, _szp],
     'bevvox_hard_voxelize_scatter': [_vp, _vp, _vp, _i, _i64, _i64, _i, _fp, _fp, _ip, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp],
     'bevvox_hard_voxelize': [_vp, _vp, _i, _i64, _i64, _i, _fp, _fp, _ip, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp],

@@ -82,10 +82,12 @@ __device__ __forceinline__ void add4(float4 &a, const float4 &v) {
   a.w += v.w;
 }
 
-// ---- forward, NCHW source: CTA = (b, y, 32-cell x-run); every element of the run's C destination rows written once
-template <typename E>
+// ---- forward, NCHW source: CTA = (b, y, 32-cell x-run); every element of the run's C destination rows written once.
+// TO (both forward kernels): element type of the destination rows, fp32 or fp16 / bf16 (each element rounded once; a
+// copy when E == TO).
+template <typename E, typename TO = float>
 __global__ void __launch_bounds__(kRsThreads)
-resize_nearest_fwd_nchw_kernel(const E *__restrict__ src, float *__restrict__ out, int64_t out_stride, int C, int Hs,
+resize_nearest_fwd_nchw_kernel(const E *__restrict__ src, TO *__restrict__ out, int64_t out_stride, int C, int Hs,
                                int Ws, int Hd, int Wd, int tiles_x) {
   pdl_wait();
   pdl_trigger();
@@ -99,22 +101,22 @@ resize_nearest_fwd_nchw_kernel(const E *__restrict__ src, float *__restrict__ ou
   // lanes past the run's end re-read its last cell (never stored)
   const E *s = src + (int64_t)b * C * plane + (int64_t)nearest_src(y, Hs, Hd) * Ws +
                nearest_src(x0 + min(lane, ncell - 1), Ws, Wd);
-  float *o = out + (by * Wd + x0) * out_stride;
+  TO *o = out + (by * Wd + x0) * out_stride;
   for (int c0 = 0; c0 < C; c0 += kRsChunk) {
     const int ck = min(kRsChunk, C - c0);
 #pragma unroll 4
     for (int cc = warp; cc < ck; cc += kRsThreads / 32) tile[lane][cc] = to_f32(s[(int64_t)(c0 + cc) * plane]);
     __syncthreads();
     for (int j = warp; j < ncell; j += kRsThreads / 32)
-      for (int cc = lane; cc < ck; cc += 32) o[(int64_t)j * out_stride + c0 + cc] = tile[j][cc];
+      for (int cc = lane; cc < ck; cc += 32) o[(int64_t)j * out_stride + c0 + cc] = from_f32<TO>(tile[j][cc]);
     __syncthreads();
   }
 }
 
 // ---- forward, channels_last source: 8 lanes per destination row
-template <typename E>
+template <typename E, typename TO = float>
 __global__ void __launch_bounds__(kRsThreads)
-resize_nearest_fwd_rows_kernel(const E *__restrict__ src, float *__restrict__ out, int64_t out_stride, int batch, int C,
+resize_nearest_fwd_rows_kernel(const E *__restrict__ src, TO *__restrict__ out, int64_t out_stride, int batch, int C,
                                int Hs, int Ws, int Hd, int Wd) {
   pdl_wait();
   pdl_trigger();
@@ -126,16 +128,17 @@ resize_nearest_fwd_rows_kernel(const E *__restrict__ src, float *__restrict__ ou
   const int rem = (int)(cell - (int64_t)b * dst_cells);
   const int y = rem / Wd, x = rem - y * Wd;
   const E *s = src + (((int64_t)b * Hs + nearest_src(y, Hs, Hd)) * Ws + nearest_src(x, Ws, Wd)) * C;
-  float *o = out + cell * out_stride;
+  TO *o = out + cell * out_stride;
 #pragma unroll 4
   for (int q = 4 * l8; q < C; q += 32) store4(o + q, load4(s + q));
 }
 
 // ---- backward, NCHW gradient: CTA = (b, sy, 32-cell sx-run); a warp sums the preimage rows of one source cell at a
-// time (lane = channel), the tile is then written out one channel at a time (lane = cell)
-template <typename E>
+// time (lane = channel), the tile is then written out one channel at a time (lane = cell).  TG (both backward kernels):
+// element type of the gradient rows, fp32 or fp16 / bf16 (widened exactly where loaded; the sums stay fp32).
+template <typename E, typename TG = float>
 __global__ void __launch_bounds__(kRsThreads)
-resize_nearest_bwd_nchw_kernel(const float *__restrict__ g, int64_t g_stride, E *__restrict__ gsrc, int C, int Hs,
+resize_nearest_bwd_nchw_kernel(const TG *__restrict__ g, int64_t g_stride, E *__restrict__ gsrc, int C, int Hs,
                                int Ws, int Hd, int Wd, int tiles_x) {
   pdl_wait();
   pdl_trigger();
@@ -146,7 +149,7 @@ resize_nearest_bwd_nchw_kernel(const float *__restrict__ g, int64_t g_stride, E 
   const int sy = (int)(bs % Hs), b = (int)(bs / Hs);
   const int sx0 = tx * kRsCells, ncell = min(kRsCells, Ws - sx0);
   const int y_lo = nearest_first_dst(sy, Hs, Hd), y_hi = nearest_first_dst(sy + 1, Hs, Hd);
-  const float *gb = g + (int64_t)b * Hd * Wd * g_stride;
+  const TG *gb = g + (int64_t)b * Hd * Wd * g_stride;
   const int64_t plane = (int64_t)Hs * Ws;
   E *o = gsrc + (int64_t)b * C * plane + (int64_t)sy * Ws + sx0;
   for (int c0 = 0; c0 < C; c0 += kRsChunk) {
@@ -158,10 +161,10 @@ resize_nearest_bwd_nchw_kernel(const float *__restrict__ g, int64_t g_stride, E 
       for (int k = 0; k < kRsChunk / 32; ++k) acc[k] = 0.f;
       for (int y = y_lo; y < y_hi; ++y)
         for (int x = x_lo; x < x_hi; ++x) {
-          const float *row = gb + ((int64_t)y * Wd + x) * g_stride + c0;
+          const TG *row = gb + ((int64_t)y * Wd + x) * g_stride + c0;
 #pragma unroll
           for (int k = 0; k < kRsChunk / 32; ++k)
-            if (lane + 32 * k < ck) acc[k] += __ldg(row + lane + 32 * k);
+            if (lane + 32 * k < ck) acc[k] += to_f32(__ldg(row + lane + 32 * k));
         }
 #pragma unroll
       for (int k = 0; k < kRsChunk / 32; ++k)
@@ -175,9 +178,9 @@ resize_nearest_bwd_nchw_kernel(const float *__restrict__ g, int64_t g_stride, E 
 }
 
 // ---- backward, channels_last gradient: 8 lanes per source row
-template <typename E>
+template <typename E, typename TG = float>
 __global__ void __launch_bounds__(kRsThreads)
-resize_nearest_bwd_rows_kernel(const float *__restrict__ g, int64_t g_stride, E *__restrict__ gsrc, int batch, int C,
+resize_nearest_bwd_rows_kernel(const TG *__restrict__ g, int64_t g_stride, E *__restrict__ gsrc, int batch, int C,
                                int Hs, int Ws, int Hd, int Wd) {
   pdl_wait();
   pdl_trigger();
@@ -190,7 +193,7 @@ resize_nearest_bwd_rows_kernel(const float *__restrict__ g, int64_t g_stride, E 
   const int sy = rem / Ws, sx = rem - sy * Ws;
   const int y_lo = nearest_first_dst(sy, Hs, Hd), y_hi = nearest_first_dst(sy + 1, Hs, Hd);
   const int x_lo = nearest_first_dst(sx, Ws, Wd), x_hi = nearest_first_dst(sx + 1, Ws, Wd);
-  const float *gb = g + (int64_t)b * Hd * Wd * g_stride;
+  const TG *gb = g + (int64_t)b * Hd * Wd * g_stride;
   E *o = gsrc + cell * C;
   for (int c0 = 4 * l8; c0 < C; c0 += 32 * kRsVec) {
     float4 acc[kRsVec];
@@ -198,7 +201,7 @@ resize_nearest_bwd_rows_kernel(const float *__restrict__ g, int64_t g_stride, E 
     for (int k = 0; k < kRsVec; ++k) acc[k] = make_float4(0.f, 0.f, 0.f, 0.f);
     for (int y = y_lo; y < y_hi; ++y)
       for (int x = x_lo; x < x_hi; ++x) {
-        const float *row = gb + ((int64_t)y * Wd + x) * g_stride;
+        const TG *row = gb + ((int64_t)y * Wd + x) * g_stride;
 #pragma unroll
         for (int k = 0; k < kRsVec; ++k)
           if (c0 + 32 * k < C) add4(acc[k], load4(row + c0 + 32 * k));
@@ -222,38 +225,54 @@ int check_resize_args(const void *src, const void *rows, int64_t row_stride, int
   return BEVPOOL_OK;
 }
 
-template <typename E>
-int launch_resize_fwd(const void *src, int src_is_nchw, int batch, int C, int Hs, int Ws, int Hd, int Wd, float *out,
+template <typename E, typename TO = float>
+int launch_resize_fwd(const void *src, int src_is_nchw, int batch, int C, int Hs, int Ws, int Hd, int Wd, TO *out,
                       int64_t out_stride, cudaStream_t s) {
   const E *p = static_cast<const E *>(src);
   if (src_is_nchw) {
     const int tiles_x = (int)ceil_div64(Wd, kRsCells);
-    BEVPOOL_RETURN_IF_CUDA(launch_pdl(resize_nearest_fwd_nchw_kernel<E>, dim3((unsigned)((int64_t)batch * Hd * tiles_x)),
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(resize_nearest_fwd_nchw_kernel<E, TO>, dim3((unsigned)((int64_t)batch * Hd * tiles_x)),
                                       dim3(kRsThreads), 0, s, p, out, out_stride, C, Hs, Ws, Hd, Wd, tiles_x));
   } else {
     const int64_t threads = (int64_t)batch * Hd * Wd * 8;
-    BEVPOOL_RETURN_IF_CUDA(launch_pdl(resize_nearest_fwd_rows_kernel<E>, dim3((unsigned)ceil_div64(threads, kRsThreads)),
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(resize_nearest_fwd_rows_kernel<E, TO>, dim3((unsigned)ceil_div64(threads, kRsThreads)),
                                       dim3(kRsThreads), 0, s, p, out, out_stride, batch, C, Hs, Ws, Hd, Wd));
   }
   BEVPOOL_LAUNCH_CHECK();
   return BEVPOOL_OK;
 }
 
-template <typename E>
-int launch_resize_bwd(const float *g, int64_t g_stride, void *gsrc, int src_is_nchw, int batch, int C, int Hs, int Ws,
+template <typename E, typename TG = float>
+int launch_resize_bwd(const TG *g, int64_t g_stride, void *gsrc, int src_is_nchw, int batch, int C, int Hs, int Ws,
                       int Hd, int Wd, cudaStream_t s) {
   E *p = static_cast<E *>(gsrc);
   if (src_is_nchw) {
     const int tiles_x = (int)ceil_div64(Ws, kRsCells);
-    BEVPOOL_RETURN_IF_CUDA(launch_pdl(resize_nearest_bwd_nchw_kernel<E>, dim3((unsigned)((int64_t)batch * Hs * tiles_x)),
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(resize_nearest_bwd_nchw_kernel<E, TG>, dim3((unsigned)((int64_t)batch * Hs * tiles_x)),
                                       dim3(kRsThreads), 0, s, g, g_stride, p, C, Hs, Ws, Hd, Wd, tiles_x));
   } else {
     const int64_t threads = (int64_t)batch * Hs * Ws * 8;
-    BEVPOOL_RETURN_IF_CUDA(launch_pdl(resize_nearest_bwd_rows_kernel<E>, dim3((unsigned)ceil_div64(threads, kRsThreads)),
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(resize_nearest_bwd_rows_kernel<E, TG>, dim3((unsigned)ceil_div64(threads, kRsThreads)),
                                       dim3(kRsThreads), 0, s, g, g_stride, p, batch, C, Hs, Ws, Hd, Wd));
   }
   BEVPOOL_LAUNCH_CHECK();
   return BEVPOOL_OK;
+}
+
+template <typename TO>
+int resize_fwd_any(const void *src, int dtype, int src_is_nchw, int batch, int C, int Hs, int Ws, int Hd, int Wd, TO *out,
+                   int64_t out_stride, cudaStream_t s) {
+  if (dtype == BEVPOOL_F32) return launch_resize_fwd<float>(src, src_is_nchw, batch, C, Hs, Ws, Hd, Wd, out, out_stride, s);
+  if (dtype == BEVPOOL_F16) return launch_resize_fwd<__half>(src, src_is_nchw, batch, C, Hs, Ws, Hd, Wd, out, out_stride, s);
+  return launch_resize_fwd<__nv_bfloat16>(src, src_is_nchw, batch, C, Hs, Ws, Hd, Wd, out, out_stride, s);
+}
+
+template <typename TG>
+int resize_bwd_any(const TG *g, int64_t g_stride, void *gsrc, int dtype, int src_is_nchw, int batch, int C, int Hs, int Ws,
+                   int Hd, int Wd, cudaStream_t s) {
+  if (dtype == BEVPOOL_F32) return launch_resize_bwd<float>(g, g_stride, gsrc, src_is_nchw, batch, C, Hs, Ws, Hd, Wd, s);
+  if (dtype == BEVPOOL_F16) return launch_resize_bwd<__half>(g, g_stride, gsrc, src_is_nchw, batch, C, Hs, Ws, Hd, Wd, s);
+  return launch_resize_bwd<__nv_bfloat16>(g, g_stride, gsrc, src_is_nchw, batch, C, Hs, Ws, Hd, Wd, s);
 }
 
 }  // namespace
@@ -301,4 +320,38 @@ extern "C" int bevpool_resize_nearest_backward_from(const float *grad_rows, int6
                                      dst_h, dst_w, s);
   return launch_resize_bwd<__nv_bfloat16>(grad_rows, grad_row_stride, grad_src, src_is_nchw, batch, channels, src_h,
                                           src_w, dst_h, dst_w, s);
+}
+
+// The LiDAR half of an fp16 / bf16 concatenated buffer (row_dtype: BEVPOOL_F16 or BEVPOOL_BF16, else BEVPOOL_E_DTYPE;
+// rows, strides and alignment as above, in elements of row_dtype).  forward: each destination element is the source
+// element rounded once to row_dtype (a copy when the types agree), i.e. the fp32 rows of ..._into `.to(row_dtype)`.
+// backward: the same fp32 sums over the widened 16-bit gradient rows, rounded once to `dtype`.
+extern "C" int bevpool_resize_nearest_into16(const void *src, int dtype, int src_is_nchw, int batch, int channels, int src_h,
+                                             int src_w, int dst_h, int dst_w, void *out_rows, int64_t out_row_stride,
+                                             int row_dtype, void *stream) {
+  const int rc = check_resize_args(src, out_rows, out_row_stride, dtype, src_is_nchw, batch, channels, src_h, src_w,
+                                   dst_h, dst_w);
+  if (rc) return rc;
+  if (row_dtype != BEVPOOL_F16 && row_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (row_dtype == BEVPOOL_F16)
+    return resize_fwd_any(src, dtype, src_is_nchw, batch, channels, src_h, src_w, dst_h, dst_w, static_cast<__half *>(out_rows),
+                          out_row_stride, s);
+  return resize_fwd_any(src, dtype, src_is_nchw, batch, channels, src_h, src_w, dst_h, dst_w,
+                        static_cast<__nv_bfloat16 *>(out_rows), out_row_stride, s);
+}
+
+extern "C" int bevpool_resize_nearest_backward_from16(const void *grad_rows, int64_t grad_row_stride, int row_dtype,
+                                                      void *grad_src, int dtype, int src_is_nchw, int batch, int channels,
+                                                      int src_h, int src_w, int dst_h, int dst_w, void *stream) {
+  const int rc = check_resize_args(grad_src, grad_rows, grad_row_stride, dtype, src_is_nchw, batch, channels, src_h,
+                                   src_w, dst_h, dst_w);
+  if (rc) return rc;
+  if (row_dtype != BEVPOOL_F16 && row_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (row_dtype == BEVPOOL_F16)
+    return resize_bwd_any(static_cast<const __half *>(grad_rows), grad_row_stride, grad_src, dtype, src_is_nchw, batch, channels,
+                          src_h, src_w, dst_h, dst_w, s);
+  return resize_bwd_any(static_cast<const __nv_bfloat16 *>(grad_rows), grad_row_stride, grad_src, dtype, src_is_nchw, batch,
+                        channels, src_h, src_w, dst_h, dst_w, s);
 }

@@ -17,8 +17,10 @@
 // underflowed negative product stays -0 where the zero row would make it +0); the backward writes gradient rows for
 // occupied cells only and leaves the others untouched.
 #include "common.cuh"
+#include "tma.cuh"
 
 #include <math.h>
+#include <type_traits>
 
 namespace bevpool {
 namespace {
@@ -111,6 +113,25 @@ __device__ __forceinline__ void warp_window(const float (&th)[6], int sx, int sy
   y_hi = (int)fmax(fmin(yh, Hd - 1.0), -1.0);
 }
 
+// A chunk of 4 consecutive row elements: a float4 of fp32 rows, 8 bytes (uint2) of fp16 / bf16 rows.  ld4 widens a
+// chunk exactly to fp32; st4 rounds each element once to nearest even (fp16 beyond 65504: +-inf, as torch's `.to(dtype)`).
+template <typename T> using Chunk4 = typename std::conditional<sizeof(T) == 4, float4, uint2>::type;
+template <typename T>
+__device__ __forceinline__ float4 ld4(const Chunk4<T> *p) {
+  if constexpr (sizeof(T) == 4) {
+    return __ldg(p);
+  } else {
+    const uint2 u = __ldg(p);
+    const float2 a = CtxType<T>::to_float2(u.x), b = CtxType<T>::to_float2(u.y);
+    return make_float4(a.x, a.y, b.x, b.y);
+  }
+}
+template <typename T>
+__device__ __forceinline__ void st4(Chunk4<T> *p, const float4 &v) {
+  if constexpr (sizeof(T) == 4) stg_stream_f4(p, v);
+  else *p = make_uint2(CtxType<T>::from_float2(v.x, v.y), CtxType<T>::from_float2(v.z, v.w));
+}
+
 __device__ __forceinline__ void fma4(float4 &acc, const float4 &v, float w) {
   acc.x = fmaf(v.x, w, acc.x);
   acc.y = fmaf(v.y, w, acc.y);
@@ -119,10 +140,12 @@ __device__ __forceinline__ void fma4(float4 &acc, const float4 &v, float w) {
 }
 
 // One 8-lane group per destination pixel; lane l8 owns the float4 chunks l8, l8 + 8, ... of the row.  Every element of
-// every destination row is written exactly once, zeros included.
+// every destination row is written exactly once, zeros included.  TO: element type of the destination rows (fp32, or
+// fp16 / bf16: the fp32 sum of the taps rounded once where it is stored).
+template <typename TO = float>
 __global__ void __launch_bounds__(kWarpThreads)
 warp_affine_fwd_kernel(const float *__restrict__ theta, const float *__restrict__ src, int64_t src_stride,
-                       float *__restrict__ out, int64_t out_stride, const int32_t *__restrict__ cell_start, int batch,
+                       TO *__restrict__ out, int64_t out_stride, const int32_t *__restrict__ cell_start, int batch,
                        int C, int Hs, int Ws, int Hd, int Wd) {
   pdl_wait();
   pdl_trigger();
@@ -148,7 +171,7 @@ warp_affine_fwd_kernel(const float *__restrict__ theta, const float *__restrict_
   }
   const int C4 = C >> 2;
   const float4 *s4 = reinterpret_cast<const float4 *>(src);
-  float4 *o4 = reinterpret_cast<float4 *>(out + pix * out_stride);
+  Chunk4<TO> *o4 = reinterpret_cast<Chunk4<TO> *>(out + pix * out_stride);
   const int64_t s4_stride = src_stride >> 2;
   for (int c0 = 0; c0 < C4; c0 += 8 * kWarpChunks) {
     float4 acc[kWarpChunks];
@@ -167,15 +190,17 @@ warp_affine_fwd_kernel(const float *__restrict__ theta, const float *__restrict_
 #pragma unroll
     for (int j = 0; j < kWarpChunks; ++j) {
       const int q = c0 + 8 * j + l8;
-      if (q < C4) stg_stream_f4(o4 + q, acc[j]);
+      if (q < C4) st4<TO>(o4 + q, acc[j]);
     }
   }
 }
 
 // One 8-lane group per source cell.  The lanes test 8 candidates of the window at a time (row-major order = ascending
-// destination index); the group then adds the matches in that order, each lane for its own channel chunks.
+// destination index); the group then adds the matches in that order, each lane for its own channel chunks.  TG: element
+// type of the gradient rows (fp32, or fp16 / bf16 widened exactly where they are loaded); grad_src is fp32.
+template <typename TG = float>
 __global__ void __launch_bounds__(kWarpThreads)
-warp_affine_bwd_kernel(const float *__restrict__ theta, const float *__restrict__ grad_out, int64_t grad_out_stride,
+warp_affine_bwd_kernel(const float *__restrict__ theta, const TG *__restrict__ grad_out, int64_t grad_out_stride,
                        float *__restrict__ grad_src, int64_t grad_src_stride, const int32_t *__restrict__ cell_start,
                        int batch, int C, int Hs, int Ws, int Hd, int Wd) {
   pdl_wait();
@@ -196,7 +221,7 @@ warp_affine_bwd_kernel(const float *__restrict__ theta, const float *__restrict_
   const int bw = x_hi - x_lo + 1, bh = y_hi - y_lo + 1;
   const int64_t nc = (bw > 0 && bh > 0) ? (int64_t)bw * bh : 0;
   const int C4 = C >> 2;
-  const float4 *g4 = reinterpret_cast<const float4 *>(grad_out) + (int64_t)b * Hd * Wd * (grad_out_stride >> 2);
+  const Chunk4<TG> *g4 = reinterpret_cast<const Chunk4<TG> *>(grad_out) + (int64_t)b * Hd * Wd * (grad_out_stride >> 2);
   const int64_t g4_stride = grad_out_stride >> 2;
   float4 *o4 = reinterpret_cast<float4 *>(grad_src + cell * grad_src_stride);
   for (int c0 = 0; c0 < C4; c0 += 8 * kWarpChunks) {
@@ -225,11 +250,11 @@ warp_affine_bwd_kernel(const float *__restrict__ theta, const float *__restrict_
         m &= m - 1;
         const float wk = __shfl_sync(gmask, w, k, 8);
         const int dk = __shfl_sync(gmask, d, k, 8);
-        const float4 *row = g4 + (int64_t)dk * g4_stride;
+        const Chunk4<TG> *row = g4 + (int64_t)dk * g4_stride;
 #pragma unroll
         for (int jj = 0; jj < kWarpChunks; ++jj) {
           const int q = c0 + 8 * jj + l8;
-          if (q < C4) fma4(acc[jj], __ldg(row + q), wk);
+          if (q < C4) fma4(acc[jj], ld4<TG>(row + q), wk);
         }
       }
     }
@@ -239,6 +264,22 @@ warp_affine_bwd_kernel(const float *__restrict__ theta, const float *__restrict_
       if (q < C4) stg_stream_f4(o4 + q, acc[j]);
     }
   }
+}
+
+// Camera slice of a 16-bit concatenated gradient -> packed fp32 (B, Y, X, C) rows (exact), occupied cells only; one
+// 8-lane group per cell.
+template <typename TG>
+__global__ void __launch_bounds__(kWarpThreads)
+grad_rows_widen_kernel(const int32_t *__restrict__ cell_start, const TG *__restrict__ grad, int64_t grad_stride,
+                       float *__restrict__ rows, int64_t cells, int C) {
+  pdl_wait();
+  pdl_trigger();
+  const int64_t cell = ((int64_t)blockIdx.x * kWarpThreads + threadIdx.x) >> 3;
+  const int l8 = threadIdx.x & 7;
+  if (cell >= cells || __ldg(cell_start + cell + 1) == __ldg(cell_start + cell)) return;
+  const Chunk4<TG> *g = reinterpret_cast<const Chunk4<TG> *>(grad + cell * grad_stride);
+  float4 *o = reinterpret_cast<float4 *>(rows + cell * C);
+  for (int q = l8; q < C / 4; q += 8) stg_stream_f4(o + q, ld4<TG>(g + q));
 }
 
 int check_warp_args(const void *theta, const void *in, int64_t in_stride, const void *out, int64_t out_stride,
@@ -266,7 +307,7 @@ extern "C" int bevpool_warp_affine_forward(const float *theta, const void *src_r
                            dst_h, dst_w);
   if (rc) return rc;
   const int64_t threads = (int64_t)batch * dst_h * dst_w * 8;
-  BEVPOOL_RETURN_IF_CUDA(launch_pdl(warp_affine_fwd_kernel, dim3((unsigned)ceil_div64(threads, kWarpThreads)),
+  BEVPOOL_RETURN_IF_CUDA(launch_pdl(warp_affine_fwd_kernel<float>, dim3((unsigned)ceil_div64(threads, kWarpThreads)),
                                     dim3(kWarpThreads), 0, static_cast<cudaStream_t>(stream), theta,
                                     static_cast<const float *>(src_rows), src_row_stride, static_cast<float *>(out_rows),
                                     out_row_stride, cell_start, batch, channels, src_h, src_w, dst_h, dst_w));
@@ -282,11 +323,85 @@ extern "C" int bevpool_warp_affine_backward(const float *theta, const void *grad
                            src_h, src_w, dst_h, dst_w);
   if (rc) return rc;
   const int64_t threads = (int64_t)batch * src_h * src_w * 8;
-  BEVPOOL_RETURN_IF_CUDA(launch_pdl(warp_affine_bwd_kernel, dim3((unsigned)ceil_div64(threads, kWarpThreads)),
+  BEVPOOL_RETURN_IF_CUDA(launch_pdl(warp_affine_bwd_kernel<float>, dim3((unsigned)ceil_div64(threads, kWarpThreads)),
                                     dim3(kWarpThreads), 0, static_cast<cudaStream_t>(stream), theta,
                                     static_cast<const float *>(grad_out_rows), grad_out_row_stride,
                                     static_cast<float *>(grad_src_rows), grad_src_row_stride, cell_start, batch, channels,
                                     src_h, src_w, dst_h, dst_w));
+  BEVPOOL_LAUNCH_CHECK();
+  return BEVPOOL_OK;
+}
+
+// The BDA warp between the fp32 pooled scratch and the fp16 / bf16 concatenated rows (out_dtype / grad_dtype: BEVPOOL_F16
+// or BEVPOOL_BF16, else BEVPOOL_E_DTYPE).  Same taps, order and cell_start skipping as the fp32 entry points: the
+// forward's destination rows equal theirs `.to(out_dtype)` bit for bit, and the backward's fp32 gradient rows equal
+// theirs on the widened gradient.
+extern "C" int bevpool_warp_affine_forward16(const float *theta, const void *src_rows, int64_t src_row_stride, void *out_rows,
+                                             int64_t out_row_stride, int out_dtype, const int32_t *cell_start, int batch,
+                                             int channels, int src_h, int src_w, int dst_h, int dst_w, void *stream) {
+  int rc = check_warp_args(theta, src_rows, src_row_stride, out_rows, out_row_stride, batch, channels, src_h, src_w,
+                           dst_h, dst_w);
+  if (rc) return rc;
+  if (out_dtype != BEVPOOL_F16 && out_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
+  const dim3 grid((unsigned)ceil_div64((int64_t)batch * dst_h * dst_w * 8, kWarpThreads));
+  const float *src = static_cast<const float *>(src_rows);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (out_dtype == BEVPOOL_F16)
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(warp_affine_fwd_kernel<__half>, grid, dim3(kWarpThreads), 0, s, theta, src, src_row_stride,
+                                      static_cast<__half *>(out_rows), out_row_stride, cell_start, batch, channels, src_h, src_w,
+                                      dst_h, dst_w));
+  else
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(warp_affine_fwd_kernel<__nv_bfloat16>, grid, dim3(kWarpThreads), 0, s, theta, src,
+                                      src_row_stride, static_cast<__nv_bfloat16 *>(out_rows), out_row_stride, cell_start, batch,
+                                      channels, src_h, src_w, dst_h, dst_w));
+  BEVPOOL_LAUNCH_CHECK();
+  return BEVPOOL_OK;
+}
+
+extern "C" int bevpool_warp_affine_backward16(const float *theta, const void *grad_out_rows, int64_t grad_out_row_stride,
+                                              int grad_dtype, void *grad_src_rows, int64_t grad_src_row_stride,
+                                              const int32_t *cell_start, int batch, int channels, int src_h, int src_w,
+                                              int dst_h, int dst_w, void *stream) {
+  int rc = check_warp_args(theta, grad_out_rows, grad_out_row_stride, grad_src_rows, grad_src_row_stride, batch, channels,
+                           src_h, src_w, dst_h, dst_w);
+  if (rc) return rc;
+  if (grad_dtype != BEVPOOL_F16 && grad_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
+  const dim3 grid((unsigned)ceil_div64((int64_t)batch * src_h * src_w * 8, kWarpThreads));
+  float *gsrc = static_cast<float *>(grad_src_rows);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (grad_dtype == BEVPOOL_F16)
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(warp_affine_bwd_kernel<__half>, grid, dim3(kWarpThreads), 0, s, theta,
+                                      static_cast<const __half *>(grad_out_rows), grad_out_row_stride, gsrc, grad_src_row_stride,
+                                      cell_start, batch, channels, src_h, src_w, dst_h, dst_w));
+  else
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(warp_affine_bwd_kernel<__nv_bfloat16>, grid, dim3(kWarpThreads), 0, s, theta,
+                                      static_cast<const __nv_bfloat16 *>(grad_out_rows), grad_out_row_stride, gsrc,
+                                      grad_src_row_stride, cell_start, batch, channels, src_h, src_w, dst_h, dst_w));
+  BEVPOOL_LAUNCH_CHECK();
+  return BEVPOOL_OK;
+}
+
+// Without a BDA warp the pooling backward reads the camera slice of the concatenated gradient directly; a 16-bit one is
+// first widened into fp32 rows here, for the cells the plan's cell_start marks occupied (the only rows that backward
+// reads; the others are left untouched).
+extern "C" int bevpool_grad_rows_widen(const int32_t *cell_start, const void *grad_rows, int64_t grad_row_stride,
+                                       int grad_dtype, float *rows, int batch, int channels, int num_voxel_x,
+                                       int num_voxel_y, void *stream) {
+  if (!cell_start || !grad_rows || !rows || batch <= 0 || num_voxel_x <= 0 || num_voxel_y <= 0) return BEVPOOL_E_ARG;
+  if (channels <= 0 || (channels % 4) != 0) return BEVPOOL_E_CHANNELS;
+  if (grad_row_stride < channels || (grad_row_stride % 4) != 0) return BEVPOOL_E_ARG;
+  if (grad_dtype != BEVPOOL_F16 && grad_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
+  const int64_t cells = (int64_t)batch * num_voxel_x * num_voxel_y;
+  if (cells >= (int64_t)INT32_MAX) return BEVPOOL_E_RANGE;
+  if (!aligned16(grad_rows) || !aligned16(rows)) return BEVPOOL_E_ALIGN;
+  const dim3 grid((unsigned)ceil_div64(cells * 8, kWarpThreads));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (grad_dtype == BEVPOOL_F16)
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(grad_rows_widen_kernel<__half>, grid, dim3(kWarpThreads), 0, s, cell_start,
+                                      static_cast<const __half *>(grad_rows), grad_row_stride, rows, cells, channels));
+  else
+    BEVPOOL_RETURN_IF_CUDA(launch_pdl(grad_rows_widen_kernel<__nv_bfloat16>, grid, dim3(kWarpThreads), 0, s, cell_start,
+                                      static_cast<const __nv_bfloat16 *>(grad_rows), grad_row_stride, rows, cells, channels));
   BEVPOOL_LAUNCH_CHECK();
   return BEVPOOL_OK;
 }

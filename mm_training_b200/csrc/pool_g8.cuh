@@ -103,6 +103,39 @@ __device__ __forceinline__ void g8_store_row_plain(float *row, int l8, const flo
   if (NF2) *reinterpret_cast<float2 *>(row + 32 * NF4 + 2 * l8) = make_float2(v[4 * NF4], v[4 * NF4 + 1]);
 }
 
+// two fp32 values rounded to nearest even into one 32-bit word of fp16 / bf16 (fp16: +-inf beyond 65504)
+__device__ __forceinline__ uint32_t pack2_rn(__half, float a, float b) {
+  const __half2 h = __floats2half2_rn(a, b);
+  return *reinterpret_cast<const uint32_t *>(&h);
+}
+__device__ __forceinline__ uint32_t pack2_rn(__nv_bfloat16, float a, float b) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<const uint32_t *>(&h);
+}
+
+// A finished output row (the only place an output element is rounded): fp32 stored as it is (g8_store_row), fp16 / bf16
+// rounded once to nearest even -- lane l8 writes 8 bytes per float4 chunk and 4 bytes for the float2 tail.
+template <int NV2, typename TO>
+__device__ __forceinline__ void g8_store_out(TO *row, int l8, const float (&v)[2 * NV2]) {
+  if constexpr (sizeof(TO) == 4) {
+    g8_store_row<NV2>(reinterpret_cast<char *>(row), l8, v);
+  } else {
+    constexpr int NF4 = NV2 / 2, NF2 = NV2 & 1;
+#pragma unroll
+    for (int k = 0; k < NF4; ++k)
+      *reinterpret_cast<uint2 *>(row + 32 * k + 4 * l8) =
+          make_uint2(pack2_rn(TO(), v[4 * k], v[4 * k + 1]), pack2_rn(TO(), v[4 * k + 2], v[4 * k + 3]));
+    if (NF2) *reinterpret_cast<uint32_t *>(row + 32 * NF4 + 2 * l8) = pack2_rn(TO(), v[4 * NF4], v[4 * NF4 + 1]);
+  }
+}
+
+// zeros into elements [4q, 4q + 4) of an output row: one float4, or 8 bytes of a 16-bit type (all-zero bits either way)
+template <typename TO>
+__device__ __forceinline__ void st_zero4(TO *row, int64_t q) {
+  if constexpr (sizeof(TO) == 4) stg_stream_f4(reinterpret_cast<float4 *>(row) + q, make_float4(0.f, 0.f, 0.f, 0.f));
+  else reinterpret_cast<uint2 *>(row)[q] = make_uint2(0u, 0u);
+}
+
 // ---- packed fp32 math (Blackwell FFMA2 / FADD2: two fp32 lanes per instruction) ---------------
 template <int NREG>
 __device__ __forceinline__ void axpy_row(float (&acc)[NREG], float a, const float (&v)[NREG]) {
@@ -148,11 +181,13 @@ __host__ __device__ __forceinline__ int fwd_slice_len(int K, int num_slices) {
 // slot order), so no id array is read.  The kernel works on the cells [cell_base, cell_base + total_cells)
 // and on the list entries [cell_start[cell_base], cell_start[cell_base + total_cells)); fill_period == 0
 // launches no zero-fill CTAs (the caller filled the empty cells elsewhere).
-template <int NV2, bool kFused, int U, bool kIdent = false>
+// TO: element type of `out` (fp32, or fp16 / bf16 for run plans: each finished cell is rounded once where it is stored;
+// the partial sums in the workspace stay fp32).
+template <int NV2, bool kFused, int U, bool kIdent = false, typename TO = float>
 __global__ void __launch_bounds__(kFwWarpsPerCta * 32)
 pool_forward_share_kernel(const int32_t *__restrict__ cell_start, const int32_t *__restrict__ sorted_ids,
                           const int32_t *__restrict__ sorted_cells, const float *__restrict__ rows,
-                          const float *__restrict__ depth, float *__restrict__ out,
+                          const float *__restrict__ depth, TO *__restrict__ out,
                           float *__restrict__ ws_head, float *__restrict__ ws_tail, int64_t cell_base,
                           int64_t total_cells, FastDiv div_dhw, FastDiv div_hw, int fill_period,
                           int64_t row_capacity, int64_t out_stride) {
@@ -169,7 +204,6 @@ pool_forward_share_kernel(const int32_t *__restrict__ cell_start, const int32_t 
     const int nfw = (gridDim.x / fill_period) * kFwWarpsPerCta;
     const int64_t per_warp = ((total_cells + nfw - 1) / nfw + 31) & ~(int64_t)31;
     const int64_t c_begin = cell_base + fwarp * per_warp, c_end = min(cell_base + total_cells, c_begin + per_warp);
-    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
     auto load_cs = [&](int64_t c0, int &cs, int &ce) {
       cs = ce = 0;
       if (c0 < c_end) {
@@ -186,14 +220,13 @@ pool_forward_share_kernel(const int32_t *__restrict__ cell_start, const int32_t 
       const unsigned occ = __ballot_sync(kFull, ce > cs);
       if (occ != kFull) {
         if (out_stride == C) {
-          float4 *o4 = reinterpret_cast<float4 *>(out + c0 * C);
 #pragma unroll 4
           for (int i = lane; i < ncell * C4; i += 32)
-            if (!((occ >> (i / C4)) & 1u)) stg_stream_f4(o4 + i, z);
+            if (!((occ >> (i / C4)) & 1u)) st_zero4(out + c0 * C, i);
         } else {                               // rows inside a wider buffer (concatenated BEV features)
 #pragma unroll 4
           for (int i = lane; i < ncell * C4; i += 32)
-            if (!((occ >> (i / C4)) & 1u)) stg_stream_f4(reinterpret_cast<float4 *>(out + (c0 + i / C4) * out_stride) + i % C4, z);
+            if (!((occ >> (i / C4)) & 1u)) st_zero4(out + (c0 + i / C4) * out_stride, i % C4);
         }
       }
       cs = cs_n;
@@ -288,7 +321,7 @@ pool_forward_share_kernel(const int32_t *__restrict__ cell_start, const int32_t 
             g8_store_row<NV2>(reinterpret_cast<char *>(head_row), l8, acc);
             in_head = false;
           } else {
-            g8_store_row<NV2>(reinterpret_cast<char *>(out + (size_t)kk[u] * out_stride), l8, acc);
+            g8_store_out<NV2>(out + (size_t)kk[u] * out_stride, l8, acc);
           }
 #pragma unroll
           for (int r = 0; r < NREG; ++r) acc[r] = 0.f;
@@ -305,11 +338,11 @@ pool_forward_share_kernel(const int32_t *__restrict__ cell_start, const int32_t 
 
 // Combines the partial sums of cells cut by slice boundaries: the slice where such a cell
 // begins owns it and adds, in slice order, the head partials of the slices it continues into.
-template <int NV2>
+template <int NV2, typename TO = float>
 __global__ void __launch_bounds__(128)
 pool_forward_fixup_kernel(const int32_t *__restrict__ cell_start, const int32_t *__restrict__ sorted_cells,
                           const float *__restrict__ ws_head, const float *__restrict__ ws_tail,
-                          float *__restrict__ out, int64_t cell_base, int64_t total_cells, int num_slices,
+                          TO *__restrict__ out, int64_t cell_base, int64_t total_cells, int num_slices,
                           int64_t row_capacity, int64_t out_stride) {
   pdl_wait();
   pdl_trigger();
@@ -333,7 +366,7 @@ pool_forward_fixup_kernel(const int32_t *__restrict__ cell_start, const int32_t 
     for (int r = 0; r < NREG; ++r) acc[r] += v[r];
     if (!(thi < K && __ldg(sorted_cells + thi - 1) == key && __ldg(sorted_cells + thi) == key)) break;
   }
-  g8_store_row<NV2>(reinterpret_cast<char *>(out + (size_t)key * out_stride), l8, acc);
+  g8_store_out<NV2>(out + (size_t)key * out_stride, l8, acc);
 }
 
 inline bool g8_supported(int C) {

@@ -111,12 +111,14 @@ __device__ __forceinline__ void half_rows_to_f32(float *s_ctx, int tid) {
 // TC: element type of the context (fp32, or fp16 / bf16 under autocast).  A 16-bit context arrives in the first half
 // of the tile buffer and is widened to fp32 rows before the first chunk is reduced (exactly: every fp16 / bf16 value
 // is an fp32 value), so the reduction and its summation order are those of the fp32 kernel.
-template <int NV2, bool kNchw, bool kLogits = false, typename TC = float>
+// TO: element type of `out`, which this stage only zero-fills: fp32, or uint16_t for an fp16 / bf16 output (a zero
+// has the same bits in both).  The run rows stay fp32.
+template <int NV2, bool kNchw, bool kLogits = false, typename TC = float, typename TO = float>
 __global__ void __launch_bounds__(kRaThreads, 4)
 frustum_reduce_kernel(const __grid_constant__ CUtensorMap ctx_map, const int32_t *__restrict__ run_code,
                       const int4 *__restrict__ pair_rec, const float *__restrict__ depth,
                       const TC *__restrict__ ctx_nhwc, float *__restrict__ run_rows,
-                      const int32_t *__restrict__ cell_start, float *__restrict__ out, int32_t *__restrict__ status,
+                      const int32_t *__restrict__ cell_start, TO *__restrict__ out, int32_t *__restrict__ status,
                       int img0, int64_t cell_base, int64_t num_cells, int D, int H, int W, int d_split, int d_per_cta,
                       int tiles_h, int tiles_w, int64_t capacity, int vec, int fill, int hints, int64_t out_stride,
                       int64_t dep_img_stride, const float2 *__restrict__ stats) {
@@ -273,21 +275,19 @@ frustum_reduce_kernel(const __grid_constant__ CUtensorMap ctx_map, const int32_t
         const unsigned em = __ballot_sync(kFull, lane < ncell && ce[a] == cs[a]);
         if (ncell == kRaZeroCells && em == kFull && out_stride == C) {
           if (lane == 0) {
-            if (hints) tma_store_1d_hint(out + c0 * C, s_zero, kRaZeroCells * C * 4, l2_policy_evict_first());
-            else tma_store_1d(out + c0 * C, s_zero, kRaZeroCells * C * 4);
+            if (hints) tma_store_1d_hint(out + c0 * C, s_zero, kRaZeroCells * C * sizeof(TO), l2_policy_evict_first());
+            else tma_store_1d(out + c0 * C, s_zero, kRaZeroCells * C * sizeof(TO));
             issued_bulk = true;
           }
         } else if (em) {
-          const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
           if (out_stride == C) {
-            float4 *o4 = reinterpret_cast<float4 *>(out + c0 * C);
 #pragma unroll 4
             for (int i = lane; i < ncell * C4; i += 32)
-              if ((em >> (i / C4)) & 1u) stg_stream_f4(o4 + i, z);
-          } else {                                           // rows inside a wider (concatenated) buffer: C floats every out_stride
+              if ((em >> (i / C4)) & 1u) st_zero4(out + c0 * C, i);
+          } else {                                           // rows inside a wider (concatenated) buffer: C elements every out_stride
 #pragma unroll 4
             for (int i = lane; i < ncell * C4; i += 32)
-              if ((em >> (i / C4)) & 1u) stg_stream_f4(reinterpret_cast<float4 *>(out + (c0 + i / C4) * out_stride) + i % C4, z);
+              if ((em >> (i / C4)) & 1u) st_zero4(out + (c0 + i / C4) * out_stride, i % C4);
           }
         }
       }
@@ -434,9 +434,9 @@ depth_stats_kernel(const float *__restrict__ logits, int64_t img_stride, int D, 
 
 using namespace bevpool;
 
-template <int NV2, bool kNchw, bool kLogits = false, typename TC = float>
+template <int NV2, bool kNchw, bool kLogits = false, typename TC = float, typename TO = float>
 static int launch_stage_a(const CUtensorMap &ctx_map, const PlanView &pv, const float *dp, const TC *cx, float *rr,
-                          float *out, int32_t *status, int img0, int64_t cell_base, int64_t num_cells, int nb, int num_cams,
+                          TO *out, int32_t *status, int img0, int64_t cell_base, int64_t num_cells, int nb, int num_cams,
                           int D, int H, int W, int64_t capacity, int vec, int fill, int hints, int d_split, int64_t out_stride,
                           cudaStream_t s, int64_t dep_img_stride = 0, const float2 *stats = nullptr) {
   if (dep_img_stride <= 0) dep_img_stride = (int64_t)D * H * W;
@@ -449,8 +449,8 @@ static int launch_stage_a(const CUtensorMap &ctx_map, const PlanView &pv, const 
   (void)C;
   const size_t smem = RaSmem<NV2>::bytes;
   if (smem > 48 * 1024)
-    BEVPOOL_RETURN_IF_CUDA(cudaFuncSetAttribute(frustum_reduce_kernel<NV2, kNchw, kLogits, TC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  BEVPOOL_RETURN_IF_CUDA(launch_pdl_if(pdl_forward_enabled(), frustum_reduce_kernel<NV2, kNchw, kLogits, TC>, dim3((unsigned)ctas), dim3(kRaThreads), smem, s,
+    BEVPOOL_RETURN_IF_CUDA(cudaFuncSetAttribute(frustum_reduce_kernel<NV2, kNchw, kLogits, TC, TO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  BEVPOOL_RETURN_IF_CUDA(launch_pdl_if(pdl_forward_enabled(), frustum_reduce_kernel<NV2, kNchw, kLogits, TC, TO>, dim3((unsigned)ctas), dim3(kRaThreads), smem, s,
       ctx_map, pv.run_code, pv.pair_rec, dp, cx, rr, pv.cell_start, out, status, img0, cell_base, num_cells, D, H, W, splits, d_per_cta, tiles_h,
       tiles_w, capacity, vec, fill, hints, out_stride, dep_img_stride, stats));
   BEVPOOL_LAUNCH_CHECK();
@@ -475,31 +475,85 @@ static const RunKnobs &run_knobs() {
   return k;
 }
 
-// stage A of every frame group for a 16-bit context (no logits variant)
-template <typename TC>
-static int launch_stage_a_half(bool nchw, const CUtensorMap &ctx_map, const PlanView &pv, const float *dp, const void *cx,
-                               float *rr, float *out, int32_t *status, int img0, int64_t cell_base, int64_t num_cells, int nb,
-                               int num_cams, int D, int H, int W, int C, int64_t capacity, int vec, int fill, int hints,
-                               int d_split, int64_t out_stride, cudaStream_t s) {
+// stage A of one frame group without logits, for a context of element type TC; TO as in frustum_reduce_kernel
+template <typename TC, typename TO>
+static int launch_stage_a_typed(bool nchw, const CUtensorMap &ctx_map, const PlanView &pv, const float *dp, const void *cx,
+                                float *rr, TO *out, int32_t *status, int img0, int64_t cell_base, int64_t num_cells, int nb,
+                                int num_cams, int D, int H, int W, int C, int64_t capacity, int vec, int fill, int hints,
+                                int d_split, int64_t out_stride, cudaStream_t s) {
   const TC *c = static_cast<const TC *>(cx);
   int rc = BEVPOOL_OK;
   if (nchw) {
-    BEVPOOL_G8_DISPATCH(C, (rc = launch_stage_a<NV2, true, false, TC>(ctx_map, pv, dp, c, rr, out, status, img0, cell_base, num_cells, nb,
-                                                                      num_cams, D, H, W, capacity, vec, fill, hints, d_split, out_stride, s)));
+    BEVPOOL_G8_DISPATCH(C, (rc = launch_stage_a<NV2, true, false, TC, TO>(ctx_map, pv, dp, c, rr, out, status, img0, cell_base, num_cells,
+                                                                          nb, num_cams, D, H, W, capacity, vec, fill, hints, d_split,
+                                                                          out_stride, s)));
   } else {
-    BEVPOOL_G8_DISPATCH(C, (rc = launch_stage_a<NV2, false, false, TC>(ctx_map, pv, dp, c, rr, out, status, img0, cell_base, num_cells, nb,
-                                                                       num_cams, D, H, W, capacity, vec, fill, hints, d_split, out_stride, s)));
+    BEVPOOL_G8_DISPATCH(C, (rc = launch_stage_a<NV2, false, false, TC, TO>(ctx_map, pv, dp, c, rr, out, status, img0, cell_base, num_cells,
+                                                                           nb, num_cams, D, H, W, capacity, vec, fill, hints, d_split,
+                                                                           out_stride, s)));
   }
   return rc;
 }
 
-// ctx_dtype: element type of `context` (BEVPOOL_F32 / F16 / BF16); depth, run rows and output are fp32 (`dtype`)
+// stage A of one frame group: every context type, and the logits variant (fp32 output only)
+template <typename TO>
+static int launch_stage_a_any(int ctx_dtype, bool nchw, const float2 *stats, const CUtensorMap &ctx_map, const PlanView &pv,
+                              const float *dp, const void *cx, float *rr, TO *out, int32_t *status, int img0, int64_t cell_base,
+                              int64_t num_cells, int nb, int num_cams, int D, int H, int W, int C, int64_t capacity, int vec,
+                              int fill, int hints, int d_split, int64_t out_stride, int64_t dep_img_stride, cudaStream_t s) {
+  int rc = BEVPOOL_OK;
+  if (ctx_dtype == BEVPOOL_F16)
+    return launch_stage_a_typed<__half>(nchw, ctx_map, pv, dp, cx, rr, out, status, img0, cell_base, num_cells, nb, num_cams, D, H,
+                                        W, C, capacity, vec, fill, hints, d_split, out_stride, s);
+  if (ctx_dtype == BEVPOOL_BF16)
+    return launch_stage_a_typed<__nv_bfloat16>(nchw, ctx_map, pv, dp, cx, rr, out, status, img0, cell_base, num_cells, nb, num_cams,
+                                               D, H, W, C, capacity, vec, fill, hints, d_split, out_stride, s);
+  if constexpr (sizeof(TO) == 4) {
+    if (nchw && stats) {
+      BEVPOOL_G8_DISPATCH(C, (rc = launch_stage_a<NV2, true, true>(ctx_map, pv, dp, static_cast<const float *>(cx), rr, out, status, img0,
+                                                                   cell_base, num_cells, nb, num_cams, D, H, W, capacity, vec, fill,
+                                                                   hints, d_split, out_stride, s, dep_img_stride, stats)));
+      return rc;
+    }
+  }
+  return launch_stage_a_typed<float>(nchw, ctx_map, pv, dp, cx, rr, out, status, img0, cell_base, num_cells, nb, num_cams, D, H, W,
+                                     C, capacity, vec, fill, hints, d_split, out_stride, s);
+}
+
+// stage B of one frame group: even-share segmented sum of the run rows (identity ids) into `out`, rounded once per
+// element where TO is 16-bit; fill CTAs only if stage A did not fill
+template <typename TO>
+static int launch_stage_b(const PlanView &pv, const float *rr, TO *out, float *workspace, int64_t cell_base, int64_t ncells,
+                          int C, int64_t capacity, int period_b, int cps_b, int64_t out_stride, cudaStream_t s) {
+  const FastDiv one = make_fastdiv(1u);
+  const unsigned ctas_b = (unsigned)(sm_count() * (period_b ? period_b : cps_b));
+  const int slices = (int)(period_b ? ctas_b - ctas_b / period_b : ctas_b) * kFwWarpsPerCta * 4;
+  float *ws_head = workspace;
+  float *ws_tail = ws_head + (size_t)slices * C;
+  cudaError_t le = cudaSuccess;
+  BEVPOOL_G8_DISPATCH(C, (le = launch_pdl_if(pdl_forward_enabled(), pool_forward_share_kernel<NV2, false, 4, true, TO>, dim3(ctas_b),
+                                             dim3(kFwWarpsPerCta * 32), 0, s, pv.cell_start, (const int32_t *)nullptr,
+                                             pv.sorted_cells, rr, (const float *)nullptr, out, ws_head, ws_tail, cell_base,
+                                             ncells, one, one, period_b, capacity, out_stride)));
+  BEVPOOL_RETURN_IF_CUDA(le);
+  BEVPOOL_LAUNCH_CHECK();
+  BEVPOOL_G8_DISPATCH(C, (le = launch_pdl_if(pdl_forward_enabled(), pool_forward_fixup_kernel<NV2, TO>,
+                                             dim3((unsigned)ceil_div64((int64_t)slices * 8, 128)), dim3(128), 0, s,
+                                             pv.cell_start, pv.sorted_cells, (const float *)ws_head, (const float *)ws_tail, out,
+                                             cell_base, ncells, slices, capacity, out_stride)));
+  BEVPOOL_RETURN_IF_CUDA(le);
+  BEVPOOL_LAUNCH_CHECK();
+  return BEVPOOL_OK;
+}
+
+// ctx_dtype: element type of `context` (BEVPOOL_F32 / F16 / BF16); depth and run rows are fp32 (`dtype`); out_dtype:
+// element type of the output rows (BEVPOOL_F32, or F16 / BF16: every value still computed in fp32, rounded once)
 static int fused_forward_runs_impl(const void *plan, const void *depth, const void *context, bool nchw, void *out_nhwc,
                                    int dtype, int batch, int num_cams, int depth_bins, int feat_h, int feat_w,
                                    int channels, int X, int Y, void *run_rows, int64_t run_rows_capacity,
                                    void *workspace, void *stream, int64_t out_stride = 0, int64_t dep_img_stride = 0,
                                    const float2 *stats = nullptr, int64_t ctx_img_stride = 0, bool prezeroed = false,
-                                   int ctx_dtype = BEVPOOL_F32) {
+                                   int ctx_dtype = BEVPOOL_F32, int out_dtype = BEVPOOL_F32) {
   if (ctx_img_stride <= 0) ctx_img_stride = (int64_t)channels * feat_h * feat_w;
   if (out_stride == 0) out_stride = channels;
   if (stats && !nchw) return BEVPOOL_E_ARG;                   // the logits entry point exists for the NCHW layout only
@@ -510,6 +564,7 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
   const int64_t np = (int64_t)num_cams * depth_bins * feat_h * feat_w;
   if (dtype != BEVPOOL_F32) return BEVPOOL_E_DTYPE;
   if (ctx_dtype != BEVPOOL_F32 && ctx_dtype != BEVPOOL_F16 && ctx_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
+  if (out_dtype != BEVPOOL_F32 && out_dtype != BEVPOOL_F16 && out_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
   if (!g8_supported(channels)) return BEVPOOL_E_CHANNELS;
   if (!plan || !depth || !context || !out_nhwc || !run_rows || !workspace || run_rows_capacity <= 0) return BEVPOOL_E_ARG;
   if (!aligned16(context) || !aligned16(out_nhwc) || !aligned16(run_rows) || !aligned16(workspace)) return BEVPOOL_E_ALIGN;
@@ -526,7 +581,7 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
   // prezeroed: the caller zero-filled the output itself (e.g. on a side stream, behind the plan build): nobody fills
   const int fill = prezeroed ? 0 : kn.fill, hints = kn.hints, cps_b = kn.cps_b;
   const float *dp = static_cast<const float *>(depth), *cx = static_cast<const float *>(context);
-  float *rr = static_cast<float *>(run_rows), *out = static_cast<float *>(out_nhwc);
+  float *rr = static_cast<float *>(run_rows);
   CUtensorMap ctx_map{};
   if (nchw) {
     const uint64_t dims[4] = {(uint64_t)feat_w, (uint64_t)feat_h, (uint64_t)channels, (uint64_t)batch * num_cams};
@@ -540,7 +595,6 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
       if ((rc = make_tensor_map(&ctx_map, t, context, 4, dims, strides, box))) return rc;
     }
   }
-  const FastDiv one = make_fastdiv(1u);
   for (int b0 = 0; b0 < batch; b0 += fpc) {
     const int nb = batch - b0 < fpc ? batch - b0 : fpc;
     const int64_t cell_base = (int64_t)b0 * G, ncells = (int64_t)nb * G;
@@ -552,44 +606,28 @@ static int fused_forward_runs_impl(const void *plan, const void *depth, const vo
       const int max_split = (int)ceil_div64(depth_bins, kRaDC);
       d_split = d_split < 1 ? 1 : (d_split > max_split ? max_split : d_split);
     }
-    if (ctx_dtype == BEVPOOL_F16) {
-      rc = launch_stage_a_half<__half>(nchw, ctx_map, pv, dp, context, rr, out, status, b0 * num_cams, cell_base, ncells, nb, num_cams,
-                                       depth_bins, feat_h, feat_w, channels, run_rows_capacity, vec, fill, hints, d_split, out_stride, s);
-    } else if (ctx_dtype == BEVPOOL_BF16) {
-      rc = launch_stage_a_half<__nv_bfloat16>(nchw, ctx_map, pv, dp, context, rr, out, status, b0 * num_cams, cell_base, ncells, nb,
-                                              num_cams, depth_bins, feat_h, feat_w, channels, run_rows_capacity, vec, fill, hints,
-                                              d_split, out_stride, s);
-    } else if (nchw && stats) {
-      BEVPOOL_G8_DISPATCH(channels, (rc = launch_stage_a<NV2, true, true>(ctx_map, pv, dp, cx, rr, out, status, b0 * num_cams, cell_base, ncells, nb,
-                                                                          num_cams, depth_bins, feat_h, feat_w, run_rows_capacity, vec, fill, hints,
-                                                                          d_split, out_stride, s, dep_img_stride, stats)));
-    } else if (nchw) {
-      BEVPOOL_G8_DISPATCH(channels, (rc = launch_stage_a<NV2, true>(ctx_map, pv, dp, cx, rr, out, status, b0 * num_cams, cell_base, ncells, nb, num_cams,
-                                                                    depth_bins, feat_h, feat_w, run_rows_capacity, vec, fill, hints, d_split, out_stride, s)));
-    } else {
-      BEVPOOL_G8_DISPATCH(channels, (rc = launch_stage_a<NV2, false>(ctx_map, pv, dp, cx, rr, out, status, b0 * num_cams, cell_base, ncells, nb, num_cams,
-                                                                     depth_bins, feat_h, feat_w, run_rows_capacity, vec, fill, hints, d_split, out_stride, s)));
-    }
+    const int img0 = b0 * num_cams;
+    if (out_dtype == BEVPOOL_F32)
+      rc = launch_stage_a_any(ctx_dtype, nchw, stats, ctx_map, pv, dp, context, rr, static_cast<float *>(out_nhwc), status, img0,
+                              cell_base, ncells, nb, num_cams, depth_bins, feat_h, feat_w, channels, run_rows_capacity, vec, fill,
+                              hints, d_split, out_stride, dep_img_stride, s);
+    else
+      rc = launch_stage_a_any(ctx_dtype, nchw, stats, ctx_map, pv, dp, context, rr, static_cast<uint16_t *>(out_nhwc), status, img0,
+                              cell_base, ncells, nb, num_cams, depth_bins, feat_h, feat_w, channels, run_rows_capacity, vec, fill,
+                              hints, d_split, out_stride, dep_img_stride, s);
     if (rc) return rc;
-    // stage B: even-share segmented sum of the run rows (identity ids), fill CTAs only if stage A did not fill
     const int period_b = (fill || prezeroed) ? 0 : cps_b + 1;
-    const unsigned ctas_b = (unsigned)(sm_count() * (period_b ? period_b : cps_b));
-    const int slices = (int)(period_b ? ctas_b - ctas_b / period_b : ctas_b) * kFwWarpsPerCta * 4;
-    float *ws_head = static_cast<float *>(workspace);
-    float *ws_tail = ws_head + (size_t)slices * channels;
-    cudaError_t le = cudaSuccess;
-    BEVPOOL_G8_DISPATCH(channels, (le = launch_pdl_if(pdl_forward_enabled(), pool_forward_share_kernel<NV2, false, 4, true>, dim3(ctas_b),
-                                                   dim3(kFwWarpsPerCta * 32), 0, s, pv.cell_start, (const int32_t *)nullptr,
-                                                   pv.sorted_cells, (const float *)rr, (const float *)nullptr, out, ws_head,
-                                                   ws_tail, cell_base, ncells, one, one, period_b, run_rows_capacity, out_stride)));
-    BEVPOOL_RETURN_IF_CUDA(le);
-    BEVPOOL_LAUNCH_CHECK();
-    BEVPOOL_G8_DISPATCH(channels, (le = launch_pdl_if(pdl_forward_enabled(), pool_forward_fixup_kernel<NV2>,
-                                                   dim3((unsigned)ceil_div64((int64_t)slices * 8, 128)), dim3(128), 0, s,
-                                                   pv.cell_start, pv.sorted_cells, (const float *)ws_head,
-                                                   (const float *)ws_tail, out, cell_base, ncells, slices, run_rows_capacity, out_stride)));
-    BEVPOOL_RETURN_IF_CUDA(le);
-    BEVPOOL_LAUNCH_CHECK();
+    float *ws = static_cast<float *>(workspace);
+    if (out_dtype == BEVPOOL_F32)
+      rc = launch_stage_b(pv, rr, static_cast<float *>(out_nhwc), ws, cell_base, ncells, channels, run_rows_capacity, period_b, cps_b,
+                          out_stride, s);
+    else if (out_dtype == BEVPOOL_F16)
+      rc = launch_stage_b(pv, rr, static_cast<__half *>(out_nhwc), ws, cell_base, ncells, channels, run_rows_capacity, period_b, cps_b,
+                          out_stride, s);
+    else
+      rc = launch_stage_b(pv, rr, static_cast<__nv_bfloat16 *>(out_nhwc), ws, cell_base, ncells, channels, run_rows_capacity, period_b,
+                          cps_b, out_stride, s);
+    if (rc) return rc;
   }
   return BEVPOOL_OK;
 }
@@ -634,6 +672,20 @@ extern "C" int bevpool_fused_forward_runs_mixed(const void *plan, const void *de
   return fused_forward_runs_impl(plan, depth, context, (flags & 1) != 0, out_rows, BEVPOOL_F32, batch, num_cams, depth_bins,
                                  feat_h, feat_w, channels, X, Y, run_rows, run_rows_capacity, workspace, stream, out_row_stride,
                                  0, nullptr, 0, (flags & 2) != 0, context_dtype);
+}
+
+// 16-bit concat under autocast: ..._runs_mixed writing fp16 / bf16 rows (out_dtype).  Every value is computed in fp32 as
+// there; the only rounding is the one RNE rounding of each output element where stage B stores it, so the rows equal the
+// fp32 call's rows `.to(out_dtype)` bit for bit.
+extern "C" int bevpool_fused_forward_runs_into16(const void *plan, const void *depth, const void *context, int context_dtype,
+                                                 int flags, void *out_rows, int64_t out_row_stride, int out_dtype, int batch,
+                                                 int num_cams, int depth_bins, int feat_h, int feat_w, int channels, int X, int Y,
+                                                 void *run_rows, int64_t run_rows_capacity, void *workspace, void *stream) {
+  if (out_row_stride <= 0) return BEVPOOL_E_ARG;
+  if (out_dtype != BEVPOOL_F16 && out_dtype != BEVPOOL_BF16) return BEVPOOL_E_DTYPE;
+  return fused_forward_runs_impl(plan, depth, context, (flags & 1) != 0, out_rows, BEVPOOL_F32, batch, num_cams, depth_bins,
+                                 feat_h, feat_w, channels, X, Y, run_rows, run_rows_capacity, workspace, stream, out_row_stride,
+                                 0, nullptr, 0, (flags & 2) != 0, context_dtype, out_dtype);
 }
 
 // lss_fpn.py:423 + :441-443 folded into the forward: the kernel reads DepthNet's output tensor itself -- depth_feature

@@ -69,8 +69,15 @@ def _rows(x: torch.Tensor):
 
 def warp_forward_rows(theta: torch.Tensor, src, src_stride: int, out, out_stride: int,
                       cell_start: Optional[torch.Tensor], B: int, C: int, src_hw, dsize) -> None:
+    """fp32 ``src`` rows -> ``out`` rows; an fp16 / bf16 ``out`` gets the fp32 result rounded once per element."""
     H, W = src_hw
     Hd, Wd = dsize
+    if out.dtype != torch.float32:
+        _lib.check(_lib.lib().bevpool_warp_affine_forward16(
+            theta.data_ptr(), src.data_ptr(), src_stride, out.data_ptr(), out_stride, _lib.dtype_code(out),
+            None if cell_start is None else cell_start.data_ptr(), B, C, H, W, Hd, Wd, _lib.stream_ptr(theta.device)),
+            'bevpool_warp_affine_forward16')
+        return
     _lib.check(_lib.lib().bevpool_warp_affine_forward(
         theta.data_ptr(), src.data_ptr(), src_stride, out.data_ptr(), out_stride,
         None if cell_start is None else cell_start.data_ptr(), B, C, H, W, Hd, Wd, _lib.stream_ptr(theta.device)),
@@ -79,8 +86,15 @@ def warp_forward_rows(theta: torch.Tensor, src, src_stride: int, out, out_stride
 
 def warp_backward_rows(theta: torch.Tensor, grad_out, grad_out_stride: int, grad_src, grad_src_stride: int,
                        cell_start: Optional[torch.Tensor], B: int, C: int, src_hw, dsize) -> None:
+    """``grad_out`` rows -> fp32 ``grad_src`` rows; an fp16 / bf16 ``grad_out`` is widened exactly where it is read."""
     H, W = src_hw
     Hd, Wd = dsize
+    if grad_out.dtype != torch.float32:
+        _lib.check(_lib.lib().bevpool_warp_affine_backward16(
+            theta.data_ptr(), grad_out.data_ptr(), grad_out_stride, _lib.dtype_code(grad_out), grad_src.data_ptr(),
+            grad_src_stride, None if cell_start is None else cell_start.data_ptr(), B, C, H, W, Hd, Wd,
+            _lib.stream_ptr(theta.device)), 'bevpool_warp_affine_backward16')
+        return
     _lib.check(_lib.lib().bevpool_warp_affine_backward(
         theta.data_ptr(), grad_out.data_ptr(), grad_out_stride, grad_src.data_ptr(), grad_src_stride,
         None if cell_start is None else cell_start.data_ptr(), B, C, H, W, Hd, Wd, _lib.stream_ptr(theta.device)),

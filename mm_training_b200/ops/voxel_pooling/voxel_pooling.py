@@ -367,7 +367,8 @@ def fused_forward(plan: PoolingPlan, depth: torch.Tensor, context: torch.Tensor,
     channels-last ``buf``.  ``prezeroed`` (run plans): the kernels write the rows of occupied cells only and leave the
     others as they are -- for an ``out`` that already holds zeros (``fused_forward_cold``) or whose empty cells are never
     read (the BDA warp's scratch).  A point plan writes every cell either way.  fp32 ``depth`` with an fp16 / bf16
-    ``context`` (autocast) gives fp32 rows equal, bit for bit, to the call on ``context.float()``."""
+    ``context`` (autocast) gives fp32 rows equal, bit for bit, to the call on ``context.float()``.  An fp16 / bf16 ``out``
+    (run plans) receives the fp32 rows rounded once, bit for bit ``.to(out.dtype)`` of what an fp32 ``out`` receives."""
     BN, D, H, W = depth.shape
     C = context.shape[1]
     X, Y, _ = plan.voxel_num
@@ -383,9 +384,12 @@ def fused_forward(plan: PoolingPlan, depth: torch.Tensor, context: torch.Tensor,
     with torch.cuda.device(depth.device):
         if out is None:
             out, prezeroed = torch.empty(B, Y, X, C, dtype=depth.dtype, device=depth.device), False
-        assert out.shape == (B, Y, X, C) and out.dtype == depth.dtype
+        half_out = out.dtype in (torch.float16, torch.bfloat16) and depth.dtype == torch.float32
+        assert out.shape == (B, Y, X, C) and (out.dtype == depth.dtype or half_out)
         stride = C if out.is_contiguous() else _strided_rows(out.permute(0, 3, 1, 2))
         assert stride is not None, 'out must be (B, Y, X, C) rows at a uniform cell stride'
+        if route == 'points' and half_out:
+            raise ValueError(f'an {out.dtype} out needs a run plan and a run kernel for C={C}')
         if route == 'points':
             if plan.mode == 'runs':
                 raise ValueError(f'run plans need float32 and C in {RUN_CHANNELS}; build a point plan for C={C}, {depth.dtype}')
@@ -403,6 +407,12 @@ def fused_forward(plan: PoolingPlan, depth: torch.Tensor, context: torch.Tensor,
         nchw = route == 'nchw'
         ctx_arg = context if nchw else (context_rows_nhwc(context) if context_rows is None else context_rows)
         flags = (1 if nchw else 0) | (2 if prezeroed else 0)
+        if half_out:
+            _lib.check(_lib.lib().bevpool_fused_forward_runs_into16(
+                plan.ptr, depth.data_ptr(), ctx_arg.data_ptr(), _lib.dtype_code(context), flags, out.data_ptr(), stride,
+                _lib.dtype_code(out), B, N, D, H, W, C, X, Y, run_rows.data_ptr(), cap, ws.data_ptr(),
+                _lib.stream_ptr(depth.device)), 'bevpool_fused_forward_runs_into16')
+            return out
         if mixed:
             _lib.check(_lib.lib().bevpool_fused_forward_runs_mixed(
                 plan.ptr, depth.data_ptr(), ctx_arg.data_ptr(), _lib.dtype_code(context), flags, out.data_ptr(), stride,
@@ -621,10 +631,12 @@ class VoxelPoolingFusedConcat(Function):
     """``torch.cat([voxel_pooling_fused(...), other_bev], dim=1)`` without the copies of the camera half; with ``theta``
     the camera half is ``warp_affine(voxel_pooling_fused(...), M, (Y, X))`` (``theta`` = ``bev_augment.warp_theta(M)``);
     with ``resize`` the other half is ``F.interpolate(other_bev, size=(Y, X), mode='nearest')``.  The other half is
-    written by ``bevpool_resize_nearest_into`` in either case (identity maps when the sizes agree)."""
+    written by ``bevpool_resize_nearest_into`` in either case (identity maps when the sizes agree).  ``dtype`` fp16 /
+    bf16: the buffer holds the fp32 values rounded once, and the backward reads the 16-bit gradient as it comes (camera
+    rows widened to fp32 for occupied cells only, by the warp backward or ``bevpool_grad_rows_widen``)."""
 
     @staticmethod
-    def forward(ctx, depth, context, other_bev, voxel_num, plan, theta=None, resize=False):
+    def forward(ctx, depth, context, other_bev, voxel_num, plan, theta=None, resize=False, dtype=torch.float32):
         _lib.require_cuda(depth, context, other_bev)
         X, Y, _ = _voxel_num_ints(voxel_num)
         C = context.shape[1]
@@ -637,7 +649,7 @@ class VoxelPoolingFusedConcat(Function):
         route = _route(plan.mode, context, depth)
         with torch.cuda.device(depth.device):
             rows = None if route == 'nchw' else context_rows_nhwc(context)
-            buf = torch.empty(B, Y, X, Ct, dtype=torch.float32, device=depth.device)
+            buf = torch.empty(B, Y, X, Ct, dtype=dtype, device=depth.device)
             if theta is None:
                 fused_forward(plan, depth, context, rows, out=buf[..., :C])
             else:
@@ -648,11 +660,18 @@ class VoxelPoolingFusedConcat(Function):
                                        prezeroed=True)
                 warp_forward_rows(theta, pooled, C, buf, Ct, plan.cell_start, B, C, (Y, X), (Y, X))
             # the other half (resampled or not): the one copy a cat cannot avoid
-            _lib.check(_lib.lib().bevpool_resize_nearest_into(
-                other_bev.data_ptr(), _lib.dtype_code(other_bev), other_nchw, B, C2, Yl, Xl, Y, X, buf[..., C:].data_ptr(),
-                Ct, _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_into')
+            if dtype == torch.float32:
+                _lib.check(_lib.lib().bevpool_resize_nearest_into(
+                    other_bev.data_ptr(), _lib.dtype_code(other_bev), other_nchw, B, C2, Yl, Xl, Y, X,
+                    buf[..., C:].data_ptr(), Ct, _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_into')
+            else:
+                _lib.check(_lib.lib().bevpool_resize_nearest_into16(
+                    other_bev.data_ptr(), _lib.dtype_code(other_bev), other_nchw, B, C2, Yl, Xl, Y, X,
+                    buf[..., C:].data_ptr(), Ct, _lib.dtype_code(buf), _lib.stream_ptr(depth.device)),
+                    'bevpool_resize_nearest_into16')
         ctx.plan, ctx.route, ctx.C, ctx.other_dtype, ctx.theta = plan, route, C, other_bev.dtype, theta
         ctx.other_shape, ctx.other_nchw, ctx.other_code = (B, C2, Yl, Xl), other_nchw, _lib.dtype_code(other_bev)
+        ctx.half = dtype != torch.float32
         ctx.save_for_backward(depth, context, rows)
         return buf.permute(0, 3, 1, 2)
 
@@ -663,7 +682,11 @@ class VoxelPoolingFusedConcat(Function):
         B = plan.batch
         X, Y, _ = plan.voxel_num
         g = grad_cat.permute(0, 2, 3, 1)
-        if not g.is_contiguous() or g.dtype != torch.float32:           # channels_last gradients (the usual case) pass as they are
+        half = ctx.half
+        if half:                                    # read in its own dtype; only a layout other than channels_last is copied
+            if not g.is_contiguous() or g.data_ptr() % 16 != 0:
+                g = g.contiguous()
+        elif not g.is_contiguous() or g.dtype != torch.float32:           # channels_last gradients (the usual case) pass as they are
             g = g.float().contiguous()
         Ct = g.shape[-1]
         with torch.cuda.device(depth.device):
@@ -674,6 +697,12 @@ class VoxelPoolingFusedConcat(Function):
                 from ..bev_augment import warp_backward_rows
                 grad_rows, stride = _warp_scratch(B, Y, X, C, depth.device), C
                 warp_backward_rows(ctx.theta, g, Ct, grad_rows, C, plan.cell_start, B, C, (Y, X), (Y, X))
+            elif half:
+                # the camera slice widened to fp32 rows, occupied cells only: the rows the column backward reads
+                grad_rows, stride = _warp_scratch(B, Y, X, C, depth.device), C
+                _lib.check(_lib.lib().bevpool_grad_rows_widen(
+                    plan.cell_start.data_ptr(), g.data_ptr(), Ct, _lib.dtype_code(g), grad_rows.data_ptr(), B, C, X, Y,
+                    _lib.stream_ptr(depth.device)), 'bevpool_grad_rows_widen')
             grad_depth, grad_context = _fused_backward_rows(plan, ctx.route, grad_rows, stride, depth, context, rows)
             _, C2, Yl, Xl = ctx.other_shape
             if (Yl, Xl) == (Y, X):
@@ -686,15 +715,20 @@ class VoxelPoolingFusedConcat(Function):
                     grad_other = torch.empty(B, C2, Yl, Xl, dtype=ctx.other_dtype, device=depth.device)
                 else:
                     grad_other = torch.empty(B, Yl, Xl, C2, dtype=ctx.other_dtype, device=depth.device).permute(0, 3, 1, 2)
-                _lib.check(_lib.lib().bevpool_resize_nearest_backward_from(
-                    g[..., C:].data_ptr(), Ct, grad_other.data_ptr(), ctx.other_code, ctx.other_nchw, B, C2,
-                    Yl, Xl, Y, X, _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_backward_from')
-        return grad_depth, grad_context, grad_other, None, None, None, None
+                if half:
+                    _lib.check(_lib.lib().bevpool_resize_nearest_backward_from16(
+                        g[..., C:].data_ptr(), Ct, _lib.dtype_code(g), grad_other.data_ptr(), ctx.other_code, ctx.other_nchw,
+                        B, C2, Yl, Xl, Y, X, _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_backward_from16')
+                else:
+                    _lib.check(_lib.lib().bevpool_resize_nearest_backward_from(
+                        g[..., C:].data_ptr(), Ct, grad_other.data_ptr(), ctx.other_code, ctx.other_nchw, B, C2,
+                        Yl, Xl, Y, X, _lib.stream_ptr(depth.device)), 'bevpool_resize_nearest_backward_from')
+        return grad_depth, grad_context, grad_other, None, None, None, None, None
 
 
 def voxel_pooling_fused_concat(depth: torch.Tensor, context: torch.Tensor, other_bev: torch.Tensor, voxel_num: VoxelNum,
                                plan: PoolingPlan, *, bda_affine: Optional[torch.Tensor] = None,
-                               resize_other: Optional[str] = None) -> torch.Tensor:
+                               resize_other: Optional[str] = None, dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     """Concat epilogue of the camera branch (``models/bev_depth.py:187-189``): returns
     ``torch.cat([voxel_pooling_fused(None, depth, context, voxel_num, plan), other_bev], dim=1)`` as a float32
     channels-last tensor.  On a run plan (fp32, W % 4 == 0) the pooled rows are written straight into the concatenated
@@ -712,9 +746,21 @@ def voxel_pooling_fused_concat(depth: torch.Tensor, context: torch.Tensor, other
     straight into the concatenated buffer, and the gradient of ``other_bev`` is gathered straight out of the concatenated
     gradient: the exact adjoint of the forward's index maps, summed in fp32 in torch's order (ascending y, then x) and
     rounded once, in the dtype and memory format of ``other_bev``; no atomics.  ``None`` (default): ``other_bev`` must
-    already be (B, C2, Y, X).  Other modes raise ``ValueError``."""
+    already be (B, C2, Y, X).  Other modes raise ``ValueError``.
+
+    ``dtype``: ``None`` / ``torch.float32`` (default) returns the float32 buffer above.  ``torch.bfloat16`` /
+    ``torch.float16`` (what the first conv casts to under autocast) returns that dtype, equal bit for bit to the float32
+    result ``.to(dtype)``: every value is still computed in fp32, and each output element is rounded once where it is
+    stored (fp16 overflow gives +-inf).  Its backward takes the 16-bit gradient as it comes, in any memory format, and
+    gives ``depth``, ``context`` and ``other_bev`` the gradients the float32 call gives for ``grad.float()``, bit for bit,
+    in the same dtypes and layouts; with identical grid sizes the gradient of an ``other_bev`` of that dtype is a view.
+    On the native path the result is a channels-last view of one (B, Y, X, C + C2) buffer, and no float32 copy of the
+    buffer or of its gradient is made; elsewhere the float32 result is cast.  Other dtypes raise ``ValueError``."""
     if resize_other not in (None, 'nearest'):
         raise ValueError(f"resize_other must be None or 'nearest' (got {resize_other!r})")
+    if dtype not in (None, torch.float32, torch.float16, torch.bfloat16):
+        raise ValueError(f'dtype must be None, torch.float32, torch.float16 or torch.bfloat16 (got {dtype})')
+    half = dtype in (torch.float16, torch.bfloat16)
     if other_bev.shape[0] != plan.batch:
         raise ValueError(f'other_bev has batch {other_bev.shape[0]}, the plan {plan.batch}')
     X, Y, _ = plan.voxel_num
@@ -728,6 +774,8 @@ def voxel_pooling_fused_concat(depth: torch.Tensor, context: torch.Tensor, other
         if bda_affine is not None:
             from ..bev_augment import warp_theta
             theta = warp_theta(bda_affine, (Y, X), (Y, X)).to(depth.device)
+        if half:
+            return VoxelPoolingFusedConcat.apply(depth, context, other_bev, voxel_num, plan, theta, resize, dtype)
         return VoxelPoolingFusedConcat.apply(depth, context, other_bev, voxel_num, plan, theta, resize)
     camera = voxel_pooling_fused(None, depth, context, voxel_num, plan)
     if bda_affine is not None:
@@ -735,7 +783,8 @@ def voxel_pooling_fused_concat(depth: torch.Tensor, context: torch.Tensor, other
         camera = warp_affine(camera, bda_affine, (Y, X))
     if resize:
         other_bev = torch.nn.functional.interpolate(other_bev, size=(Y, X), mode='nearest')
-    return torch.cat([camera, other_bev.to(camera.dtype)], dim=1)
+    out = torch.cat([camera, other_bev.to(camera.dtype)], dim=1)
+    return out.to(dtype) if half else out
 
 
 class VoxelPoolingFusedLogits(Function):
